@@ -2,6 +2,7 @@
 """bench.py -- transect-flux throughput on synthetic ORCA-shaped data (BASELINE.json metric).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--workload auto|C3|C4|C5] [--dtype f64|f32] [--impl reference]
+                    [--dump-outputs DIR]
 
 One "step" = one pass of the hot path (K2 edge-flux assembly + K3 batched transect reduction, plus the NCCL
 allgather of the flux series when N > 1) over the whole time series of the workload.
@@ -79,7 +80,25 @@ def parse_args():
     ap.add_argument('--ring-slot-mb', type=int, default=0)
     ap.add_argument('--no-pad', action='store_true',
                     help='store u/v densely; default: level planes padded to 32 bytes when ncell*itemsize is not')
-    return ap.parse_args()
+    ap.add_argument('--dump-outputs', metavar='DIR', default='',
+                    help='after the timed steps, write what the last step computed (the flux series) as DIR/<name>.npy')
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error('--steps must be at least 1')
+    return args
+
+
+DUMP_BUDGET_BYTES = 64 << 20
+
+
+def dump_outputs(path, arrays):
+    """--dump-outputs: every array as float64 <path>/<name>.npy.  The inputs are a function of the arguments only
+    (synth.py is seeded), so two builds run with the same arguments can be compared file for file.  Should the total
+    pass 64 MB, every array keeps the same fixed stride of its rows (time steps)."""
+    os.makedirs(path, exist_ok=True)
+    stride = max(1, math.ceil(sum(a.size * 8 for a in arrays.values()) / DUMP_BUDGET_BYTES))
+    for name, a in arrays.items():
+        numpy.save(os.path.join(path, name + '.npy'), numpy.ascontiguousarray(a[::stride], numpy.float64))
 
 
 def pick_workload(args, world):
@@ -257,7 +276,7 @@ def run_reference(args):
         cpu_reference_pass(O, syn, plis, fields[:1], args.order)
     times = []
     for _ in range(args.steps):
-        dt, _ = cpu_reference_pass(O, syn, plis, fields, args.order)
+        dt, series = cpu_reference_pass(O, syn, plis, fields, args.order)
         times.append(dt)
     dt = float(numpy.mean(times))
     units = syn.units_per_step() * sample
@@ -275,6 +294,8 @@ def run_reference(args):
         'gpu_launches': 0,
     }
     print(json.dumps(line), flush=True)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {'flux_series': series})
 
 
 # ---------------------------------------------------------------------------------------------------
@@ -845,7 +866,7 @@ def run_config(cx, args, name, nt_total, scaling, steps, warmup, balance, with_e
         'hbm_gbs_aggregate': 2.0 * esize * units_step_all / (ms_per_step * 1e-3) / 1e9,
         'roofline': roofline, 'clocks': clocks, 'gpu_launches': keep['launches'],
         'one_off': {'locator_s': wl.t_locator, 'k1_compute_weights_s': wl.t_k1},
-        'parity': parity,
+        'parity': parity, 'series': series,
     }
     if e2e is not None:
         out['e2e'] = e2e['e2e']
@@ -874,6 +895,7 @@ def run_b200(args):
         sampler.start()
     main = run_config(cx, args, name, nt_total, scaling, args.steps, args.warmup, args.balance,
                       with_e2e=not args.no_e2e, with_cpu=not args.no_cpu, sampler=sampler)
+    outputs = {'flux_series': main.pop('series')} if rank == 0 else None
     target = None
     if world == 8 and args.workload == 'auto' and not args.no_target:
         # BASELINE's target: ORCA12 x 73 snapshots x 1024 transects on 8 GPUs, balanced (time step, panel) sharding
@@ -884,6 +906,7 @@ def run_b200(args):
         t = run_config(cx, args, 'C5', 73, 'strong', max(3, min(args.steps, args.target_steps)), 3, True,
                        with_e2e=False, with_cpu=False, sampler=tsampler)
         if rank == 0:
+            outputs['target_c5_flux_series'] = t.pop('series')
             rl = t['roofline']
             target = {'workload': t['config']['workload'], 'ms': t['ms_per_step'], 'value': t['value'], 'unit': UNIT,
                       'steps': max(3, min(args.steps, args.target_steps)), 'warmup': 3,
@@ -904,6 +927,8 @@ def run_b200(args):
         if target is not None:
             line['target_c5'] = target
         print(json.dumps(line), flush=True)
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, outputs)
     if world > 1:
         cx.dist.barrier()
         cx.dist.destroy_process_group()

@@ -25,7 +25,7 @@ import types
 import numpy
 
 REF = '/root/reference/nemoflux'
-OUT = os.environ.get('NFX_GOLDEN_OUT') or os.path.dirname(os.path.abspath(__file__))   # the test regenerates elsewhere
+OUT = os.environ.get('NFX_GOLDEN_OUT') or os.path.dirname(os.path.abspath(__file__))   # regenerate elsewhere to compare
 
 
 def _stub_modules():

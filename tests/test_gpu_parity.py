@@ -941,3 +941,28 @@ def test_many_levels_up_to_the_shared_memory_limit(gpu, oracle, dtype):
         p.fluxSeries(u, u, torch.ones(nz, dtype=torch.float64, device='cuda'), args[3], args[4])
     with pytest.raises(_lib.NemofluxGpuError, match='3000 levels'):
         gpu.edgeFluxAssemble(u, u, torch.ones(nz, dtype=torch.float64, device='cuda'), args[3], args[4])
+
+
+def test_bench_dump_outputs_is_the_timed_series(gpu, oracle, tmp_path):
+    """bench.py --dump-outputs DIR on the GPU arm: the series the last timed step returned, all time steps, equal to the
+    oracle's series to the flux bar; a second run with the same arguments writes the same bits"""
+    import subprocess
+    import sys
+    from conftest import ROOT
+    from nemoflux_b200 import synth
+    got = []
+    for run in range(2):
+        d = tmp_path / f'run{run}'
+        cmd = [sys.executable, os.path.join(ROOT, 'bench.py'), '--workload', 'tiny', '--steps', '2', '--warmup', '1',
+               '--no-e2e', '--no-cpu', '--dump-outputs', str(d)]
+        out = subprocess.run(cmd, capture_output=True, text=True, timeout=600, cwd=ROOT)
+        assert out.returncode == 0, out.stderr[-2000:]
+        assert os.listdir(d) == ['flux_series.npy']
+        got.append(numpy.load(d / 'flux_series.npy'))
+    syn = synth.make('tiny')
+    assert got[0].dtype == numpy.float64 and got[0].shape == (syn.nt, syn.ntransects)
+    assert numpy.array_equal(got[0], got[1])
+    uh = numpy.stack([syn.uv_host(t)[0] for t in range(syn.nt)])
+    vh = numpy.stack([syn.uv_host(t)[1] for t in range(syn.nt)])
+    ref = oracle.flux_series(syn.points, syn.transects, uh, vh, syn.thickness)
+    assert numpy.abs(got[0] - ref).max() <= FLUX_RTOL * numpy.abs(ref).max()

@@ -65,7 +65,7 @@ WOCE_HEADER = ('EXPOCODE 09AR9404_1    S3 (P12)\n                               
 
 def test_latlonreader_matches_reference_outputs(tmp_path):
     """golden = what the reference's LatLonReader returned for its 12 transect files; the files are rebuilt in
-    the same WOCE layout from the golden points (and the originals are parsed too where they are mounted)"""
+    the same WOCE layout from the golden points"""
     from nemoflux_b200.latlonreader import LatLonReader
     gold = json.load(open(os.path.join(GOLDEN, 'golden_summary.json')))['latlonreader']
     assert len(gold) == 12 and len(gold['S3_sta_bdep.txt']) == 50 and len(gold['atlantic/S3.txt']) == 10
@@ -79,9 +79,6 @@ def test_latlonreader_matches_reference_outputs(tmp_path):
             f.write('\n')
         got = LatLonReader(str(p)).getLonLats()
         assert got.shape == (len(pts), 2) and numpy.array_equal(got, numpy.array(pts))
-        ref = os.path.join('/root/reference/data', name)
-        if os.path.exists(ref):
-            assert numpy.array_equal(LatLonReader(ref).getLonLats(), numpy.array(pts))
     # integer-looking coordinates and lines that must be skipped
     p = tmp_path / 'odd.txt'
     p.write_text(WOCE_HEADER + '  0      0.0   63     -10  0\n  x      0.0   1 2\n  0      5   63 -10\n  0  0.0 -46.0  164 0')
@@ -187,11 +184,14 @@ def test_datagen_mesh_mask(tmp_path):
     assert not os.path.exists(prefix + 'nmesh_mask.nc')
 
 
-def test_hdf5_reader_on_the_reference_grid_file():
-    """nemoflux's real-data files are NetCDF-4 (HDF5); the reference ships one, data/sa/T.nc (README.md:118ff).  The
-    package's own reader (h5lite via ncio: v2 object headers, dense links in a fractal heap, contiguous float32
-    data, dense attributes) must give the arrays committed as tests/golden/sa_T_grid.npz, and those must be a
-    sane NEMO T grid: vertices SW, SE, NE, NW, neighbours sharing their nodes, S3_sa.txt inside"""
+def test_hdf5_reader_on_the_reference_grid_file(tmp_path):
+    """nemoflux's real-data files are NetCDF-4 (HDF5); the reference ships one, data/sa/T.nc (README.md:118ff), whose
+    arrays and dimension names are committed as tests/golden/sa_T_grid.npz.  Those must be a sane NEMO T grid:
+    vertices SW, SE, NE, NW, neighbours sharing their nodes, S3_sa.txt inside.  A NetCDF-4 file with the same
+    variables, dimension scales (_Netcdf4Dimid / _Netcdf4Coordinates, dimensions without a variable) and attributes
+    is written from them by tests/h5build.py (version-2 object headers, contiguous float32 data); the package's own
+    reader (h5lite via ncio) must give back the committed arrays, and the reference's data-preparation tool must cut it"""
+    import h5build
     from nemoflux_b200 import ncio
     g = numpy.load(os.path.join(GOLDEN, 'sa_T_grid.npz'))
     lon, lat, zb = g['bounds_lon'], g['bounds_lat'], g['deptht_bounds']
@@ -202,9 +202,21 @@ def test_hdf5_reader_on_the_reference_grid_file():
     assert (zb[1:, 0] == zb[:-1, 1]).all() and zb[0, 0] == 0.0 and 5000. < zb[-1, 1] < 6500.     # 75 NEMO levels
     for x, y in ((16., -40.4), (28., -34.5), (31., -28.5), (36., -30.5)):                       # data/sa/S3_sa.txt:5-8
         assert lon.min() < x < lon.max() and lat.min() < y < lat.max()
-    path = '/root/reference/data/sa/T.nc'
-    if not os.path.exists(path):
-        pytest.skip('the reference tree is not mounted here')
+    dims = {str(name): str(d).split('|') for name, d in g['dims']}
+    sizes = {}
+    for name, dn in sorted(dims.items()):
+        sizes.update(zip(dn, g[name].shape))
+    dimid = {dn: numpy.int32(i) for i, dn in enumerate(sizes)}
+    variables = {dn: dict(data=numpy.zeros(n, numpy.float32),
+                          attrs={'CLASS': 'DIMENSION_SCALE', '_Netcdf4Dimid': dimid[dn],
+                                 'NAME': f'This is a netCDF dimension but not a netCDF variable.{n:10d}'})
+                 for dn, n in sizes.items() if dn not in dims}
+    for name, dn in dims.items():
+        variables[name] = dict(data=g[name], attrs={'_Netcdf4Coordinates': numpy.array([dimid[d] for d in dn])})
+    variables['deptht']['attrs'] = {'CLASS': 'DIMENSION_SCALE', 'NAME': 'deptht', '_Netcdf4Dimid': dimid['deptht'],
+                                    'standard_name': 'depth', 'units': 'm', 'bounds': 'deptht_bounds'}
+    path = str(tmp_path / 'T.nc')
+    h5build.write_new(path, variables)
     with ncio.open_dataset(path) as nc:
         assert set(nc.variables) == {'bounds_lon', 'bounds_lat', 'deptht', 'deptht_bounds'}
         assert nc['bounds_lon'].dimensions == ('y', 'x', 'nvertex') and nc['deptht_bounds'].dimensions == ('deptht', 'axis_nbounds')
@@ -212,16 +224,15 @@ def test_hdf5_reader_on_the_reference_grid_file():
         for name in ('bounds_lon', 'bounds_lat', 'deptht_bounds', 'deptht'):
             assert numpy.array_equal(nc[name][:], g[name]), name
         assert numpy.array_equal(nc['bounds_lat'][3, 5:7], g['bounds_lat'][3, 5:7])             # partial reads (memmap)
-    # the reference's data-preparation tool on its own file (subsetNEMO.py:6-93): NetCDF-4 in, classic out
-    import tempfile
+    # the reference's data-preparation tool on its grid file (subsetNEMO.py:6-93): NetCDF-4 in, classic out
     from nemoflux_b200 import subsetnemo
-    with tempfile.TemporaryDirectory() as tmp:
-        subsetnemo.subset(tfile=path, outputdir=tmp, jmin=10, jmax=40, imin=20, imax=90, verbose=False)
-        with ncio.open_dataset(os.path.join(tmp, 'T.nc')) as nc:
-            assert nc['bounds_lon'].dimensions == ('y', 'x', 'nvertex') and nc['bounds_lon'].shape == (30, 70, 4)
-            assert numpy.array_equal(nc['bounds_lon'][:], g['bounds_lon'][10:40, 20:90])
-            assert numpy.array_equal(nc['bounds_lat'][:], g['bounds_lat'][10:40, 20:90])
-            assert numpy.array_equal(nc['deptht_bounds'][:], g['deptht_bounds']) and nc['deptht'].units == 'm'
+    out = tmp_path / 'subset'
+    subsetnemo.subset(tfile=path, outputdir=str(out), jmin=10, jmax=40, imin=20, imax=90, verbose=False)
+    with ncio.open_dataset(str(out / 'T.nc')) as nc:
+        assert nc['bounds_lon'].dimensions == ('y', 'x', 'nvertex') and nc['bounds_lon'].shape == (30, 70, 4)
+        assert numpy.array_equal(nc['bounds_lon'][:], g['bounds_lon'][10:40, 20:90])
+        assert numpy.array_equal(nc['bounds_lat'][:], g['bounds_lat'][10:40, 20:90])
+        assert numpy.array_equal(nc['deptht_bounds'][:], g['deptht_bounds']) and nc['deptht'].units == 'm'
 
 
 def test_hdf5_chunked_deflate_shuffle_decoding():
@@ -506,6 +517,31 @@ def test_bench_reference_arm_contract():
     env = dict(os.environ, RANK='1', WORLD_SIZE='2', LOCAL_RANK='1')
     out = subprocess.run(cmd, capture_output=True, text=True, timeout=300, cwd=ROOT, env=env)
     assert out.returncode == 0 and not [ln for ln in out.stdout.splitlines() if ln.startswith('{')]
+
+
+def test_bench_dump_outputs_reference_arm(oracle, tmp_path):
+    """bench.py --dump-outputs DIR writes the flux series of the last timed step as float64 .npy: the same file from
+    run to run whatever the number of steps, equal to the oracle's series of the sampled time steps; --steps 0 is
+    refused instead of timing nothing"""
+    from nemoflux_b200 import synth
+    cmd = [sys.executable, os.path.join(ROOT, 'bench.py'), '--impl', 'reference', '--workload', 'tiny', '--warmup', '0',
+           '--cpu-steps', '3']
+    got = []
+    for steps in (1, 2):
+        d = tmp_path / f'steps{steps}'
+        out = subprocess.run(cmd + ['--steps', str(steps), '--dump-outputs', str(d)], capture_output=True, text=True,
+                             timeout=300, cwd=ROOT)
+        assert out.returncode == 0, out.stderr[-2000:]
+        assert os.listdir(d) == ['flux_series.npy']
+        got.append(numpy.load(d / 'flux_series.npy'))
+    assert got[0].dtype == numpy.float64 and got[0].shape == (3, 12) and numpy.array_equal(got[0], got[1])
+    syn = synth.make('tiny')
+    uh = numpy.stack([syn.uv_host(t)[0] for t in range(3)])
+    vh = numpy.stack([syn.uv_host(t)[1] for t in range(3)])
+    ref = oracle.flux_series(syn.points, syn.transects, uh, vh, syn.thickness)
+    assert numpy.abs(got[0] - ref).max() <= 1e-12 * numpy.abs(ref).max()
+    out = subprocess.run(cmd + ['--steps', '0'], capture_output=True, text=True, timeout=300, cwd=ROOT)
+    assert out.returncode != 0 and '--steps must be at least 1' in out.stderr
 
 
 def test_f32_bit_shuffle_conversion_in_emulation():
