@@ -74,6 +74,11 @@ extern "C" {
                                       (0 = automatic: one-panel grids the batches the resident CTAs span + 1, else 1) */
 
 #define NFX_OPT_RING_MAX_MB 16      /* fused pass: upper bound of the whole edge-flux ring in MB (0 = default 24) */
+#define NFX_OPT_SPARSE_COLUMNS 17   /* fused pass: 0 = K2 reads every column of u, v; 2 = only the groups of columns
+                                       whose edge fluxes the transects read (nfx_pli_get_column_groups); 1 (default) =
+                                       sparse while those groups are less than 80 % of the grid's.  Same series bits. */
+#define NFX_OPT_LAST_SERIES_SPARSE 18  /* READ ONLY: 1 = the last nfx_flux_series* call took the sparse fused pass,
+                                          0 = the dense fused pass or two launches, -1 = none yet */
 
 typedef struct nfx_grid nfx_grid;
 typedef struct nfx_pli nfx_pli;
@@ -210,6 +215,17 @@ int nfx_pli_series_status(nfx_pli** self, void* stream, int* status);
  * arrays, 256-bit evict-first loads, K2's arithmetic, no stores): best of `reps` launches over the caller's device
  * buffer (32-byte aligned, >= 9.3 GB, contents arbitrary) in GB/s.  Measurement aid for bench.py's roofline. */
 int nfx_probe_read_bandwidth(const void* buf, int64_t nbytes, int reps, double* gbs, void* stream);
+/* The same walk over a list of column groups only (the access pattern of the sparse fused pass): groups device
+ * (ngroups) int32, ascending indices of 256-bit vectors (4 doubles) of the probe's 362 x 332 plane, each < 30046.
+ * *gbs counts the bytes of the listed groups only. */
+int nfx_probe_read_bandwidth_groups(const void* buf, int64_t nbytes, const int32_t* groups, int64_t ngroups, int reps,
+                                    double* gbs, void* stream);
+/* Column groups of the sparse fused pass for uo/vo of `dtype` (its panel size), summation `order` and `vec` columns
+ * per group (1, 2, 4 or 8): per panel q, groups[panel_offsets[q] .. panel_offsets[q+1]) are the ascending panel-local
+ * group indices g (columns [g*vec, g*vec+vec) of the panel) in which the transects read eU or eV.  Host outputs, each
+ * may be NULL: panel_offsets (npanels + 1), groups (*ngroups). */
+int nfx_pli_get_column_groups(nfx_pli** self, int dtype, int order, int vec, int64_t* panel_offsets, int32_t* groups,
+                              int64_t* ngroups);
 /* Finer-than-time-step sharding over GPUs.  The fused pass works on batches b = t*npanels + q (time step t of
  * the nt resident ones, panel q of npanels panels of panel_cells consecutive cells); this call runs only the
  * batches [batch_begin, batch_end) and returns PARTIAL sums in series (nt, ntransects): complete for the time

@@ -24,6 +24,8 @@ NFX_OPT_FUSED_ORDER = 9
 NFX_OPT_FUSED_F64_CTAS = 10
 NFX_OPT_FUSED_K3_LAG = 15
 NFX_OPT_RING_MAX_MB = 16
+NFX_OPT_SPARSE_COLUMNS = 17
+NFX_OPT_LAST_SERIES_SPARSE = 18
 
 c_i64 = ctypes.c_int64
 c_int = ctypes.c_int
@@ -85,6 +87,8 @@ SIGNATURES = {
     'nfx_pli_get_num_panels_dtype': [P(c_vp), c_int, P(c_int), P(c_i64)],
     'nfx_pli_series_status': [P(c_vp), c_vp, P(c_int)],
     'nfx_probe_read_bandwidth': [c_vp, c_i64, c_int, P(c_dbl), c_vp],
+    'nfx_probe_read_bandwidth_groups': [c_vp, c_i64, c_vp, c_i64, c_int, P(c_dbl), c_vp],
+    'nfx_pli_get_column_groups': [P(c_vp), c_int, c_int, c_int, c_vp, c_vp, P(c_i64)],
     'nfx_h5_decode_chunks': [c_vp, c_i64, c_i64, c_vp, c_vp, c_int, c_int, c_int, c_vp, c_vp, c_vp, c_int, c_vp, c_vp, c_vp],
     'nfx_flux_series_range': [P(c_vp), c_vp, c_vp, c_int, c_vp, c_vp, c_vp, c_int, c_int, c_i64, c_int, c_dbl, c_int,
                               c_i64, c_i64, c_vp, c_vp],

@@ -290,6 +290,11 @@ int nfx_set_option(int option, int value) {
                 NFX_REQUIRE(value >= 0 && value <= 2, "NFX_OPT_FAST_SERIES must be 0, 1 or 2");
                 g_fast_series = value;
                 break;
+            case NFX_OPT_SPARSE_COLUMNS:
+                NFX_REQUIRE(value >= 0 && value <= 2, "NFX_OPT_SPARSE_COLUMNS must be 0, 1 or 2");
+                g_sparse_columns = value;
+                break;
+            case NFX_OPT_LAST_SERIES_SPARSE: throw Error(NFX_E_INVALID, "NFX_OPT_LAST_SERIES_SPARSE is read only");
             case NFX_OPT_RING_SLOT_MB:
                 NFX_REQUIRE(value >= 0 && value <= 64, "ring slot must be 1..64 MB (0 = automatic)");
                 g_slot_bytes = (int64_t)value << 20;
@@ -315,6 +320,8 @@ int nfx_get_option(int option, int* value) {
             case NFX_OPT_LAST_SERIES_PATH: *value = g_last_series_fused; break;
             case NFX_OPT_FAST_SERIES: *value = g_fast_series; break;
             case NFX_OPT_RING_SLOT_MB: *value = (int)(g_slot_bytes >> 20); break;
+            case NFX_OPT_SPARSE_COLUMNS: *value = g_sparse_columns; break;
+            case NFX_OPT_LAST_SERIES_SPARSE: *value = g_last_series_sparse; break;
             default: throw Error(NFX_E_INVALID, "unknown option");
         }
     });
@@ -725,6 +732,7 @@ int nfx_flux_series_e3(nfx_pli** self, const void* u, const void* v, const void*
         NFX_REQUIRE(e3_nt == 1 || e3_nt == nt, "e3u/e3v must hold 1 (time-invariant) or nt time steps");
         const int64_t e3_tstride = e3_nt == 1 ? 0 : (int64_t)nz * ld;
         g_last_series_fused = 0;
+        g_last_series_sparse = 0;
         if (eflux == nullptr && use_fused_e3(p, dtype, u, v, e3u, e3v, e3_tstride, ld)) {
             g_last_series_fused = 1;
             flux_series_fast(p, u, v, dtype, nullptr, arc1, arc2, nt, nz, ld, sverdrup, fill, order, series,
@@ -781,6 +789,7 @@ int nfx_flux_series_ld(nfx_pli** self, const void* u, const void* v, int dtype, 
         const int64_t ncell = p.grid->ncell;
         NFX_REQUIRE(ld >= ncell, "ld must be >= the number of cells");
         g_last_series_fused = 0;
+        g_last_series_sparse = 0;
         if (eflux == nullptr && use_fused(p, dtype, u, v, ld)) {
             g_last_series_fused = 1;
             flux_series_fast(p, u, v, dtype, thickness, arc1, arc2, nt, nz, ld, sverdrup, fill, order, series,
@@ -832,6 +841,40 @@ int nfx_probe_read_bandwidth(const void* buf, int64_t nbytes, int reps, double* 
         DevBuf<double> sink;
         sink.alloc(1);
         *gbs = probe_read_bandwidth(buf, nbytes, reps, sink.p, (cudaStream_t)stream);
+    });
+}
+
+int nfx_probe_read_bandwidth_groups(const void* buf, int64_t nbytes, const int32_t* groups, int64_t ngroups, int reps,
+                                    double* gbs, void* stream) {
+    return guarded([&] {
+        int dev;
+        require_gpu(&dev);
+        NFX_REQUIRE(buf && groups && gbs, "NULL pointer");
+        DevBuf<double> sink;
+        sink.alloc(1);
+        *gbs = probe_read_bandwidth_groups(buf, nbytes, groups, ngroups, reps, sink.p, (cudaStream_t)stream);
+    });
+}
+
+int nfx_pli_get_column_groups(nfx_pli** self, int dtype, int order, int vec, int64_t* panel_offsets, int32_t* groups,
+                              int64_t* ngroups) {
+    return guarded([&] {
+        NFX_REQUIRE(self && *self, "NULL handle");
+        NFX_REQUIRE(dtype == NFX_F64 || dtype == NFX_F32, "dtype must be NFX_F64 or NFX_F32");
+        NFX_REQUIRE(vec == 1 || vec == 2 || vec == 4 || vec == 8, "vec must be 1, 2, 4 or 8");
+        PliDev& p = (*self)->d;
+        NFX_REQUIRE(p.grid && p.grid->ncell > 0, "setGrid / setPoints was not called");
+        NFX_REQUIRE(order == NFX_ORDER_LIST || order == NFX_ORDER_MAP, "order must be NFX_ORDER_LIST or NFX_ORDER_MAP");
+        NFX_REQUIRE(p.csr[order][0].rowptr.p != nullptr, "computeWeights was not called");
+        DeviceGuard g(p.grid->device);
+        const int64_t panel = fused_panel_cells(p.grid->ncell, dtype);
+        PanelPlan& pl = p.plan[order];
+        if (!pl.built || pl.panel_cells != panel) build_panel_plan(p, order, panel, nullptr);
+        if (pl.grp_vec != vec) build_column_groups(pl, p.grid->ncell, p.ntransects, vec, nullptr);
+        NFX_CUDA(cudaStreamSynchronize(nullptr));
+        if (ngroups) *ngroups = pl.ngroups;
+        d2h(panel_offsets, pl.grp_ptr.p, (size_t)pl.npanels + 1);
+        d2h(groups, pl.grp.p, (size_t)pl.ngroups);
     });
 }
 
@@ -1021,6 +1064,7 @@ static void flux_series_host_impl(nfx_pli** self, const void* u, const void* v, 
     NFX_CUDA(cudaStreamSynchronize(ks));
     NFX_CUDA(cudaStreamSynchronize(cs));
     g_last_series_fused = fused ? 1 : 0;
+    if (!fused) g_last_series_sparse = 0;
     if (fused && fused_error_flag(p, ks) != 0)
         throw Error(NFX_E_INTERNAL, "fused K2+K3 pass aborted (a bounded wait overflowed)");
 }

@@ -146,6 +146,15 @@ struct PanelPlan {
     DevBuf<int64_t> tr_ptr;       // (M + 1) per transect: range in tr_sr
     DevBuf<int64_t> tr_sr;        // (nsr) sub-row ids of every transect, ascending
     std::vector<int64_t> h_panel_sr;   // host copy of panel_sr
+    // Column groups: per panel, ascending, the panel-local indices g of the groups of grp_vec columns [g*vec, g*vec+vec)
+    // in which idx reads u or v.  The K2 tiles of the sparse fused pass load only these (built for the vector width
+    // of the pass, see build_column_groups; grp_vec = 0: not built for this plan yet).
+    int grp_vec = 0;
+    int64_t ngroups = 0;          // groups in the list, all panels
+    int64_t ngroups_all = 0;      // groups of grp_vec columns the panels hold (the dense pass loads all of them)
+    int max_grp_per_panel = 0;
+    DevBuf<int32_t> grp;
+    DevBuf<int64_t> grp_ptr;      // (npanels + 1) offsets into grp
 };
 constexpr int64_t kSubRow = 4096;
 
@@ -237,9 +246,10 @@ void rows_integrate(const int64_t* rowptr, const int32_t* idx, const double* w, 
 void reduce_subrows(const double* partial, int nt, int64_t nsr, const int64_t* tr_ptr, const int64_t* tr_sr,
                     int ntransects, double* series, cudaStream_t s);
 void build_panel_plan(PliDev& p, int order, int64_t panel_cells, cudaStream_t s);
+void build_column_groups(PanelPlan& pl, int64_t ncell, int ntransects, int vec, cudaStream_t s);
 
 // K2+K3 fused persistent pass (nfx_k23_fused.cu)
-void flux_series_fused(PliDev& p, const PanelPlan& pl, const void* u, const void* v, int dtype, const double* thickness,
+void flux_series_fused(PliDev& p, PanelPlan& pl, const void* u, const void* v, int dtype, const double* thickness,
                        const double* arc1, const double* arc2, int nt, int nz, int64_t ld, int sverdrup, double fill,
                        int64_t batch_begin, int64_t batch_end, double* out, cudaStream_t s, const void* e3u = nullptr,
                        const void* e3v = nullptr, int64_t e3_tstride = 0);
@@ -257,6 +267,10 @@ extern int g_fused_order;
 extern int g_fused_k3_lag;
 extern int g_fused_ring_max_mb;
 extern int g_fused_f64_ctas;
+extern int g_sparse_columns;
+extern int g_last_series_sparse;
+double probe_read_bandwidth_groups(const void* buf, int64_t nbytes, const int32_t* groups, int64_t ngroups, int reps,
+                                   double* sink, cudaStream_t s);   // nfx_probe.cu
 int k3_group_for(int64_t nnz, int64_t nrows);
 
 }  // namespace nfx

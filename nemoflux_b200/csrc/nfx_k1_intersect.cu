@@ -758,7 +758,65 @@ __global__ void k_panel_rows(const int64_t* __restrict__ rowptr, const int32_t* 
         for (int q = lane; q < npanels; q += 32) counts[(int64_t)q * ntransects + m] = pos[q];
 }
 
+// ---- column groups of the sparse fused pass: panel q holds the groups [q * gpp, q * gpp + gpp) of vec columns ------
+__global__ void k_group_flags(const int64_t* __restrict__ rowptr, const int32_t* __restrict__ idx, int ntransects,
+                              int64_t ncell, int64_t panel_cells, int vec, int64_t gpp, int64_t* __restrict__ flags) {
+    const int q = blockIdx.y;
+    const int64_t pc = min(panel_cells, ncell - (int64_t)q * panel_cells);
+    const int64_t e1 = rowptr[(int64_t)(q + 1) * ntransects];
+    for (int64_t n = rowptr[(int64_t)q * ntransects] + (int64_t)blockIdx.x * blockDim.x + threadIdx.x; n < e1;
+         n += (int64_t)gridDim.x * blockDim.x) {
+        const int64_t f = idx[n];   // [eU | eV] of the panel: u column f, or v column f - pc
+        flags[q * gpp + (f < pc ? f : f - pc) / vec] = 1;
+    }
+}
+
+// grp[pos[i]] = panel-local index of every flagged group i, grp_ptr[q] = position of the first group of panel q
+__global__ void k_group_compact(const int64_t* __restrict__ flags, const int64_t* __restrict__ pos, int64_t ng,
+                                int64_t gpp, int npanels, int32_t* __restrict__ grp, int64_t* __restrict__ grp_ptr) {
+    const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i < ng && flags[i]) grp[pos[i]] = (int32_t)(i % gpp);
+    if (i <= npanels) grp_ptr[i] = pos[min(i * gpp, ng)];
+}
+
 }  // namespace
+
+// A one-off per (plan, vector width): runs on the first fused pass after computeWeights, outside any time-step loop.
+void build_column_groups(PanelPlan& pl, int64_t ncell, int ntransects, int vec, cudaStream_t s) {
+    NFX_REQUIRE(pl.built, "column groups: the panel plan is not built");
+    NFX_REQUIRE(pl.npanels == 1 || pl.panel_cells % vec == 0, "column groups: a group would straddle two panels");
+    const int64_t gpp = (pl.panel_cells + vec - 1) / vec;
+    const int64_t ng = (ncell + vec - 1) / vec;   // = (npanels - 1) * gpp + the groups of the last panel
+    DevBuf<int64_t> flags, pos, tmp;
+    flags.alloc((size_t)ng);
+    pos.alloc((size_t)ng + 1);
+    NFX_CUDA(cudaMemsetAsync(flags.p, 0, sizeof(int64_t) * ng, s));
+    if (pl.nnz > 0) {
+        const int64_t per_panel = std::max<int64_t>(1, pl.nnz / pl.npanels);
+        const dim3 grid(nblk(std::min<int64_t>(per_panel, (int64_t)256 * 1024), 256), (unsigned)pl.npanels);
+        k_group_flags<<<grid, 256, 0, s>>>(pl.rowptr.p, pl.idx.p, ntransects, ncell, pl.panel_cells, vec, gpp, flags.p);
+        count_launch();
+    }
+    exclusive_scan(flags.p, pos.p, ng, tmp, s);
+    int64_t total = 0;
+    NFX_CUDA(cudaMemcpyAsync(&total, pos.p + ng, sizeof(int64_t), cudaMemcpyDeviceToHost, s));
+    NFX_CUDA(cudaStreamSynchronize(s));
+    pl.grp.ensure((size_t)std::max<int64_t>(total, 1));
+    pl.grp_ptr.ensure((size_t)pl.npanels + 1);
+    k_group_compact<<<nblk(std::max<int64_t>(ng, pl.npanels + 1), 256), 256, 0, s>>>(flags.p, pos.p, ng, gpp, pl.npanels,
+                                                                                    pl.grp.p, pl.grp_ptr.p);
+    count_launch();
+    NFX_CUDA(cudaGetLastError());
+    std::vector<int64_t> h_ptr((size_t)pl.npanels + 1);
+    NFX_CUDA(cudaMemcpyAsync(h_ptr.data(), pl.grp_ptr.p, sizeof(int64_t) * h_ptr.size(), cudaMemcpyDeviceToHost, s));
+    NFX_CUDA(cudaStreamSynchronize(s));   // before the scratch buffers go
+    int64_t mx = 0;
+    for (int q = 0; q < pl.npanels; ++q) mx = std::max(mx, h_ptr[q + 1] - h_ptr[q]);
+    pl.ngroups = total;
+    pl.ngroups_all = ng;
+    pl.max_grp_per_panel = (int)mx;
+    pl.grp_vec = vec;
+}
 
 void build_panel_plan(PliDev& p, int order, int64_t panel_cells, cudaStream_t s) {
     NFX_REQUIRE(p.has_compact, "the flux path needs nfx_grid_set_cgrid_shape before computeWeights");
@@ -770,6 +828,7 @@ void build_panel_plan(PliDev& p, int order, int64_t panel_cells, cudaStream_t s)
     NFX_REQUIRE(npanels >= 1 && npanels <= kMaxPanels, "panel plan: too many panels");
     pl.panel_cells = panel_cells;
     pl.npanels = npanels;
+    pl.grp_vec = 0;
     const int64_t nrows = (int64_t)npanels * M;
     pl.rowptr.ensure((size_t)nrows + 1);
     if (M == 0 || c.nnz == 0) {

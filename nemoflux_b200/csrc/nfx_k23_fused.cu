@@ -33,6 +33,10 @@ int g_fused_ring_max_mb = 0;  // NFX_OPT_RING_MAX_MB: upper bound of the whole r
 int g_fused_k3_lag = 0;      // NFX_OPT_FUSED_K3_LAG: 0 = automatic, else the lag of the K3 items in batches
 int g_fused_order = 3;       // NFX_OPT_FUSED_ORDER: bit 0 = visit the batches panel-major, bit 1 = K3 gathers unrolled x8
                              // (same-box A/B, profiles/r1_fused_order_ab.md: -3 % and -1 % time on multi-panel grids)
+int g_sparse_columns = 1;    // NFX_OPT_SPARSE_COLUMNS: 0 = dense, 1 = automatic, 2 = always sparse
+int g_last_series_sparse = -1;   // NFX_OPT_LAST_SERIES_SPARSE (read only)
+// automatic mode takes the sparse pass while its groups are less than this share of the panels' groups
+constexpr double kSparseMaxShare = 0.8;
 
 namespace {
 
@@ -64,6 +68,8 @@ struct FusedArgs {
     int64_t ncell, ld, panel, slot_elems;   // ld = cells per level plane in memory (>= ncell)
     int nt, nz, ntransects, npanels, nbatches, ntiles, nk3, ring_slots;
     const int* batch_map;   // (nbatches) global batch index t * npanels + q of the b-th batch visited
+    const int32_t* grp;     // sparse pass: PanelPlan::grp (column groups of VEC the K2 tiles load), nullptr = dense
+    const int64_t* grp_ptr;
     int k3_lag;             // the K3 items of batch b - k3_lag are queued behind the K2 tiles of batch b
     int k3_unroll8;
     double scale, fill;
@@ -166,7 +172,11 @@ k23_fused(const FusedArgs a) {
             const int q = gb - (int)t * a.npanels;
             const int64_t pc0 = (int64_t)q * a.panel;
             const int64_t pc = min(a.panel, a.ncell - pc0);
-            const int64_t cl = ((int64_t)r * kFusedBlock + threadIdx.x) * VEC;   // column inside the panel
+            int64_t cl = ((int64_t)r * kFusedBlock + threadIdx.x) * VEC;   // column inside the panel
+            if (a.grp) {   // sparse: the r-th 256 groups of the panel's list; a tile past its end loads nothing
+                const int64_t gi = a.grp_ptr[q] + (int64_t)r * kFusedBlock + threadIdx.x;
+                cl = gi < a.grp_ptr[q + 1] ? (int64_t)a.grp[gi] * VEC : pc;
+            }
             if (cl < pc) {
                 const int64_t c = pc0 + cl;
                 const T* pu = u + t * a.nz * a.ld + c;
@@ -422,7 +432,7 @@ int fused_tile_columns(int dtype, const void* u, const void* v, int64_t ncell, i
     return 1;
 }
 
-void flux_series_fused(PliDev& p, const PanelPlan& pl, const void* u, const void* v, int dtype, const double* thickness,
+void flux_series_fused(PliDev& p, PanelPlan& pl, const void* u, const void* v, int dtype, const double* thickness,
                        const double* arc1, const double* arc2, int nt, int nz, int64_t ld, int sverdrup, double fill,
                        int64_t batch_begin, int64_t batch_end, double* out, cudaStream_t s, const void* e3u,
                        const void* e3v, int64_t e3_tstride) {
@@ -465,8 +475,19 @@ void flux_series_fused(PliDev& p, const PanelPlan& pl, const void* u, const void
                 "fused pass: bad batch range");
     a.nbatches = (int)(batch_end - batch_begin);
     a.k3_unroll8 = (g_fused_order >> 1) & 1;
+    // sparse pass: the K2 tiles walk the plan's column groups, i.e. only the vectors of u, v whose edge fluxes a K3 item
+    // reads.  Every edge flux K3 reads is computed as in the dense pass: the series is the same bit for bit.
+    bool sparse = false;
+    if (g_sparse_columns != 0) {
+        if (pl.grp_vec != vec) build_column_groups(pl, ncell, M, vec, s);
+        sparse = g_sparse_columns == 2 || (double)pl.ngroups < kSparseMaxShare * (double)pl.ngroups_all;
+    }
+    g_last_series_sparse = sparse ? 1 : 0;
+    a.grp = sparse ? pl.grp.p : nullptr;
+    a.grp_ptr = sparse ? pl.grp_ptr.p : nullptr;
     const int64_t item_cols = (int64_t)kFusedBlock * vec;
-    a.ntiles = (int)((std::min(pl.panel_cells, ncell) + item_cols - 1) / item_cols);
+    a.ntiles = sparse ? std::max(1, (pl.max_grp_per_panel + kFusedBlock - 1) / kFusedBlock)
+                      : (int)((std::min(pl.panel_cells, ncell) + item_cols - 1) / item_cols);
     a.nk3 = std::max(1, (pl.max_sr_per_panel + kWarps - 1) / kWarps);
     a.scale = 6371000.0 / 1.e6;
     a.fill = fill;

@@ -5,6 +5,8 @@
 // k2_edgeflux_ldg / k23_fused walk uo and vo -- one CTA per tile of columns, nz level planes, two arrays, 256-bit
 // evict-first loads, 5 levels of both arrays in flight, K2's multiply-add per value -- and stores nothing, so
 // bench.py can quote the pass against the ceiling of the box it runs on instead of a constant from another machine.
+// nfx_probe_read_bandwidth_groups does the same walk over a list of 256-bit column groups only: the access pattern of
+// the sparse fused pass, which is judged against that ceiling rather than the dense one.
 #include "nfx_common.cuh"
 #include "nfx_stream_ops.cuh"
 
@@ -16,10 +18,14 @@ using namespace dev;
 constexpr int kProbeBlock = 256;
 constexpr int kProbeUnroll = 5;
 
+// GROUPS: thread i reads the 256-bit vector groups[i] of every plane instead of vector i (the sparse fused pass)
+template <bool GROUPS>
 __global__ void __launch_bounds__(kProbeBlock, 3)
-k_probe_read(const double4x* __restrict__ a, const double4x* __restrict__ b, int64_t plane4, int nz, double* sink) {
-    const int64_t c = (int64_t)blockIdx.x * kProbeBlock + threadIdx.x;
-    if (c >= plane4) return;
+k_probe_read(const double4x* __restrict__ a, const double4x* __restrict__ b, int64_t plane4, const int32_t* groups,
+             int64_t nwalk, int nz, double* sink) {
+    const int64_t i = (int64_t)blockIdx.x * kProbeBlock + threadIdx.x;
+    if (i >= nwalk) return;
+    const int64_t c = GROUPS ? (int64_t)groups[i] : i;
     const double4x* pa = a + (int64_t)blockIdx.y * nz * plane4 + c;
     const double4x* pb = b + (int64_t)blockIdx.y * nz * plane4 + c;
     double s[8] = {0, 0, 0, 0, 0, 0, 0, 0};
@@ -55,34 +61,41 @@ k_probe_read(const double4x* __restrict__ a, const double4x* __restrict__ b, int
 }  // namespace
 
 // buf: device buffer of nbytes (32-byte aligned, contents arbitrary), treated as two arrays of (nt, 75, plane)
-// doubles with the ORCA1 plane of 120 184 cells; returns the best of `reps` launches in GB/s
-double probe_read_bandwidth(const void* buf, int64_t nbytes, int reps, double* sink, cudaStream_t s) {
+// doubles with the ORCA1 plane of 120 184 cells; walks every vector of a plane, or only groups[0 .. ngroups) when
+// groups != nullptr; returns the best of `reps` launches in GB/s of the bytes walked
+static double probe_walk(const void* buf, int64_t nbytes, const int32_t* groups, int64_t ngroups, int reps, double* sink,
+                         cudaStream_t s) {
     NFX_REQUIRE(buf && (((uintptr_t)buf) & 31) == 0, "probe: the buffer must be 32-byte aligned");
     const int64_t plane4 = 30046;   // 362 x 332 cells / 4
     const int nz = 75;
     const int64_t step_bytes = 32 * plane4 * nz;
     const int64_t nt = (nbytes / 2) / step_bytes;
     NFX_REQUIRE(nt >= 64, "probe: the buffer must hold at least 9.3 GB (64 time steps of two arrays)");
+    NFX_REQUIRE(!groups || (ngroups > 0 && ngroups <= plane4), "probe: 1 .. 30046 groups");
     const int64_t nt_use = std::min<int64_t>(nt, 65535);
+    const int64_t nwalk = groups ? ngroups : plane4;
     const double4x* a = reinterpret_cast<const double4x*>(buf);
     const double4x* b = a + nt_use * nz * plane4;
-    const dim3 grid((unsigned)((plane4 + kProbeBlock - 1) / kProbeBlock), (unsigned)nt_use);
+    const dim3 grid((unsigned)((nwalk + kProbeBlock - 1) / kProbeBlock), (unsigned)nt_use);
+    auto launch = [&] {
+        if (groups) k_probe_read<true><<<grid, kProbeBlock, 0, s>>>(a, b, plane4, groups, nwalk, nz, sink);
+        else k_probe_read<false><<<grid, kProbeBlock, 0, s>>>(a, b, plane4, nullptr, nwalk, nz, sink);
+        count_launch();
+    };
     cudaEvent_t e0, e1;
     NFX_CUDA(cudaEventCreate(&e0));
     NFX_CUDA(cudaEventCreate(&e1));
     double best = 0.0;
     try {
-        k_probe_read<<<grid, kProbeBlock, 0, s>>>(a, b, plane4, nz, sink);   // warm-up
-        count_launch();
+        launch();   // warm-up
         for (int r = 0; r < std::max(reps, 1); ++r) {
             NFX_CUDA(cudaEventRecord(e0, s));
-            k_probe_read<<<grid, kProbeBlock, 0, s>>>(a, b, plane4, nz, sink);
-            count_launch();
+            launch();
             NFX_CUDA(cudaEventRecord(e1, s));
             NFX_CUDA(cudaEventSynchronize(e1));
             float ms = 0.f;
             NFX_CUDA(cudaEventElapsedTime(&ms, e0, e1));
-            best = std::max(best, 2.0 * (double)nt_use * (double)step_bytes / (ms * 1e-3) / 1e9);
+            best = std::max(best, 2.0 * (double)nt_use * 32.0 * nz * (double)nwalk / (ms * 1e-3) / 1e9);
         }
         NFX_CUDA(cudaGetLastError());
     } catch (...) {
@@ -93,6 +106,16 @@ double probe_read_bandwidth(const void* buf, int64_t nbytes, int reps, double* s
     cudaEventDestroy(e0);
     cudaEventDestroy(e1);
     return best;
+}
+
+double probe_read_bandwidth(const void* buf, int64_t nbytes, int reps, double* sink, cudaStream_t s) {
+    return probe_walk(buf, nbytes, nullptr, 0, reps, sink, s);
+}
+
+double probe_read_bandwidth_groups(const void* buf, int64_t nbytes, const int32_t* groups, int64_t ngroups, int reps,
+                                   double* sink, cudaStream_t s) {
+    NFX_REQUIRE(groups, "probe: NULL group list");
+    return probe_walk(buf, nbytes, groups, ngroups, reps, sink, s);
 }
 
 }  // namespace nfx

@@ -251,6 +251,21 @@ class PolylineIntegral(object):
         _lib.call('nfx_pli_get_num_panels_dtype', ctypes.byref(self._h), code, ctypes.byref(n), ctypes.byref(pc))
         return n.value, pc.value
 
+    def getColumnGroups(self, dtype='float64', order='map', vec=4):
+        """(panel_offsets (npanels+1), groups) int64/int32 numpy arrays: the column groups the sparse fused pass loads for
+        uo/vo of `dtype` -- per panel q, groups[panel_offsets[q]:panel_offsets[q+1]] ascending, group g = columns
+        [g*vec, g*vec+vec) of the panel in which a transect reads eU or eV"""
+        code = _lib.NFX_F32 if str(dtype) in ('float32', 'f32', 'torch.float32') else _lib.NFX_F64
+        npanels = self.getNumberOfPanels(dtype)[0]
+        offs = numpy.zeros(npanels + 1, numpy.int64)
+        n = ctypes.c_int64()
+        _lib.call('nfx_pli_get_column_groups', ctypes.byref(self._h), code, _ORDERS[order], int(vec), _np_ptr(offs),
+                  None, ctypes.byref(n))
+        groups = numpy.zeros(max(n.value, 1), numpy.int32)
+        _lib.call('nfx_pli_get_column_groups', ctypes.byref(self._h), code, _ORDERS[order], int(vec), None,
+                  _np_ptr(groups), ctypes.byref(n))
+        return offs, groups[:n.value]
+
     def seriesStatus(self):
         """Synchronise the current stream and raise NemofluxGpuError if a fused K2+K3 pass launched on this handle
         aborted (its series is NaN); returns 0 otherwise.  The device-path fluxSeries is asynchronous: call this
@@ -736,16 +751,23 @@ class H5DeviceReader(object):
         return self.decode(self.stage(starts, stops), out=out)
 
 
-def probeReadBandwidth(buf, reps=5):
+def probeReadBandwidth(buf, reps=5, groups=None):
     """read-only HBM ceiling (GB/s) of the device of `buf` (a CUDA tensor of >= 9.3 GB whose contents do not matter)
-    with the access pattern of the edge-flux kernels -- the denominator bench.py quotes next to the copy peak"""
+    with the access pattern of the edge-flux kernels -- the denominator bench.py quotes next to the copy peak.
+    groups (int32 CUDA tensor, ascending 256-bit vector indices < 30046 of the probe's 362 x 332 plane): walk only
+    those, the pattern of the sparse fused pass; the rate then counts the bytes of the listed groups."""
     torch = _torch()
     if not isinstance(buf, torch.Tensor) or not buf.is_cuda or not buf.is_contiguous():
         raise TypeError('buf must be a contiguous CUDA tensor')
     r = ctypes.c_double()
     with torch.cuda.device(buf.device):
-        _lib.call('nfx_probe_read_bandwidth', _t_ptr(buf), int(buf.numel() * buf.element_size()), int(reps),
-                  ctypes.byref(r), _stream_ptr())
+        if groups is None:
+            _lib.call('nfx_probe_read_bandwidth', _t_ptr(buf), int(buf.numel() * buf.element_size()), int(reps),
+                      ctypes.byref(r), _stream_ptr())
+        else:
+            _require_cuda(groups, torch.int32, 'groups')
+            _lib.call('nfx_probe_read_bandwidth_groups', _t_ptr(buf), int(buf.numel() * buf.element_size()),
+                      _t_ptr(groups), int(groups.numel()), int(reps), ctypes.byref(r), _stream_ptr())
     return r.value
 
 
