@@ -203,6 +203,18 @@ int nfx_flux_series(nfx_pli** self, const void* u, const void* v, int dtype, con
 int nfx_flux_series_ld(nfx_pli** self, const void* u, const void* v, int dtype, const double* thickness,
                        const double* arc1, const double* arc2, int nt, int nz, int64_t ld, int sverdrup, double fill,
                        int order, double* eflux, double* series, void* stream);
+/* Flux series per layer of model levels (extension, no counterpart in the reference).  layer_levels: HOST (nlayers+1)
+ * int, strictly ascending, 0 <= layer_levels[0], layer_levels[nlayers] <= nz; layer i = levels
+ * [layer_levels[i], layer_levels[i+1]).  Exactly one of thickness / (e3u, e3v) as in nfx_flux_series / _e3.
+ * series device (nt, nlayers, ntransects); eflux NULL (fused pass where the policy allows) or device
+ * (nt, nlayers, 2*ncell).  Layer i is nfx_flux_series* with the thickness (or e3) zeroed outside the layer, bit for bit
+ * on finite data; an infinity on a level outside the layer does not reach it.  u, v (and e3u, e3v) are read once
+ * whatever the layering.  An invalid layering (nlayers < 1, not strictly ascending, outside [0, nz],
+ * nt * nlayers * npanels over INT_MAX) returns NFX_E_INVALID before anything is launched. */
+int nfx_flux_series_layers(nfx_pli** self, const void* u, const void* v, const void* e3u, const void* e3v, int dtype,
+                           int e3_nt, const double* thickness, const double* arc1, const double* arc2, int nt, int nz,
+                           int64_t ld, int nlayers, const int* layer_levels, int sverdrup, double fill, int order,
+                           double* eflux, double* series, void* stream);
 /* The device-path series calls (nfx_flux_series*, nfx_flux_series_range*) are asynchronous on `stream`.  Their fused
  * pass spins on per-batch counters with a bound; a pass that ever overflowed it aborts and leaves NaN in `series`.
  * nfx_pli_series_status synchronises `stream` and reports that: returns 0 with *status = 0 when every pass launched
@@ -277,6 +289,13 @@ int nfx_flux_series_host(nfx_pli** self, const void* u, const void* v, int dtype
 int nfx_flux_series_host_e3(nfx_pli** self, const void* u, const void* v, const void* e3u, const void* e3v, int dtype,
                             int e3_nt, int e3_on_device, const double* arc1, const double* arc2, int nt, int nz,
                             int sverdrup, double fill, int order, int chunk_steps, double* series);
+/* nfx_flux_series_layers from HOST buffers: arguments as nfx_flux_series_host / _host_e3 (exactly one of thickness and
+ * (e3u, e3v)), layer_levels as nfx_flux_series_layers; series host (nt, nlayers, ntransects). */
+int nfx_flux_series_layers_host(nfx_pli** self, const void* u, const void* v, const void* e3u, const void* e3v,
+                                int dtype_flags, int e3_nt, int e3_on_device, const double* thickness,
+                                const double* arc1, const double* arc2, int nt, int nz, int nlayers,
+                                const int* layer_levels, int sverdrup, double fill, int order, int chunk_steps,
+                                double* series);
 
 #ifdef __cplusplus
 }

@@ -98,6 +98,10 @@ SIGNATURES = {
                              c_vp],
     'nfx_flux_series_host_e3': [P(c_vp), c_vp, c_vp, c_vp, c_vp, c_int, c_int, c_int, c_vp, c_vp, c_int, c_int, c_int,
                                 c_dbl, c_int, c_int, c_vp],
+    'nfx_flux_series_layers': [P(c_vp), c_vp, c_vp, c_vp, c_vp, c_int, c_int, c_vp, c_vp, c_vp, c_int, c_int, c_i64,
+                               c_int, c_vp, c_int, c_dbl, c_int, c_vp, c_vp, c_vp],
+    'nfx_flux_series_layers_host': [P(c_vp), c_vp, c_vp, c_vp, c_vp, c_int, c_int, c_int, c_vp, c_vp, c_vp, c_int,
+                                    c_int, c_int, c_vp, c_int, c_dbl, c_int, c_int, c_vp],
 }
 
 _LIB = None

@@ -182,11 +182,12 @@ static int64_t fused_panel_cells(int64_t ncell, int dtype) {
     return ((ncell + np0 - 1) / np0 + 1023) / 1024 * 1024;
 }
 
+// series (nt, nlayers, M); levels: device (nlayers + 1) layer boundaries, nullptr = one layer, the whole column
 static void flux_series_fast(PliDev& p, const void* u, const void* v, int dtype, const double* thickness,
                              const double* arc1, const double* arc2, int nt, int nz, int64_t ld, int sverdrup,
                              double fill, int order, double* series, cudaStream_t stream, int64_t batch_begin = 0,
                              int64_t batch_end = -1, const void* e3u = nullptr, const void* e3v = nullptr,
-                             int64_t e3_tstride = 0) {
+                             int64_t e3_tstride = 0, int nlayers = 1, const int* levels = nullptr) {
     NFX_REQUIRE(order == NFX_ORDER_LIST || order == NFX_ORDER_MAP, "order must be NFX_ORDER_LIST or NFX_ORDER_MAP");
     NFX_REQUIRE(p.csr[order][0].rowptr.p != nullptr, "computeWeights was not called");
     NFX_REQUIRE(p.has_compact, "nfx_grid_set_cgrid_shape must be called before computeWeights for the flux path");
@@ -197,11 +198,12 @@ static void flux_series_fast(PliDev& p, const void* u, const void* v, int dtype,
     const int64_t panel = fused_panel_cells(ncell, dtype);
     PanelPlan& pl = p.plan[order];
     if (!pl.built || pl.panel_cells != panel) build_panel_plan(p, order, panel, stream);
-    p.partial.ensure((size_t)nt * std::max<int64_t>(pl.nsr, 1));
-    if (batch_end < 0) batch_end = (int64_t)nt * pl.npanels;
+    const int64_t nps = (int64_t)nt * nlayers;   // pseudo-steps (time step, layer)
+    p.partial.ensure((size_t)nps * std::max<int64_t>(pl.nsr, 1));
+    if (batch_end < 0) batch_end = nps * pl.npanels;
     flux_series_fused(p, pl, u, v, dtype, thickness, arc1, arc2, nt, nz, ld, sverdrup, fill, batch_begin, batch_end,
-                      p.partial.p, stream, e3u, e3v, e3_tstride);
-    reduce_subrows(p.partial.p, nt, pl.nsr, pl.tr_ptr.p, pl.tr_sr.p, M, series, stream);
+                      p.partial.p, stream, e3u, e3v, e3_tstride, nlayers, levels);
+    reduce_subrows(p.partial.p, (int)nps, pl.nsr, pl.tr_ptr.p, pl.tr_sr.p, M, series, stream);
 }
 
 // NFX_OPT_FAST_SERIES: 1 (default) = the fused pass when the edge fluxes of one time step fit a ring slot (one
@@ -230,6 +232,37 @@ static bool use_fused_e3(const PliDev& p, int dtype, const void* u, const void* 
     if (dtype == NFX_F64) return ncell * 16 <= single_panel_bytes();
     const uintptr_t more = (uintptr_t)e3u | (uintptr_t)e3v | (uintptr_t)(e3_tstride * 4);
     return fused_tile_columns(dtype, u, v, ncell, ld, fused_panel_cells(ncell, dtype), more) >= 4;
+}
+
+// A layering handed in by the caller (host array): layer i = levels [levels[i], levels[i+1]).  Checked before anything
+// is launched; the pseudo-step batch index of the fused pass ((t * nlayers + i) * npanels + q) must fit an int.
+static void check_layers(const PliDev& p, int dtype, int nt, int nz, int nlayers, const int* levels) {
+    NFX_REQUIRE(nlayers >= 1, "layers: nlayers must be >= 1");
+    NFX_REQUIRE(levels, "layers: layer_levels is NULL");
+    NFX_REQUIRE(levels[0] >= 0 && levels[nlayers] <= nz,
+                "layers: the level boundaries must lie in [0, nz = " + std::to_string(nz) + "]");
+    for (int i = 0; i < nlayers; ++i)
+        NFX_REQUIRE(levels[i] < levels[i + 1], "layers: the level boundaries must be strictly ascending (layer " +
+                                                   std::to_string(i) + " is empty)");
+    const int64_t ncell = p.grid->ncell;
+    const int64_t pc = fused_panel_cells(ncell, dtype == NFX_F64 ? NFX_F64 : NFX_F32);
+    const int64_t npanels = (ncell + pc - 1) / pc;
+    NFX_REQUIRE((int64_t)std::max(nt, 0) * nlayers * std::max<int64_t>(npanels, 1) <= 2147483647ll,
+                "layers: nt * nlayers * npanels overflows int");
+}
+
+// device copy of a (checked) layering, uploaded on `s` when it differs from the previous one of the handle.  One layer
+// of the whole column is the plain series: nullptr, the whole-column kernels (the layered f32 instances spill a few more
+// registers and ran 8 % slower on [0, nz], profiles/r4_layers_ab_C3_C4.json).
+static const int* device_levels(PliDev& p, int nz, int nlayers, const int* levels, cudaStream_t s) {
+    if (nlayers == 1 && levels[0] == 0 && levels[1] == nz) return nullptr;
+    if (p.levels.p == nullptr || !std::equal(levels, levels + nlayers + 1, p.h_levels.begin(), p.h_levels.end())) {
+        p.h_levels.assign(levels, levels + nlayers + 1);
+        p.levels.ensure(p.h_levels.size());
+        NFX_CUDA(cudaMemcpyAsync(p.levels.p, p.h_levels.data(), sizeof(int) * p.h_levels.size(), cudaMemcpyHostToDevice,
+                                 s));
+    }
+    return p.levels.p;
 }
 
 static const Csr& pick_csr(PliDev& p, int order, int layout) {
@@ -718,6 +751,40 @@ int nfx_edgeflux_assemble_e3(const void* u, const void* v, const void* e3u, cons
     });
 }
 
+// nfx_flux_series_ld / _e3 / _layers after their argument checks: the fused pass where the policy allows and eflux is
+// NULL, else K2 into eflux (nt * nlayers, 2*ncell) and K3 over the nt * nlayers pseudo-steps.  e3u == nullptr: thickness.
+// layer_levels: host (nlayers + 1), checked by the caller; nullptr = one layer, the whole column.
+static void flux_series_device(PliDev& p, const void* u, const void* v, const void* e3u, const void* e3v, int dtype,
+                               int e3_nt, const double* thickness, const double* arc1, const double* arc2, int nt,
+                               int nz, int64_t ld, int nlayers, const int* layer_levels, int sverdrup, double fill,
+                               int order, double* eflux, double* series, cudaStream_t stream) {
+    const int64_t ncell = p.grid->ncell;
+    NFX_REQUIRE(ld >= ncell, "ld must be >= the number of cells");
+    int64_t e3_tstride = 0;
+    if (e3u) {
+        NFX_REQUIRE(e3_nt == 1 || e3_nt == nt, "e3u/e3v must hold 1 (time-invariant) or nt time steps");
+        e3_tstride = e3_nt == 1 ? 0 : (int64_t)nz * ld;
+    }
+    const int* levels = layer_levels ? device_levels(p, nz, nlayers, layer_levels, stream) : nullptr;
+    g_last_series_fused = 0;
+    g_last_series_sparse = 0;
+    if (eflux == nullptr && (e3u ? use_fused_e3(p, dtype, u, v, e3u, e3v, e3_tstride, ld) : use_fused(p, dtype, u, v, ld))) {
+        g_last_series_fused = 1;
+        flux_series_fast(p, u, v, dtype, thickness, arc1, arc2, nt, nz, ld, sverdrup, fill, order, series, stream, 0, -1,
+                         e3u, e3v, e3_tstride, nlayers, levels);
+        return;
+    }
+    const Csr& c = pick_csr(p, order, 1);
+    const int64_t nps = (int64_t)nt * nlayers;
+    if (eflux == nullptr) {   // two-launch path with an internal eflux array
+        p.stage_eflux[0].ensure((size_t)nps * 2 * ncell);
+        eflux = p.stage_eflux[0].p;
+    }
+    edgeflux_assemble_panel(u, v, dtype, thickness, arc1, arc2, nt, nz, ncell, ld, sverdrup, fill, eflux, 0, g_k2opt,
+                            stream, e3u, e3v, e3_tstride, nlayers, levels);
+    csr_integrate(c, p.ntransects, eflux, ncell * 2, (int)nps, series, stream);
+}
+
 int nfx_flux_series_e3(nfx_pli** self, const void* u, const void* v, const void* e3u, const void* e3v, int dtype,
                        int e3_nt, const double* arc1, const double* arc2, int nt, int nz, int64_t ld, int sverdrup,
                        double fill, int order, double* eflux, double* series, void* stream) {
@@ -727,26 +794,26 @@ int nfx_flux_series_e3(nfx_pli** self, const void* u, const void* v, const void*
         NFX_REQUIRE(p.grid, "setGrid was not called");
         DeviceGuard g(p.grid->device);
         NFX_REQUIRE(u && v && e3u && e3v && arc1 && arc2 && series, "NULL pointer");
-        const int64_t ncell = p.grid->ncell;
-        NFX_REQUIRE(ld >= ncell, "ld must be >= the number of cells");
-        NFX_REQUIRE(e3_nt == 1 || e3_nt == nt, "e3u/e3v must hold 1 (time-invariant) or nt time steps");
-        const int64_t e3_tstride = e3_nt == 1 ? 0 : (int64_t)nz * ld;
-        g_last_series_fused = 0;
-        g_last_series_sparse = 0;
-        if (eflux == nullptr && use_fused_e3(p, dtype, u, v, e3u, e3v, e3_tstride, ld)) {
-            g_last_series_fused = 1;
-            flux_series_fast(p, u, v, dtype, nullptr, arc1, arc2, nt, nz, ld, sverdrup, fill, order, series,
-                             (cudaStream_t)stream, 0, -1, e3u, e3v, e3_tstride);
-            return;
-        }
-        const Csr& c = pick_csr(p, order, 1);
-        if (eflux == nullptr) {
-            p.stage_eflux[0].ensure((size_t)nt * 2 * ncell);
-            eflux = p.stage_eflux[0].p;
-        }
-        edgeflux_assemble_panel(u, v, dtype, nullptr, arc1, arc2, nt, nz, ncell, ld, sverdrup, fill, eflux, 0, g_k2opt,
-                                (cudaStream_t)stream, e3u, e3v, e3_tstride);
-        csr_integrate(c, p.ntransects, eflux, ncell * 2, nt, series, (cudaStream_t)stream);
+        flux_series_device(p, u, v, e3u, e3v, dtype, e3_nt, nullptr, arc1, arc2, nt, nz, ld, 1, nullptr, sverdrup, fill,
+                           order, eflux, series, (cudaStream_t)stream);
+    });
+}
+
+int nfx_flux_series_layers(nfx_pli** self, const void* u, const void* v, const void* e3u, const void* e3v, int dtype,
+                           int e3_nt, const double* thickness, const double* arc1, const double* arc2, int nt, int nz,
+                           int64_t ld, int nlayers, const int* layer_levels, int sverdrup, double fill, int order,
+                           double* eflux, double* series, void* stream) {
+    return guarded([&] {
+        NFX_REQUIRE(self && *self, "NULL handle");
+        PliDev& p = (*self)->d;
+        NFX_REQUIRE(p.grid, "setGrid was not called");
+        DeviceGuard g(p.grid->device);
+        NFX_REQUIRE(u && v && arc1 && arc2 && series, "NULL pointer");
+        NFX_REQUIRE((e3u == nullptr) == (e3v == nullptr), "e3u and e3v go together");
+        NFX_REQUIRE((thickness != nullptr) != (e3u != nullptr), "needs exactly one of thickness and (e3u, e3v)");
+        check_layers(p, dtype, nt, nz, nlayers, layer_levels);
+        flux_series_device(p, u, v, e3u, e3v, dtype, e3_nt, thickness, arc1, arc2, nt, nz, ld, nlayers, layer_levels,
+                           sverdrup, fill, order, eflux, series, (cudaStream_t)stream);
     });
 }
 
@@ -786,24 +853,8 @@ int nfx_flux_series_ld(nfx_pli** self, const void* u, const void* v, int dtype, 
         NFX_REQUIRE(p.grid, "setGrid was not called");
         DeviceGuard g(p.grid->device);
         NFX_REQUIRE(u && v && thickness && arc1 && arc2 && series, "NULL pointer");
-        const int64_t ncell = p.grid->ncell;
-        NFX_REQUIRE(ld >= ncell, "ld must be >= the number of cells");
-        g_last_series_fused = 0;
-        g_last_series_sparse = 0;
-        if (eflux == nullptr && use_fused(p, dtype, u, v, ld)) {
-            g_last_series_fused = 1;
-            flux_series_fast(p, u, v, dtype, thickness, arc1, arc2, nt, nz, ld, sverdrup, fill, order, series,
-                             (cudaStream_t)stream);
-            return;
-        }
-        const Csr& c = pick_csr(p, order, 1);
-        if (eflux == nullptr) {   // two-launch path with an internal eflux array
-            p.stage_eflux[0].ensure((size_t)nt * 2 * ncell);
-            eflux = p.stage_eflux[0].p;
-        }
-        edgeflux_assemble_panel(u, v, dtype, thickness, arc1, arc2, nt, nz, ncell, ld, sverdrup, fill, eflux, 0, g_k2opt,
-                                (cudaStream_t)stream);
-        csr_integrate(c, p.ntransects, eflux, ncell * 2, nt, series, (cudaStream_t)stream);
+        flux_series_device(p, u, v, nullptr, nullptr, dtype, 0, thickness, arc1, arc2, nt, nz, ld, 1, nullptr, sverdrup,
+                           fill, order, eflux, series, (cudaStream_t)stream);
     });
 }
 
@@ -942,11 +993,12 @@ int nfx_flux_series(nfx_pli** self, const void* u, const void* v, int dtype, con
 // ---- everything from host buffers: double-buffered H2D staging, K2+K3 per chunk --------------------------
 // e3u/e3v (optional): per-column scale factors instead of `thickness`.  e3_on_device: borrowed device arrays
 // (e3_nt, nz, ncell) of the dtype of u, v; else host arrays -- e3_nt == 1 is uploaded once per call, e3_nt == nt
-// travels in the chunks next to u and v (same byte order as u, v).
+// travels in the chunks next to u and v (same byte order as u, v).  layer_levels (host, nlayers + 1, NULL = the whole
+// column): series (nt, nlayers, M), every chunk runs its nt_chunk * nlayers pseudo-steps.
 static void flux_series_host_impl(nfx_pli** self, const void* u, const void* v, int dtype_flags, const double* thickness,
                                   const void* e3u, const void* e3v, int e3_nt, int e3_on_device, const double* arc1,
                                   const double* arc2, int nt, int nz, int sverdrup, double fill, int order,
-                                  int chunk_steps, double* series) {
+                                  int chunk_steps, double* series, int nlayers = 1, const int* layer_levels = nullptr) {
     NFX_REQUIRE(self && *self, "NULL handle");
     const bool e3 = e3u != nullptr || e3v != nullptr;
     NFX_REQUIRE(u && v && arc1 && arc2 && series, "NULL pointer");
@@ -960,8 +1012,10 @@ static void flux_series_host_impl(nfx_pli** self, const void* u, const void* v, 
     NFX_REQUIRE(p.grid, "setGrid was not called");
     DeviceGuard g(p.grid->device);
     const Csr& c = pick_csr(p, order, 1);
+    if (layer_levels) check_layers(p, dtype, nt, nz, nlayers, layer_levels);
     const int64_t ncell = p.grid->ncell;
     const int M = p.ntransects;
+    const int64_t LM = (int64_t)nlayers * M;   // series values per time step
     if (nt == 0 || M == 0) return;
     const size_t esize = dtype == NFX_F64 ? 8 : 4;
     const size_t step_bytes = esize * (size_t)nz * (size_t)ncell;
@@ -987,10 +1041,11 @@ static void flux_series_host_impl(nfx_pli** self, const void* u, const void* v, 
             p.stage_e3v[i].ensure(step_bytes * chunk_steps);
         }
     }
-    p.stage_series.ensure((size_t)nt * M);
+    p.stage_series.ensure((size_t)nt * LM);
     p.stage_arc1.ensure(ncell);
     p.stage_arc2.ensure(ncell);
     cudaStream_t cs = p.copy_stream, ks = p.compute_stream;
+    const int* levels = layer_levels ? device_levels(p, nz, nlayers, layer_levels, ks) : nullptr;
     if (!e3) {
         p.stage_thick.ensure(nz);
         NFX_CUDA(cudaMemcpyAsync(p.stage_thick.p, thickness, sizeof(double) * nz, cudaMemcpyHostToDevice, ks));
@@ -1014,7 +1069,7 @@ static void flux_series_host_impl(nfx_pli** self, const void* u, const void* v, 
     const bool fused = e3 ? use_fused_e3(p, dtype, nullptr, nullptr, nullptr, nullptr, 0, ncell)
                           : use_fused(p, dtype, nullptr, nullptr, ncell);
     if (!fused)
-        for (int i = 0; i < 2; ++i) p.stage_eflux[i].ensure((size_t)chunk_steps * 2 * ncell);
+        for (int i = 0; i < 2; ++i) p.stage_eflux[i].ensure((size_t)chunk_steps * nlayers * 2 * ncell);
     int slot = 0;
     bool used[2] = {false, false};
     for (int t0 = 0; t0 < nt; t0 += chunk_steps, slot ^= 1) {
@@ -1047,20 +1102,20 @@ static void flux_series_host_impl(nfx_pli** self, const void* u, const void* v, 
             ce3u = (const unsigned char*)d_e3u + (per_step ? off : 0);
             ce3v = (const unsigned char*)d_e3v + (per_step ? off : 0);
         }
-        double* out = p.stage_series.p + (size_t)t0 * M;
+        double* out = p.stage_series.p + (size_t)t0 * LM;
         if (fused) {
             flux_series_fast(p, dst[0], dst[1], dtype, e3 ? nullptr : p.stage_thick.p, p.stage_arc1.p, p.stage_arc2.p, n,
-                             nz, ncell, sverdrup, fill, order, out, ks, 0, -1, ce3u, ce3v, e3_tstride);
+                             nz, ncell, sverdrup, fill, order, out, ks, 0, -1, ce3u, ce3v, e3_tstride, nlayers, levels);
         } else {
             edgeflux_assemble_panel(dst[0], dst[1], dtype, e3 ? nullptr : p.stage_thick.p, p.stage_arc1.p,
                                     p.stage_arc2.p, n, nz, ncell, ncell, sverdrup, fill, p.stage_eflux[slot].p, 0, g_k2opt,
-                                    ks, ce3u, ce3v, e3_tstride);
-            csr_integrate(c, M, p.stage_eflux[slot].p, ncell * 2, n, out, ks);
+                                    ks, ce3u, ce3v, e3_tstride, nlayers, levels);
+            csr_integrate(c, M, p.stage_eflux[slot].p, ncell * 2, n * nlayers, out, ks);
         }
         NFX_CUDA(cudaEventRecord(p.ev_done[slot], ks));
         used[slot] = true;
     }
-    NFX_CUDA(cudaMemcpyAsync(series, p.stage_series.p, sizeof(double) * (size_t)nt * M, cudaMemcpyDeviceToHost, ks));
+    NFX_CUDA(cudaMemcpyAsync(series, p.stage_series.p, sizeof(double) * (size_t)(nt * LM), cudaMemcpyDeviceToHost, ks));
     NFX_CUDA(cudaStreamSynchronize(ks));
     NFX_CUDA(cudaStreamSynchronize(cs));
     g_last_series_fused = fused ? 1 : 0;
@@ -1086,6 +1141,20 @@ int nfx_flux_series_host_e3(nfx_pli** self, const void* u, const void* v, const 
         NFX_REQUIRE(e3u && e3v, "e3u / e3v is NULL");
         flux_series_host_impl(self, u, v, dtype_flags, nullptr, e3u, e3v, e3_nt, e3_on_device, arc1, arc2, nt, nz,
                               sverdrup, fill, order, chunk_steps, series);
+    });
+}
+
+int nfx_flux_series_layers_host(nfx_pli** self, const void* u, const void* v, const void* e3u, const void* e3v,
+                                int dtype_flags, int e3_nt, int e3_on_device, const double* thickness,
+                                const double* arc1, const double* arc2, int nt, int nz, int nlayers,
+                                const int* layer_levels, int sverdrup, double fill, int order, int chunk_steps,
+                                double* series) {
+    return guarded([&] {
+        NFX_REQUIRE((thickness != nullptr) != (e3u != nullptr || e3v != nullptr),
+                    "needs exactly one of thickness and (e3u, e3v)");
+        NFX_REQUIRE(layer_levels, "layers: layer_levels is NULL");
+        flux_series_host_impl(self, u, v, dtype_flags, thickness, e3u, e3v, e3_nt, e3_on_device, arc1, arc2, nt, nz,
+                              sverdrup, fill, order, chunk_steps, series, nlayers, layer_levels);
     });
 }
 

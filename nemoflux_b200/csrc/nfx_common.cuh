@@ -191,6 +191,8 @@ struct PliDev {
     std::vector<int> h_batch_map;
     int64_t batch_map_key[4] = {-1, -1, -1, -1};   // (batch_begin, batch_end, npanels, order) of the cached map
     std::vector<int64_t> h_sub_offsets, h_map_offsets;
+    DevBuf<int> levels;            // layered series: device copy of the layer boundaries of the last layered call
+    std::vector<int> h_levels;     // ... and its host copy (the upload is skipped when they are unchanged)
     // scratch reused by the host-buffer entry points
     DevBuf<double> scratch_data, scratch_res;
     // persistent staging of nfx_flux_series_host (two slots)
@@ -233,7 +235,8 @@ void edgeflux_assemble(const void* u, const void* v, int dtype, const double* th
 void edgeflux_assemble_panel(const void* u, const void* v, int dtype, const double* thickness, const double* arc1,
                              const double* arc2, int nt, int nz, int64_t ncols, int64_t ld, int sverdrup, double fill,
                              double* eflux, int keep_l2, const K2Options& opt, cudaStream_t s,
-                             const void* e3u = nullptr, const void* e3v = nullptr, int64_t e3_tstride = 0);
+                             const void* e3u = nullptr, const void* e3v = nullptr, int64_t e3_tstride = 0,
+                             int nlayers = 1, const int* levels = nullptr);
 void edgeflux_to_cell_by_cell(const double* eflux, int nt, int ny, int nx, double* iv, cudaStream_t s);
 void edgeflux_absmax(const double* eflux, int nt, int64_t ncell, double* result_host, cudaStream_t s);
 void bswap_inplace(void* p, size_t n, int esize, cudaStream_t s);   // big-endian file bytes -> native, on the device
@@ -252,7 +255,7 @@ void build_column_groups(PanelPlan& pl, int64_t ncell, int ntransects, int vec, 
 void flux_series_fused(PliDev& p, PanelPlan& pl, const void* u, const void* v, int dtype, const double* thickness,
                        const double* arc1, const double* arc2, int nt, int nz, int64_t ld, int sverdrup, double fill,
                        int64_t batch_begin, int64_t batch_end, double* out, cudaStream_t s, const void* e3u = nullptr,
-                       const void* e3v = nullptr, int64_t e3_tstride = 0);
+                       const void* e3v = nullptr, int64_t e3_tstride = 0, int nlayers = 1, const int* levels = nullptr);
 int fused_tile_columns(int dtype, const void* u, const void* v, int64_t ncell, int64_t ld, int64_t panel,
                        uintptr_t more_bits = 0);
 int fused_error_flag(PliDev& p, cudaStream_t s);

@@ -6,11 +6,13 @@
 // then gathers from L2 instead of HBM.  Cutting the work into batches launched one after the other loses
 // more to launch tails than it wins (profiles/r1_fused_notes.md), hence one persistent kernel.
 //
-// Work is cut into batches b = (time step t, panel q of cells) whose (2, panel) slab of edge fluxes fits a
-// ring slot; the ring has R slots.  Work items are handed out in a fixed global order by an atomic counter:
+// Work is cut into batches b = (pseudo-step s, panel q of cells) whose (2, panel) slab of edge fluxes fits a
+// ring slot; the ring has R slots.  A pseudo-step s = t * nlayers + i is time step t restricted to layer i, the
+// levels [levels[i], levels[i+1]) (levels == nullptr: one layer, the whole column -- the plain series).
+// Work items are handed out in a fixed global order by an atomic counter:
 //     ... | K2 tiles of batch b (ntiles items) | K3 items of batch b-1 (nk3 items) | K2 tiles of b+1 | ...
-// K2 item: z-sum + metric factors for 256*VEC columns (field.py:145-163, 195-196, 225-228), written to ring
-//          slot b % R; waits (b >= R) until K3 of batch b-R has finished reading that slot.
+// K2 item: z-sum over the layer's levels + metric factors for 256*VEC columns (field.py:145-163, 195-196, 225-228),
+//          written to ring slot b % R; waits (b >= R) until K3 of batch b-R has finished reading that slot.
 // K3 item: 8 sub-rows (<= 4096 CSR entries of one transect inside panel q) x batch b: one warp per sub-row gathers
 //          from the slot (L2) and writes its partial sum; waits until all K2 tiles of batch b are done.
 // The batches are visited panel-major (batch_map), so a panel's slice of the CSR stays in L2 across time steps.
@@ -58,7 +60,7 @@ struct FusedArgs {
     const double* arc1;
     const double* arc2;
     double* ring;           // ring_slots slots of slot_elems doubles: [eU(panel) | eV(panel)]
-    double* out;            // (nt, nsr) partial sums of the sub-rows
+    double* out;            // (nt * nlayers, nsr) partial sums of the sub-rows
     const int64_t* sr_ptr;    // (nsr + 1) entry offsets of the sub-rows
     const int64_t* panel_sr;  // (npanels + 1) first sub-row of every panel
     int64_t nsr;
@@ -67,13 +69,15 @@ struct FusedArgs {
     int* sync;              // [0] work counter, [1] error flag, [2 .. 2+nb) K2 tiles done, [2+nb .. 2+2nb) K3 items done
     int64_t ncell, ld, panel, slot_elems;   // ld = cells per level plane in memory (>= ncell)
     int nt, nz, ntransects, npanels, nbatches, ntiles, nk3, ring_slots;
-    const int* batch_map;   // (nbatches) global batch index t * npanels + q of the b-th batch visited
+    const int* batch_map;   // (nbatches) global batch index s * npanels + q of the b-th batch visited
     const int32_t* grp;     // sparse pass: PanelPlan::grp (column groups of VEC the K2 tiles load), nullptr = dense
     const int64_t* grp_ptr;
     int k3_lag;             // the K3 items of batch b - k3_lag are queued behind the K2 tiles of batch b
     int k3_unroll8;
     double scale, fill;
     int use_scale, has_fill;
+    const int* levels;      // (nlayers + 1) ascending level boundaries, nullptr = one layer [0, nz)
+    int nlayers;
 };
 
 __device__ __forceinline__ int ld_acquire(const int* p) {
@@ -114,7 +118,9 @@ constexpr int fused_min_ctas(int wanted) {
 
 // E3: e3u[t,k,c] / e3v[t,k,c] replace the 1-D thickness dz[k] (SURVEY 8f rank 4), the arithmetic of
 // k2_edgeflux_ldg<..., E3 = true> (nfx_k2_edgeflux.cu) operation for operation -> the same edge fluxes bit for bit
-template <typename T, int VEC, int UNROLL, int CTAS = 0, bool E3 = false>
+// LAYERED: the batches are (pseudo-step, panel) pairs and the K2 tiles sum the levels of the pseudo-step's layer; a
+// template flag, so that the whole-column instances (levels == nullptr) keep their registers
+template <typename T, int VEC, int UNROLL, int CTAS = 0, bool E3 = false, bool LAYERED = false>
 __global__ void __launch_bounds__(kFusedBlock, fused_min_ctas<T, VEC, UNROLL, E3>(CTAS))
 k23_fused(const FusedArgs a) {
     extern __shared__ double s_dz[];
@@ -168,8 +174,12 @@ k23_fused(const FusedArgs a) {
             if (b >= a.nbatches) continue;
             if (b >= a.ring_slots && !cta_wait(k3done + (b - a.ring_slots), a.nk3, err, &s_ok)) break;
             const int gb = a.batch_map[b];
-            const int64_t t = gb / a.npanels;
-            const int q = gb - (int)t * a.npanels;
+            const int64_t ps = gb / a.npanels;
+            const int q = gb - (int)ps * a.npanels;
+            // layered: the sums of the whole column with dz (e3) zeroed outside the layer
+            const int64_t t = LAYERED ? ps / a.nlayers : ps;
+            const int kbeg = LAYERED ? a.levels[ps - t * a.nlayers] : 0;
+            const int kend = LAYERED ? a.levels[ps - t * a.nlayers + 1] : a.nz;
             const int64_t pc0 = (int64_t)q * a.panel;
             const int64_t pc = min(a.panel, a.ncell - pc0);
             int64_t cl = ((int64_t)r * kFusedBlock + threadIdx.x) * VEC;   // column inside the panel
@@ -190,8 +200,8 @@ k23_fused(const FusedArgs a) {
                     sv[e] = 0.0;
                 }
                 float amax = 0.f;
-                int k = 0;
-                for (; k + UNROLL <= a.nz; k += UNROLL) {
+                int k = kbeg;
+                for (; k + UNROLL <= kend; k += UNROLL) {
                     V ru[UNROLL], rv[UNROLL], re[E3 ? UNROLL : 1], rf[E3 ? UNROLL : 1];
 #pragma unroll
                     for (int qq = 0; qq < UNROLL; ++qq) {
@@ -243,7 +253,7 @@ k23_fused(const FusedArgs a) {
                         }
                     }
                 }
-                for (; k < a.nz; ++k) {
+                for (; k < kend; ++k) {
                     T x[VEC], y[VEC], ex[VEC], ey[VEC];
                     P::unpack(ld_stream(reinterpret_cast<const V*>(pu + (int64_t)k * a.ld), pol_ef), x);
                     P::unpack(ld_stream(reinterpret_cast<const V*>(pv + (int64_t)k * a.ld), pol_ef), y);
@@ -268,7 +278,7 @@ k23_fused(const FusedArgs a) {
                             sv[e] = 0.0;
                         }
 #pragma unroll 1
-                        for (int kk = 0; kk < a.nz; ++kk) {
+                        for (int kk = kbeg; kk < kend; ++kk) {
                             const double d = E3 ? 0.0 : s_dz[kk];
 #pragma unroll
                             for (int e = 0; e < VEC; ++e) {
@@ -323,8 +333,8 @@ k23_fused(const FusedArgs a) {
             if (!cta_wait(k2done + b, a.ntiles, err, &s_ok)) break;
             __threadfence();
             const int gb = a.batch_map[b];
-            const int64_t t = gb / a.npanels;
-            const int q = gb - (int)t * a.npanels;
+            const int64_t ps = gb / a.npanels;
+            const int q = gb - (int)ps * a.npanels;
             {
                 // one warp per sub-row (<= kSubRow entries): lane-strided partial sums, fixed shuffle tree
                 const int64_t sr = a.panel_sr[q] + (int64_t)(r - a.ntiles) * kWarps + wid;
@@ -341,7 +351,7 @@ k23_fused(const FusedArgs a) {
                     }
 #pragma unroll
                     for (int o = 16; o > 0; o >>= 1) acc += __shfl_xor_sync(0xffffffffu, acc, o);
-                    if (lane == 0) a.out[t * a.nsr + sr] = acc;
+                    if (lane == 0) a.out[ps * a.nsr + sr] = acc;
                 }
             }
             __syncthreads();
@@ -362,7 +372,7 @@ __global__ void k_or_flag(const int* flag, int* sticky) {
 // answer is cached per device for the common case (nz <= 128, where registers, not shared memory, bound the occupancy)
 thread_local size_t t_fused_smem = sizeof(double) * 256;
 
-template <typename T, int VEC, int UNROLL, int CTAS = 0, bool E3 = false>
+template <typename T, int VEC, int UNROLL, int CTAS = 0, bool E3 = false, bool LAYERED = false>
 int fused_grid() {
     static int grid[64] = {0};   // per device ordinal
     int dev = 0;
@@ -372,7 +382,7 @@ int fused_grid() {
     if (g == 0 || !small) {
         int sms = 0, per_sm = 0;
         NFX_CUDA(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
-        NFX_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k23_fused<T, VEC, UNROLL, CTAS, E3>, kFusedBlock,
+        NFX_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k23_fused<T, VEC, UNROLL, CTAS, E3, LAYERED>, kFusedBlock,
                                                                std::max(t_fused_smem, sizeof(double) * 256)));
         const int n = sms * std::max(per_sm, 1);
         if (!small) return n;
@@ -383,8 +393,12 @@ int fused_grid() {
 
 template <typename T, int VEC, int UNROLL, int CTAS = 0, bool E3 = false>
 void launch_fused(const FusedArgs& a, cudaStream_t s) {
-    k23_fused<T, VEC, UNROLL, CTAS, E3>
-        <<<fused_grid<T, VEC, UNROLL, CTAS, E3>(), kFusedBlock, sizeof(double) * a.nz * 2, s>>>(a);
+    if (a.levels)
+        k23_fused<T, VEC, UNROLL, CTAS, E3, true>
+            <<<fused_grid<T, VEC, UNROLL, CTAS, E3, true>(), kFusedBlock, sizeof(double) * a.nz * 2, s>>>(a);
+    else
+        k23_fused<T, VEC, UNROLL, CTAS, E3>
+            <<<fused_grid<T, VEC, UNROLL, CTAS, E3>(), kFusedBlock, sizeof(double) * a.nz * 2, s>>>(a);
 }
 
 // e3u/e3v kernels: four streamed arrays, so half the columns per thread of the thickness kernels keep the same
@@ -435,7 +449,7 @@ int fused_tile_columns(int dtype, const void* u, const void* v, int64_t ncell, i
 void flux_series_fused(PliDev& p, PanelPlan& pl, const void* u, const void* v, int dtype, const double* thickness,
                        const double* arc1, const double* arc2, int nt, int nz, int64_t ld, int sverdrup, double fill,
                        int64_t batch_begin, int64_t batch_end, double* out, cudaStream_t s, const void* e3u,
-                       const void* e3v, int64_t e3_tstride) {
+                       const void* e3v, int64_t e3_tstride, int nlayers, const int* levels) {
     const int64_t ncell = p.grid->ncell;
     const int M = p.ntransects;
     const bool e3 = e3u != nullptr;
@@ -469,9 +483,13 @@ void flux_series_fused(PliDev& p, PanelPlan& pl, const void* u, const void* v, i
     a.slot_elems = 2 * std::min(pl.panel_cells, ncell);
     a.nt = nt;
     a.nz = nz;
+    a.nlayers = nlayers;
+    a.levels = levels;
+    NFX_REQUIRE(nlayers >= 1 && (levels != nullptr || nlayers == 1), "fused pass: bad layering");
+    const int64_t nps = (int64_t)nt * nlayers;   // pseudo-steps (t, layer)
     a.ntransects = M;
     a.npanels = pl.npanels;
-    NFX_REQUIRE(batch_begin >= 0 && batch_begin <= batch_end && batch_end <= (int64_t)nt * pl.npanels,
+    NFX_REQUIRE(batch_begin >= 0 && batch_begin <= batch_end && batch_end <= nps * pl.npanels,
                 "fused pass: bad batch range");
     a.nbatches = (int)(batch_end - batch_begin);
     a.k3_unroll8 = (g_fused_order >> 1) & 1;
@@ -526,11 +544,11 @@ void flux_series_fused(PliDev& p, PanelPlan& pl, const void* u, const void* v, i
     a.k3_lag = lag;
     a.ring_slots = slots;
     p.ring.ensure((size_t)(a.slot_elems * slots));
-    NFX_CUDA(cudaMemsetAsync(out, 0xFF, sizeof(double) * (size_t)nt * std::max<int64_t>(pl.nsr, 1), s));   // NaN: a pass that
+    NFX_CUDA(cudaMemsetAsync(out, 0xFF, sizeof(double) * (size_t)nps * std::max<int64_t>(pl.nsr, 1), s));   // NaN: a pass that
     // aborts (bounded spin overflow) must not leave plausible numbers behind.  Sub-rows of batches outside
     // [batch_begin, batch_end) belong to other ranks: they contribute 0 here.
     if (pl.nsr > 0) {
-        auto zero_rows = [&](int64_t b0, int64_t b1) {   // batches [b0, b1) -> contiguous runs of sub-rows per time step
+        auto zero_rows = [&](int64_t b0, int64_t b1) {   // batches [b0, b1) -> contiguous runs of sub-rows per pseudo-step
             while (b0 < b1) {
                 const int64_t t = b0 / pl.npanels, q0 = b0 - t * pl.npanels;
                 const int64_t q1 = std::min<int64_t>(pl.npanels, q0 + (b1 - b0));
@@ -541,7 +559,7 @@ void flux_series_fused(PliDev& p, PanelPlan& pl, const void* u, const void* v, i
             }
         };
         zero_rows(0, batch_begin);
-        zero_rows(batch_end, (int64_t)nt * pl.npanels);
+        zero_rows(batch_end, nps * pl.npanels);
     }
     if (a.nbatches == 0) return;
     {

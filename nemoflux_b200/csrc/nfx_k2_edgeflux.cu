@@ -29,16 +29,20 @@ namespace {
 using namespace dev;
 
 // One thread owns VEC adjacent columns of one time step; blockIdx.y = time step.
+// LAYERED: blockIdx.y + ps0 = t * nlayers + i is a pseudo-step, time step t summed over the levels [levels[i],
+// levels[i+1]) of layer i: the sums of the whole column with dz (e3) zeroed outside the layer, bit for bit on finite
+// data.  A template flag, so that the whole-column instances keep their registers.
 // E3: per-column, per-level scale factors e3u/e3v (NEMO's vertical metric, partial cells / z*) replace the 1-D
 // layer thickness dz[k] of field.py:51 -- two more streamed arrays, same layout as u/v (SURVEY 8f rank 4).
 // ALU_MASK (float32 storage): bit q set = level q of every batch of UNROLL levels goes through clean_scaled()
 // (bit shuffle on the ALU, dz scaled by 2^896) instead of an F2F on the XU pipe; same bits either way
-template <typename T, int VEC, int UNROLL, int BLOCK, bool E3, int ALU_MASK>
+template <typename T, int VEC, int UNROLL, int BLOCK, bool E3, int ALU_MASK, bool LAYERED = false>
 __global__ void __launch_bounds__(BLOCK)
 k2_edgeflux_ldg(const T* __restrict__ u, const T* __restrict__ v, const double* __restrict__ dz,
                 const double* __restrict__ arc1, const double* __restrict__ arc2, double* __restrict__ eflux, int nz,
                 int64_t ncell, int64_t ld, double scale, int use_scale, T fill, int has_fill, int keep_l2,
-                const T* __restrict__ e3u, const T* __restrict__ e3v, int64_t e3_tstride) {
+                const T* __restrict__ e3u, const T* __restrict__ e3v, int64_t e3_tstride,
+                const int* __restrict__ levels, int nlayers, int64_t ps0) {
     // ncell = columns handled by this launch (a panel of the grid), ld = cells per level plane (row stride of u, v)
     extern __shared__ double s_dz[];   // [nz] dz, then (ALU_MASK != 0) [nz] dz * 2^896
     bool redo = false;                 // ALU_MASK: recompute this thread's columns with clean() (saw an infinity)
@@ -60,7 +64,14 @@ k2_edgeflux_ldg(const T* __restrict__ u, const T* __restrict__ v, const double* 
     float amax = 0.f;
     using P = Pack<T, VEC>;
     using V = typename P::type;
-    const int64_t t = blockIdx.y;
+    int64_t ps = blockIdx.y, t = ps;
+    int k0 = 0, k1 = nz;
+    if constexpr (LAYERED) {
+        ps += ps0;
+        t = ps / nlayers;
+        k0 = levels[ps - t * nlayers];
+        k1 = levels[ps - t * nlayers + 1];
+    }
     const int64_t c0 = ((int64_t)blockIdx.x * BLOCK + threadIdx.x) * VEC;
     if (c0 >= ncell) return;
     const T* pu = u + t * nz * ld + c0;
@@ -75,8 +86,8 @@ k2_edgeflux_ldg(const T* __restrict__ u, const T* __restrict__ v, const double* 
         su[e] = 0.0;
         sv[e] = 0.0;
     }
-    int k = 0;
-    for (; k + UNROLL <= nz; k += UNROLL) {
+    int k = k0;
+    for (; k + UNROLL <= k1; k += UNROLL) {
         V ru[UNROLL], rv[UNROLL], re[E3 ? UNROLL : 1], rf[E3 ? UNROLL : 1];
 #pragma unroll
         for (int q = 0; q < UNROLL; ++q) {
@@ -131,7 +142,7 @@ k2_edgeflux_ldg(const T* __restrict__ u, const T* __restrict__ v, const double* 
             }
         }
     }
-    for (; k < nz; ++k) {
+    for (; k < k1; ++k) {
         T a[VEC], b[VEC], ea[VEC], eb[VEC];
         P::unpack(ld_stream(reinterpret_cast<const V*>(pu + (int64_t)k * ld), pol_ef), a);
         P::unpack(ld_stream(reinterpret_cast<const V*>(pv + (int64_t)k * ld), pol_ef), b);
@@ -157,7 +168,7 @@ k2_edgeflux_ldg(const T* __restrict__ u, const T* __restrict__ v, const double* 
                 sv[e] = 0.0;
             }
 #pragma unroll 1
-            for (int kk = 0; kk < nz; ++kk) {
+            for (int kk = k0; kk < k1; ++kk) {
                 const double d = E3 ? 0.0 : s_dz[kk];
 #pragma unroll
                 for (int e = 0; e < VEC; ++e) {
@@ -169,7 +180,7 @@ k2_edgeflux_ldg(const T* __restrict__ u, const T* __restrict__ v, const double* 
             }
         }
     }
-    double* ou = eflux + t * 2 * ncell + c0;
+    double* ou = eflux + ps * 2 * ncell + c0;
     double* ov = ou + ncell;
     // the last vector of a row may hang over the end of the grid (padded planes, ld > ncell): loads are safe,
     // metric factors and stores are only touched for the nvalid real columns
@@ -208,6 +219,11 @@ struct E3Args {
     int64_t tstride = 0;
 };
 
+struct LayerArgs {
+    const int* levels = nullptr;   // device (n + 1) level boundaries, nullptr = one layer, the whole column
+    int n = 1;
+};
+
 template <typename T, int VEC, int UNROLL, int BLOCK>
 void launch_ldg(const T* u, const T* v, const double* dz, const double* arc1, const double* arc2, double* eflux, int nt,
                 int nz, int64_t ncell, int64_t ld, double scale, int use_scale, T fill, int has_fill, int keep_l2,
@@ -219,14 +235,15 @@ void launch_ldg(const T* u, const T* v, const double* dz, const double* arc1, co
     if (e3.e3u)   // float32: every level through the bit shuffle (restored exactly by one multiply per value)
         k2_edgeflux_ldg<T, VEC, UNROLL, BLOCK, true, (sizeof(T) == 4 ? (1 << UNROLL) - 1 : 0)><<<grid, BLOCK, sizeof(double) * nz, s>>>(
             u, v, dz, arc1, arc2, eflux, nz, ncell, ld, scale, use_scale, fill, has_fill, keep_l2, (const T*)e3.e3u,
-            (const T*)e3.e3v, e3.tstride);
+            (const T*)e3.e3v, e3.tstride, nullptr, 1, 0);
     else if (alu_mask >= 0 && sizeof(T) == 4 && UNROLL == 5) {
         switch (alu_mask) {
 #define NFX_ALU_CASE(M)                                                                                             \
     case M:                                                                                                         \
         k2_edgeflux_ldg<T, VEC, UNROLL, BLOCK, false, (sizeof(T) == 4 && UNROLL == 5) ? M : 0>                      \
             <<<grid, BLOCK, sizeof(double) * nz * 2, s>>>(u, v, dz, arc1, arc2, eflux, nz, ncell, ld, scale,      \
-                                                          use_scale, fill, has_fill, keep_l2, nullptr, nullptr, 0); \
+                                                          use_scale, fill, has_fill, keep_l2, nullptr, nullptr, 0,  \
+                                                          nullptr, 1, 0);                                            \
         break;
             NFX_ALU_CASE(0)
             NFX_ALU_CASE(0x01)
@@ -238,17 +255,49 @@ void launch_ldg(const T* u, const T* v, const double* dz, const double* arc1, co
         }
     } else
         k2_edgeflux_ldg<T, VEC, UNROLL, BLOCK, false, kAluMask><<<grid, BLOCK, sizeof(double) * nz * 2, s>>>(
-            u, v, dz, arc1, arc2, eflux, nz, ncell, ld, scale, use_scale, fill, has_fill, keep_l2, nullptr, nullptr, 0);
+            u, v, dz, arc1, arc2, eflux, nz, ncell, ld, scale, use_scale, fill, has_fill, keep_l2, nullptr, nullptr, 0,
+            nullptr, 1, 0);
+}
+
+// layered sums: nt * nlayers pseudo-steps in launches of at most 65535 (gridDim.y), block of 256, every float32 level
+// through the bit shuffle -- the default shape of launch_ldg (the K2 tuning options change speed, never bits)
+template <typename T, int VEC, int UNROLL, bool E3>
+void launch_ldg_layers(const T* u, const T* v, const double* dz, const double* arc1, const double* arc2, double* eflux,
+                       int nt, int nz, int64_t ncell, int64_t ld, double scale, int use_scale, T fill, int has_fill,
+                       int keep_l2, const E3Args& e3, const LayerArgs& ly, cudaStream_t s) {
+    constexpr int kBlock = 256;
+    constexpr int kAluMask = sizeof(T) == 4 ? (E3 ? (1 << UNROLL) - 1 : 0x1f) : 0;
+    static_assert(E3 || UNROLL == 5, "whole-column shape: 5 levels per batch");
+    const int64_t nthreads = (ncell + VEC - 1) / VEC;
+    const int64_t nps = (int64_t)nt * ly.n;
+    for (int64_t ps0 = 0; ps0 < nps; ps0 += 65535) {
+        dim3 grid((unsigned)((nthreads + kBlock - 1) / kBlock), (unsigned)std::min<int64_t>(65535, nps - ps0));
+        k2_edgeflux_ldg<T, VEC, UNROLL, kBlock, E3, kAluMask, true><<<grid, kBlock, sizeof(double) * nz * 2, s>>>(
+            u, v, dz, arc1, arc2, eflux, nz, ncell, ld, scale, use_scale, fill, has_fill, keep_l2, (const T*)e3.e3u,
+            (const T*)e3.e3v, e3.tstride, ly.levels, ly.n, ps0);
+    }
 }
 
 template <typename T, int VEC>
 void dispatch_ldg(const T* u, const T* v, const double* dz, const double* arc1, const double* arc2, double* eflux, int nt,
                   int nz, int64_t ncell, int64_t ld, double scale, int use_scale, T fill, int has_fill, int keep_l2,
-                  const E3Args& e3, const K2Options& opt, cudaStream_t s) {
+                  const E3Args& e3, const LayerArgs& ly, const K2Options& opt, cudaStream_t s) {
     // four float32 streams (e3u/e3v): 15 levels in flight at 80 registers stream 14 % faster than 5 at 72
     // (6.37 vs 5.58 TB/s, tools/e3_bench.py --k2-unroll); every other shape is within 1 % from 3 to 15
     const int unroll = opt.unroll > 0 ? opt.unroll : (e3.e3u && sizeof(T) == 4 && VEC > 1) ? 15 : 5;
     const int block = opt.block > 0 ? opt.block : 256;
+    if (ly.levels) {
+        if (!e3.e3u)
+            launch_ldg_layers<T, VEC, 5, false>(u, v, dz, arc1, arc2, eflux, nt, nz, ncell, ld, scale, use_scale, fill,
+                                                has_fill, keep_l2, e3, ly, s);
+        else if (sizeof(T) == 4 && VEC > 1)
+            launch_ldg_layers<T, VEC, 15, true>(u, v, dz, arc1, arc2, eflux, nt, nz, ncell, ld, scale, use_scale, fill,
+                                                has_fill, keep_l2, e3, ly, s);
+        else
+            launch_ldg_layers<T, VEC, 5, true>(u, v, dz, arc1, arc2, eflux, nt, nz, ncell, ld, scale, use_scale, fill,
+                                               has_fill, keep_l2, e3, ly, s);
+        return;
+    }
 #define NFX_K2_CASE(U, B)                                                                                          \
     if (unroll == U && block == B) {                                                                               \
         launch_ldg<T, VEC, U, B>(u, v, dz, arc1, arc2, eflux, nt, nz, ncell, ld, scale, use_scale, fill, has_fill,  \
@@ -522,11 +571,13 @@ void bswap_inplace(void* p, size_t n, int esize, cudaStream_t s) {
 }
 
 // One launch over `ncols` adjacent columns (a panel of the grid, pointers already offset to its first column)
-// and `nt` time steps; ld = cells per level plane.  eflux: (nt, 2*ncols).
+// and `nt` time steps; ld = cells per level plane.  eflux: (nt, 2*ncols).  Layered (levels: device, nlayers + 1
+// ascending level boundaries): eflux (nt, nlayers, 2*ncols), layer i summed over the levels [levels[i], levels[i+1]);
+// always the direct-load kernel (the TMA variant sums whole columns only).
 void edgeflux_assemble_panel(const void* u, const void* v, int dtype, const double* thickness, const double* arc1,
                              const double* arc2, int nt, int nz, int64_t ncols, int64_t ld, int sverdrup, double fill,
                              double* eflux, int keep_l2, const K2Options& opt, cudaStream_t s, const void* e3u,
-                             const void* e3v, int64_t e3_tstride) {
+                             const void* e3v, int64_t e3_tstride, int nlayers, const int* levels) {
     NFX_REQUIRE(u && v && arc1 && arc2 && eflux, "edgeflux: NULL pointer");
     NFX_REQUIRE((e3u == nullptr) == (e3v == nullptr), "edgeflux: e3u and e3v go together");
     NFX_REQUIRE(thickness || e3u, "edgeflux: needs the layer thickness or e3u/e3v");
@@ -534,6 +585,10 @@ void edgeflux_assemble_panel(const void* u, const void* v, int dtype, const doub
     e3.e3u = e3u;
     e3.e3v = e3v;
     e3.tstride = e3_tstride;
+    LayerArgs ly;
+    ly.levels = levels;
+    ly.n = nlayers;
+    NFX_REQUIRE(nlayers >= 1 && (levels != nullptr || nlayers == 1), "edgeflux: bad layering");
     NFX_REQUIRE(nt >= 0 && nz > 0 && ncols > 0 && ld >= ncols, "edgeflux: bad sizes");
     NFX_REQUIRE(dtype == NFX_F64 || dtype == NFX_F32, "edgeflux: dtype must be NFX_F64 or NFX_F32");
     NFX_REQUIRE(nt <= 65535, "edgeflux: at most 65535 time steps per call");
@@ -545,7 +600,7 @@ void edgeflux_assemble_panel(const void* u, const void* v, int dtype, const doub
                                 (uintptr_t)(e3_tstride * (dtype == NFX_F64 ? 8 : 4));
     const bool aligned16 = (addr_bits & 15) == 0;
     const bool aligned32 = (addr_bits & 31) == 0 && opt.variant != NFX_K2_LDG128;
-    const bool want_tma = (opt.variant == NFX_K2_TMA) && ld == ncols && !e3u;
+    const bool want_tma = (opt.variant == NFX_K2_TMA) && ld == ncols && !e3u && !levels;
     if (want_tma && aligned16 && dtype == NFX_F64 && ncols % 2 == 0) {
         const int cfg = opt.unroll;   // tile configuration selector for the sweep (0 = default)
         const double* pu = (const double*)u;
@@ -575,13 +630,13 @@ void edgeflux_assemble_panel(const void* u, const void* v, int dtype, const doub
         const double* pv = (const double*)v;
         if (aligned32 && ld % 4 == 0 && (ncols % 4 == 0 || ld >= (ncols + 3) / 4 * 4))
             dispatch_ldg<double, 4>(pu, pv, thickness, arc1, arc2, eflux, nt, nz, ncols, ld, scale, sverdrup, fill,
-                                    has_fill, keep_l2, e3, opt, s);
+                                    has_fill, keep_l2, e3, ly, opt, s);
         else if (aligned16 && ld % 2 == 0 && (ncols % 2 == 0 || ld >= (ncols + 1) / 2 * 2))
             dispatch_ldg<double, 2>(pu, pv, thickness, arc1, arc2, eflux, nt, nz, ncols, ld, scale, sverdrup, fill,
-                                    has_fill, keep_l2, e3, opt, s);
+                                    has_fill, keep_l2, e3, ly, opt, s);
         else
             dispatch_ldg<double, 1>(pu, pv, thickness, arc1, arc2, eflux, nt, nz, ncols, ld, scale, sverdrup, fill,
-                                    has_fill, keep_l2, e3, opt, s);
+                                    has_fill, keep_l2, e3, ly, opt, s);
     } else {
         const float* pu = (const float*)u;
         const float* pv = (const float*)v;
@@ -590,13 +645,13 @@ void edgeflux_assemble_panel(const void* u, const void* v, int dtype, const doub
         const bool wide = opt.variant == NFX_K2_LDG;
         if (wide && aligned32 && ld % 8 == 0 && (ncols % 8 == 0 || ld >= (ncols + 7) / 8 * 8))
             dispatch_ldg<float, 8>(pu, pv, thickness, arc1, arc2, eflux, nt, nz, ncols, ld, scale, sverdrup,
-                                   (float)fill, has_fill, keep_l2, e3, opt, s);
+                                   (float)fill, has_fill, keep_l2, e3, ly, opt, s);
         else if (aligned16 && ld % 4 == 0 && (ncols % 4 == 0 || ld >= (ncols + 3) / 4 * 4))
             dispatch_ldg<float, 4>(pu, pv, thickness, arc1, arc2, eflux, nt, nz, ncols, ld, scale, sverdrup,
-                                   (float)fill, has_fill, keep_l2, e3, opt, s);
+                                   (float)fill, has_fill, keep_l2, e3, ly, opt, s);
         else
             dispatch_ldg<float, 1>(pu, pv, thickness, arc1, arc2, eflux, nt, nz, ncols, ld, scale, sverdrup,
-                                   (float)fill, has_fill, keep_l2, e3, opt, s);
+                                   (float)fill, has_fill, keep_l2, e3, ly, opt, s);
     }
     count_launch();
     NFX_CUDA(cudaGetLastError());

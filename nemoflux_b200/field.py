@@ -309,14 +309,13 @@ class Field(object):
                 return None
             return [nemoflux_gpu.H5DeviceReader(d, self.device) for d in readers]
 
-    def _flux_series_device_decode(self, readers, chunk_steps=0, prefetch=True):
+    def _flux_series_device_decode(self, readers, chunk_steps=0, prefetch=True, layers=None):
         """flux series of chunked + deflated uo / vo: the COMPRESSED chunks cross PCIe and are inflated, unshuffled and
         placed on the device (csrc/nfx_inflate.cu), then K2 + K3 run on the decoded slab.  A reader thread copies the
         compressed chunks of block i + 1 from the memory-mapped files into pinned staging while block i is decoded."""
         import threading
         import torch
-        M = len(self.plis)
-        out = numpy.zeros((self.nt, M))
+        out = numpy.zeros(self._series_shape(layers))
         esize = readers[0].ds.dtype.itemsize
         step_bytes = esize * self.nz * self.ny * self.nx
         # The decoder works on one chunk per warp and 20 warps fit an SM: a block of as many chunks as the device holds
@@ -355,7 +354,7 @@ class Field(object):
             if i + 1 < len(blocks) and not prefetch:
                 stage(i + 1)
             ser = self.pli.fluxSeries(ud, vd, self._d_thickness, self._d_arc1, self._d_arc2, sverdrup=self.sverdrup,
-                                      fill=fill, e3u=self._d_e3u, e3v=self._d_e3v)
+                                      fill=fill, e3u=self._d_e3u, e3v=self._d_e3v, layers=layers)
             out[t0:t0 + m] = ser.cpu().numpy()
             if th is not None:
                 th.join()
@@ -363,8 +362,19 @@ class Field(object):
                                 bytes_decoded=sum(r.bytes_decoded for r in readers))
         return out
 
-    def fluxSeries(self, chunk_steps=0, prefetch=True, device_decode=None):
+    def _series_shape(self, layers):
+        return (self.nt, len(self.plis)) if layers is None else (self.nt, len(layers) - 1, len(self.plis))
+
+    def levelsForDepths(self, depths):
+        """depths in metres, ascending -> level boundaries for fluxSeries(layers=), see levelsForDepths below"""
+        return levelsForDepths(self.bounds_depth, depths)
+
+    def layerInterfaces(self):
+        return layerInterfaces(self.bounds_depth)
+
+    def fluxSeries(self, chunk_steps=0, prefetch=True, device_decode=None, layers=None):
         """(nt, M) flux of every transect at every time step -- the loop of fluxplot.py:51-59 in a few launches.
+        layers (level boundaries, see levelsForDepths): (nt, nlayers, M), the flux of every layer of model levels.
 
         The time axis is streamed from the files in chunks: a reader thread fills one of two PINNED host buffers
         (file read, numpy releases the GIL) while the previous chunk goes through the host-buffer entry point of
@@ -378,10 +388,10 @@ class Field(object):
         if device_decode is not False:
             readers = self._device_readers()
             if readers is not None:
-                return self._flux_series_device_decode(readers, chunk_steps, prefetch)
+                return self._flux_series_device_decode(readers, chunk_steps, prefetch, layers)
             if device_decode is True:
                 raise RuntimeError('ERROR: uo / vo are not chunked HDF5 variables with a [shuffle,] [deflate] pipeline')
-        out = numpy.zeros((self.nt, len(self.plis)))
+        out = numpy.zeros(self._series_shape(layers))
         dtype = numpy.dtype(self.ncU['uo'].dtype).newbyteorder('=')
         step_bytes = dtype.itemsize * self.nz * self.ny * self.nx
         # ~300 MB per variable and chunk (sweep in profiles/r1_file_e2e_C3.json: 4 f64 / 8 f32 ORCA1 steps): small enough that reading chunk i+1 overlaps the upload of chunk i even
@@ -441,7 +451,7 @@ class Field(object):
                 th.start()
             nu, nv = views[slot]                    # numpy views of the pinned buffers (kept alive by `bufs`)
             out[t0:t0 + m] = self.pli.fluxSeries(nu[:m], nv[:m], self.thickness, arc1, arc2, sverdrup=self.sverdrup,
-                                                 fill=state.pop(i), e3u=self._d_e3u, e3v=self._d_e3v)
+                                                 fill=state.pop(i), e3u=self._d_e3u, e3v=self._d_e3v, layers=layers)
             if th is not None:
                 th.join()
             elif i + 1 < len(chunks):
@@ -452,6 +462,31 @@ class Field(object):
     def close(self):
         self.ncU.close()
         self.ncV.close()
+
+
+def layerInterfaces(bounds_depth):
+    """(nz + 1) depths in metres of the level interfaces of deptht_bounds (nz, 2): the top of every level, then the
+    bottom of the last"""
+    b = numpy.asarray(bounds_depth, numpy.float64)
+    return numpy.concatenate([b[:, 0], b[-1:, 1]])
+
+
+def levelsForDepths(bounds_depth, depths):
+    """depths in metres, ascending -> level boundaries: each depth snapped to the nearest interface of
+    layerInterfaces(bounds_depth) (ties go to the shallower one).  Raises ValueError when two depths snap to the same
+    interface (the layer between them would be empty) or the snapped depths are not ascending."""
+    iface = layerInterfaces(bounds_depth)
+    d = numpy.asarray(depths, numpy.float64).reshape(-1)
+    if d.size < 2 or not numpy.all(numpy.isfinite(d)):
+        raise ValueError('depths: at least two finite depths are needed')
+    levels = [int(numpy.argmin(numpy.abs(iface - x))) for x in d]
+    for i in range(len(levels) - 1):
+        if levels[i + 1] == levels[i]:
+            raise ValueError(f'depths {d[i]:g} and {d[i + 1]:g} m snap to the same level interface '
+                             f'({iface[levels[i]]:g} m): the layer between them would be empty')
+        if levels[i + 1] < levels[i]:
+            raise ValueError('depths must be ascending')
+    return levels
 
 
 def parseLonLatPoints(text):

@@ -1,10 +1,14 @@
 """fluxplot -- drop-in for nemoflux/fluxplot.py: flux time series of every transect (same flags).
 
     python -m nemoflux_b200.fluxplot -t T.nc -u U.nc -v V.nc -i "../data/nz/S*.txt" [-s] [--output series.csv]
+        [--layers "0,10,35,75" | --depthLayers "0,200,1000,6000"]
 
 The reference loops ``for itime: fld.update(); for pli: pli.getIntegral(...)`` (fluxplot.py:51-59); here the
 whole (nt, M) series comes from Field.fluxSeries() (K2+K3 over chunks of time steps).  The series is printed
 and optionally written as CSV; it is plotted only when matplotlib is importable and --plot is given.
+--layers (model-level boundaries) or --depthLayers (depths in metres, snapped to the nearest level interfaces) split
+every transect's flux by depth: one column per (transect, layer), transect-major, headed label[top-bottom m] with the
+interfaces that were integrated.
 """
 import argparse
 import os
@@ -13,6 +17,17 @@ import numpy
 
 from .field import Field
 from .fluxviz import parseTransects
+
+
+def parseList(text, kind=float):
+    """'0,200,1000' -> [0.0, 200.0, 1000.0] (kind=int: integers only)"""
+    try:
+        vals = [kind(x) for x in text.replace(' ', '').split(',') if x != '']
+    except ValueError:
+        raise argparse.ArgumentTypeError(f'expected a comma-separated list of {kind.__name__} values, got {text!r}')
+    if len(vals) < 2:
+        raise argparse.ArgumentTypeError(f'expected at least two boundaries, got {text!r}')
+    return vals
 
 
 def main(argv=None):
@@ -26,21 +41,32 @@ def main(argv=None):
     ap.add_argument('-o', '--output', default='', help='write the series as CSV (time, one column per transect)')
     ap.add_argument('--plot', action='store_true')
     ap.add_argument('--meshFile', default='', help='optional mesh_mask file: e3u_0/e3v_0 (and e2u/e1v) scale factors')
+    lay = ap.add_mutually_exclusive_group()
+    lay.add_argument('--layers', type=lambda x: parseList(x, int), default=None,
+                     help='flux per layer of model levels: level boundaries "0,10,35,75"')
+    lay.add_argument('--depthLayers', type=parseList, default=None,
+                     help='flux per depth range: depths in metres "0,200,1000,6000", snapped to level interfaces')
     a = ap.parse_args(argv)
     pts, names = parseTransects(a.lonLatPoints, a.iFiles)
     print(f'target points:\n {pts}')
     fld = Field(a.tFile, a.uFile, a.vFile, pts, a.sverdrup, meshFile=a.meshFile or None)
-    series = fld.fluxSeries()
+    layers = fld.levelsForDepths(a.depthLayers) if a.depthLayers is not None else a.layers
+    series = fld.fluxSeries(layers=layers)
     timeVals = [fld.timeObj.getTimeAsDate(i) for i in range(fld.nt)]
     units = 'Sv' if a.sverdrup else 'A m^2/s'
     labels = [os.path.basename(n) for n in names]
+    rows = series
+    if layers is not None:
+        iface = fld.layerInterfaces()
+        labels = [f'{lab}[{iface[k0]:g}-{iface[k1]:g} m]' for lab in labels for k0, k1 in zip(layers[:-1], layers[1:])]
+        rows = numpy.asarray(series).transpose(0, 2, 1).reshape(fld.nt, -1)      # (time, transect-major layers)
     print('time,' + ','.join(labels) + f'   [{units}]')
-    for t, row in zip(timeVals, series):
+    for t, row in zip(timeVals, rows):
         print(f'{t},' + ','.join(f'{x:.15g}' for x in row))
     if a.output:
         with open(a.output, 'w') as f:
             f.write('time,' + ','.join(labels) + '\n')
-            for t, row in zip(timeVals, series):
+            for t, row in zip(timeVals, rows):
                 f.write(f'{t},' + ','.join(repr(float(x)) for x in row) + '\n')
     if a.plot:
         try:
@@ -49,8 +75,8 @@ def main(argv=None):
             print('matplotlib is not installed: no plot')
         else:
             lineTypes = ['b-', 'm--', 'c-.', 'r:', 'g-', 'k--']
-            for i in range(series.shape[1]):
-                plt.plot(timeVals, series[:, i], lineTypes[i % len(lineTypes)])
+            for i in range(rows.shape[1]):
+                plt.plot(timeVals, rows[:, i], lineTypes[i % len(lineTypes)])
             if len(labels) > 1:
                 plt.legend(labels)
             plt.title('Water flow')

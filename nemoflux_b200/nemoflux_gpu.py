@@ -275,7 +275,7 @@ class PolylineIntegral(object):
         return st.value
 
     def fluxSeries(self, u, v, thickness, arc1, arc2, sverdrup=False, fill=float('nan'), order='map', eflux=None,
-                   out=None, chunk_steps=0, batch_range=None, e3u=None, e3v=None):
+                   out=None, chunk_steps=0, batch_range=None, e3u=None, e3v=None, layers=None):
         """flux time series of every transect: (nt, M).
 
         u, v: (nt, nz, ny, nx) [or (nz, ny, nx)] float64/float32, either cuda tensors (device path: K2+K3 on
@@ -290,17 +290,25 @@ class PolylineIntegral(object):
         e3u, e3v: per-column vertical scale factors, (1 or nt, nz, cells) with the dtype and plane layout of
         uo/vo (with host uo/vo: CUDA tensors uploaded once by the caller -- a mesh_mask's e3u_0/e3v_0 -- or host
         arrays in the byte order of uo/vo, streamed with them when they hold nt time steps); they replace the 1-D thickness (SURVEY 8f rank 4; fused pass with eflux=None when the
-        policy of nfx_flux_series_e3 allows, else two launches)."""
+        policy of nfx_flux_series_e3 allows, else two launches).
+
+        layers: ascending model-level boundaries [l0 < l1 < ... < lN] with 0 <= l0 and lN <= nz -> the series is
+        (nt, N, M): [t, i, m] is transect m's flux at step t restricted to the levels [l_i, l_{i+1}) -- bit for bit the
+        series with the thickness (or e3u/e3v) zeroed outside the layer, on finite data.  uo/vo are read once whatever
+        the layering; eflux, if given, is (nt, N, 2*ncell).  Not combined with batch_range."""
         torch = _torch()
+        lev = _layer_levels(layers)
+        if lev is not None and batch_range is not None:
+            raise ValueError('batch_range and layers cannot be combined')
         if isinstance(u, torch.Tensor) and u.is_cuda:
             return self._flux_series_device(u, v, thickness, arc1, arc2, sverdrup, fill, order, eflux, out, batch_range,
-                                            e3u, e3v)
+                                            e3u, e3v, lev)
         if batch_range is not None:
             raise ValueError('batch_range needs CUDA tensors')
-        return self._flux_series_host(u, v, thickness, arc1, arc2, sverdrup, fill, order, chunk_steps, e3u, e3v)
+        return self._flux_series_host(u, v, thickness, arc1, arc2, sverdrup, fill, order, chunk_steps, e3u, e3v, lev)
 
     def _flux_series_device(self, u, v, thickness, arc1, arc2, sverdrup, fill, order, eflux, out, batch_range=None,
-                            e3u=None, e3v=None):
+                            e3u=None, e3v=None, lev=None):
         torch = _torch()
         ncells = self._grid.getNumberOfCells() if self._grid is not None else -1
         if u.dim() == 3 and u.shape[2] != ncells and u.shape[1] * u.shape[2] == ncells:
@@ -320,8 +328,27 @@ class PolylineIntegral(object):
             if t.numel() != n:
                 raise ValueError(f'{name} must hold {n} values, got {t.numel()}')
         m = self.getNumberOfTransects()
+        shape = (nt, m) if lev is None else (nt, lev.size - 1, m)
         if nt == 0 or m == 0:       # nothing to integrate: no launch (empty tensors have no device address)
-            return out if out is not None else torch.zeros((nt, m), dtype=torch.float64, device=u.device)
+            return out if out is not None else torch.zeros(shape, dtype=torch.float64, device=u.device)
+        if lev is not None:
+            e3_nt = _check_e3(e3u, e3v, u, nt, nz, ncell, ld) if use_e3 else 0
+            if eflux is not None:
+                _require_cuda(eflux, torch.float64, 'eflux')
+                if eflux.numel() != nt * (lev.size - 1) * 2 * ncell:
+                    raise ValueError(f'eflux must hold nt*nlayers*2*ncell = {nt * (lev.size - 1) * 2 * ncell} values')
+            if out is None:
+                out = torch.empty(shape, dtype=torch.float64, device=u.device)
+            _require_cuda(out, torch.float64, 'out')
+            if out.numel() != nt * (lev.size - 1) * m:
+                raise ValueError(f'out must hold nt*nlayers*M = {nt * (lev.size - 1) * m} values')
+            ptr = lambda t: _t_ptr(t) if t is not None else None   # noqa: E731
+            with torch.cuda.device(u.device):
+                _lib.call('nfx_flux_series_layers', ctypes.byref(self._h), _t_ptr(u), _t_ptr(v), ptr(e3u), ptr(e3v),
+                          _dtype_code(str(u.dtype)), e3_nt, None if use_e3 else _t_ptr(thickness), _t_ptr(arc1),
+                          _t_ptr(arc2), nt, nz, ld, lev.size - 1, _np_ptr(lev), int(bool(sverdrup)), float(fill),
+                          _ORDERS[order], ptr(eflux), _t_ptr(out), _stream_ptr())
+            return out
         if use_e3:
             e3_nt = _check_e3(e3u, e3v, u, nt, nz, ncell, ld)
             if eflux is not None:
@@ -364,7 +391,8 @@ class PolylineIntegral(object):
                       _ORDERS[order], _t_ptr(eflux) if eflux is not None else None, _t_ptr(out), _stream_ptr())
         return out
 
-    def _flux_series_host(self, u, v, thickness, arc1, arc2, sverdrup, fill, order, chunk_steps, e3u=None, e3v=None):
+    def _flux_series_host(self, u, v, thickness, arc1, arc2, sverdrup, fill, order, chunk_steps, e3u=None, e3v=None,
+                          lev=None):
         torch = _torch()
         keep = (u, v, e3u, e3v)  # keep pinned tensors alive while numpy views are in use
         if isinstance(u, torch.Tensor):
@@ -387,7 +415,7 @@ class PolylineIntegral(object):
         if a1.size != ncell or a2.size != ncell:
             raise ValueError('arc1/arc2 sizes do not match uo')
         m = self.getNumberOfTransects()
-        out = numpy.zeros((nt, m), numpy.float64)
+        out = numpy.zeros((nt, m) if lev is None else (nt, lev.size - 1, m), numpy.float64)
         if e3u is not None or e3v is not None:
             if e3u is None or e3v is None:
                 raise ValueError('e3u and e3v go together')
@@ -414,6 +442,12 @@ class PolylineIntegral(object):
             if tuple(e3u.shape) != tuple(e3v.shape) or n3 not in (nz * ncell, nt * nz * ncell):
                 raise ValueError('e3u/e3v must hold (1 or nt, nz, ny*nx) values of the same shape')
             e3_nt = n3 // (nz * ncell)
+            if lev is not None:
+                _lib.call('nfx_flux_series_layers_host', ctypes.byref(self._h), _np_ptr(u), _np_ptr(v), pu, pv, code,
+                          e3_nt, int(on_device), None, _np_ptr(a1), _np_ptr(a2), nt, nz, lev.size - 1, _np_ptr(lev),
+                          int(bool(sverdrup)), float(fill), _ORDERS[order], int(chunk_steps), _np_ptr(out))
+                del keep
+                return out
             _lib.call('nfx_flux_series_host_e3', ctypes.byref(self._h), _np_ptr(u), _np_ptr(v), pu, pv, code, e3_nt,
                       int(on_device), _np_ptr(a1), _np_ptr(a2), nt, nz, int(bool(sverdrup)), float(fill), _ORDERS[order],
                       int(chunk_steps), _np_ptr(out))
@@ -422,6 +456,12 @@ class PolylineIntegral(object):
         th = numpy.ascontiguousarray(_to_numpy(thickness), numpy.float64)
         if th.size != nz:
             raise ValueError('thickness size does not match uo')
+        if lev is not None:
+            _lib.call('nfx_flux_series_layers_host', ctypes.byref(self._h), _np_ptr(u), _np_ptr(v), None, None, code, 0, 0,
+                      _np_ptr(th), _np_ptr(a1), _np_ptr(a2), nt, nz, lev.size - 1, _np_ptr(lev), int(bool(sverdrup)),
+                      float(fill), _ORDERS[order], int(chunk_steps), _np_ptr(out))
+            del keep
+            return out
         _lib.call('nfx_flux_series_host', ctypes.byref(self._h), _np_ptr(u), _np_ptr(v), code,
                   _np_ptr(th), _np_ptr(a1), _np_ptr(a2), nt, nz, int(bool(sverdrup)), float(fill), _ORDERS[order],
                   int(chunk_steps), _np_ptr(out))
@@ -491,6 +531,21 @@ def _to_numpy(x):
     if isinstance(x, torch.Tensor):
         return x.detach().cpu().numpy()
     return numpy.asarray(x)
+
+
+def _layer_levels(layers):
+    """layers -> contiguous int32 array of level boundaries (None stays None).  Only the form is checked here; the
+    library rejects boundaries that are not strictly ascending inside [0, nz]."""
+    if layers is None:
+        return None
+    a = numpy.asarray(_to_numpy(layers))
+    if a.ndim != 1 or a.size < 2:
+        raise ValueError(f'layers must be a 1-D sequence of at least 2 level boundaries, got shape {a.shape}')
+    if a.dtype.kind not in 'iu' and not (a.dtype.kind == 'f' and numpy.all(a == numpy.round(a))):
+        raise ValueError('layers must hold integer level indices')
+    if numpy.any(numpy.abs(a) > 2 ** 31 - 1):
+        raise ValueError('layers: level index out of range')
+    return numpy.ascontiguousarray(a, numpy.int32)
 
 
 def _plane_layout(t, name, ncell_expected=None):
