@@ -215,6 +215,20 @@ int nfx_flux_series_layers(nfx_pli** self, const void* u, const void* v, const v
                            int e3_nt, const double* thickness, const double* arc1, const double* arc2, int nt, int nz,
                            int64_t ld, int nlayers, const int* layer_levels, int sverdrup, double fill, int order,
                            double* eflux, double* series, void* stream);
+/* Transport section (extension, no counterpart in the reference): the flux of every sub-segment (cell crossing, the
+ * emission order of nfx_pli_get_subsegments) per layer of model levels.  Arguments as nfx_flux_series_layers without
+ * order and eflux; section device (nt, nlayers, nsub):
+ *   section[t, i, s] = ((w[s,0]*E[idx[4s]] + w[s,1]*E[idx[4s+1]]) + w[s,2]*E[idx[4s+2]]) + w[s,3]*E[idx[4s+3]]
+ * with idx the list-order compact flux index (E, W, N, S edges; -1 = 0), E the layer-i edge flux exactly as
+ * nfx_flux_series_layers writes it into eflux, separate multiplies and adds (no FMA): summing a transect's sub-segments
+ * gives its layered series to rounding.  One launch per 65535 time steps, asynchronous on `stream`, no spin waits (it
+ * neither sets nor reports the handle's fused-pass error flag).  An invalid layering, a NULL pointer or transects
+ * computed without nfx_grid_set_cgrid_shape return NFX_E_INVALID before anything is launched; nt == 0 or no
+ * sub-segment launches nothing. */
+int nfx_flux_section(nfx_pli** self, const void* u, const void* v, const void* e3u, const void* e3v, int dtype,
+                     int e3_nt, const double* thickness, const double* arc1, const double* arc2, int nt, int nz,
+                     int64_t ld, int nlayers, const int* layer_levels, int sverdrup, double fill, double* section,
+                     void* stream);
 /* The device-path series calls (nfx_flux_series*, nfx_flux_series_range*) are asynchronous on `stream`.  Their fused
  * pass spins on per-batch counters with a bound; a pass that ever overflowed it aborts and leaves NaN in `series`.
  * nfx_pli_series_status synchronises `stream` and reports that: returns 0 with *status = 0 when every pass launched
@@ -296,6 +310,13 @@ int nfx_flux_series_layers_host(nfx_pli** self, const void* u, const void* v, co
                                 const double* arc1, const double* arc2, int nt, int nz, int nlayers,
                                 const int* layer_levels, int sverdrup, double fill, int order, int chunk_steps,
                                 double* series);
+/* nfx_flux_section from HOST buffers: arguments as nfx_flux_series_layers_host without order (native or
+ * NFX_BIG_ENDIAN data, chunk_steps, e3 on the device or on the host, time-invariant or per step);
+ * section host (nt, nlayers, nsub). */
+int nfx_flux_section_host(nfx_pli** self, const void* u, const void* v, const void* e3u, const void* e3v,
+                          int dtype_flags, int e3_nt, int e3_on_device, const double* thickness, const double* arc1,
+                          const double* arc2, int nt, int nz, int nlayers, const int* layer_levels, int sverdrup,
+                          double fill, int chunk_steps, double* section);
 
 #ifdef __cplusplus
 }

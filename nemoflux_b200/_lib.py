@@ -102,6 +102,10 @@ SIGNATURES = {
                                c_int, c_vp, c_int, c_dbl, c_int, c_vp, c_vp, c_vp],
     'nfx_flux_series_layers_host': [P(c_vp), c_vp, c_vp, c_vp, c_vp, c_int, c_int, c_int, c_vp, c_vp, c_vp, c_int,
                                     c_int, c_int, c_vp, c_int, c_dbl, c_int, c_int, c_vp],
+    'nfx_flux_section': [P(c_vp), c_vp, c_vp, c_vp, c_vp, c_int, c_int, c_vp, c_vp, c_vp, c_int, c_int, c_i64, c_int,
+                         c_vp, c_int, c_dbl, c_vp, c_vp],
+    'nfx_flux_section_host': [P(c_vp), c_vp, c_vp, c_vp, c_vp, c_int, c_int, c_int, c_vp, c_vp, c_vp, c_int, c_int,
+                              c_int, c_vp, c_int, c_dbl, c_int, c_vp],
 }
 
 _LIB = None

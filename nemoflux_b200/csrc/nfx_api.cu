@@ -235,8 +235,8 @@ static bool use_fused_e3(const PliDev& p, int dtype, const void* u, const void* 
 }
 
 // A layering handed in by the caller (host array): layer i = levels [levels[i], levels[i+1]).  Checked before anything
-// is launched; the pseudo-step batch index of the fused pass ((t * nlayers + i) * npanels + q) must fit an int.
-static void check_layers(const PliDev& p, int dtype, int nt, int nz, int nlayers, const int* levels) {
+// is launched.
+static void check_layer_levels(int nz, int nlayers, const int* levels) {
     NFX_REQUIRE(nlayers >= 1, "layers: nlayers must be >= 1");
     NFX_REQUIRE(levels, "layers: layer_levels is NULL");
     NFX_REQUIRE(levels[0] >= 0 && levels[nlayers] <= nz,
@@ -244,6 +244,11 @@ static void check_layers(const PliDev& p, int dtype, int nt, int nz, int nlayers
     for (int i = 0; i < nlayers; ++i)
         NFX_REQUIRE(levels[i] < levels[i + 1], "layers: the level boundaries must be strictly ascending (layer " +
                                                    std::to_string(i) + " is empty)");
+}
+
+// ... and for the series: the pseudo-step batch index of the fused pass ((t * nlayers + i) * npanels + q) must fit an int
+static void check_layers(const PliDev& p, int dtype, int nt, int nz, int nlayers, const int* levels) {
+    check_layer_levels(nz, nlayers, levels);
     const int64_t ncell = p.grid->ncell;
     const int64_t pc = fused_panel_cells(ncell, dtype == NFX_F64 ? NFX_F64 : NFX_F32);
     const int64_t npanels = (ncell + pc - 1) / pc;
@@ -817,6 +822,38 @@ int nfx_flux_series_layers(nfx_pli** self, const void* u, const void* v, const v
     });
 }
 
+// the list-order compact CSR the section gathers through (4 entries per sub-segment, emission order)
+static const Csr& section_csr(const PliDev& p) {
+    NFX_REQUIRE(p.csr[NFX_ORDER_LIST][0].rowptr.p != nullptr, "computeWeights was not called");
+    NFX_REQUIRE(p.has_compact, "nfx_grid_set_cgrid_shape must be called before computeWeights for the flux path");
+    return p.csr[NFX_ORDER_LIST][1];
+}
+
+int nfx_flux_section(nfx_pli** self, const void* u, const void* v, const void* e3u, const void* e3v, int dtype,
+                     int e3_nt, const double* thickness, const double* arc1, const double* arc2, int nt, int nz,
+                     int64_t ld, int nlayers, const int* layer_levels, int sverdrup, double fill, double* section,
+                     void* stream) {
+    return guarded([&] {
+        NFX_REQUIRE(self && *self, "NULL handle");
+        PliDev& p = (*self)->d;
+        NFX_REQUIRE(p.grid, "setGrid was not called");
+        DeviceGuard g(p.grid->device);
+        NFX_REQUIRE(u && v && arc1 && arc2 && section, "NULL pointer");
+        NFX_REQUIRE((e3u == nullptr) == (e3v == nullptr), "e3u and e3v go together");
+        NFX_REQUIRE((thickness != nullptr) != (e3u != nullptr), "needs exactly one of thickness and (e3u, e3v)");
+        NFX_REQUIRE(nt >= 0 && nz > 0, "bad sizes");
+        NFX_REQUIRE(ld >= p.grid->ncell, "ld must be >= the number of cells");
+        NFX_REQUIRE(!e3u || e3_nt == 1 || e3_nt == nt, "e3u/e3v must hold 1 (time-invariant) or nt time steps");
+        check_layer_levels(nz, nlayers, layer_levels);
+        const Csr& c = section_csr(p);
+        if (nt == 0 || p.nsub == 0) return;
+        const cudaStream_t s = (cudaStream_t)stream;
+        const int* levels = device_levels(p, nz, nlayers, layer_levels, s);
+        flux_section(u, v, dtype, thickness, e3u, e3v, e3u && e3_nt != 1 ? (int64_t)nz * ld : 0, arc1, arc2, c.idx.p,
+                     c.w, p.nsub, p.grid->ncell, ld, nt, nz, nlayers, levels, sverdrup, fill, section, s);
+    });
+}
+
 int nfx_edgeflux_to_cell_by_cell(const double* eflux, int nt, int ny, int nx, double* iv, void* stream) {
     return guarded([&] {
         int dev;
@@ -990,18 +1027,45 @@ int nfx_flux_series(nfx_pli** self, const void* u, const void* v, int dtype, con
                               order, eflux, series, stream);
 }
 
-// ---- everything from host buffers: double-buffered H2D staging, K2+K3 per chunk --------------------------
+// ---- everything from host buffers: double-buffered H2D staging, a device pass per chunk ------------------
 // e3u/e3v (optional): per-column scale factors instead of `thickness`.  e3_on_device: borrowed device arrays
 // (e3_nt, nz, ncell) of the dtype of u, v; else host arrays -- e3_nt == 1 is uploaded once per call, e3_nt == nt
-// travels in the chunks next to u and v (same byte order as u, v).  layer_levels (host, nlayers + 1, NULL = the whole
-// column): series (nt, nlayers, M), every chunk runs its nt_chunk * nlayers pseudo-steps.
-static void flux_series_host_impl(nfx_pli** self, const void* u, const void* v, int dtype_flags, const double* thickness,
-                                  const void* e3u, const void* e3v, int e3_nt, int e3_on_device, const double* arc1,
-                                  const double* arc2, int nt, int nz, int sverdrup, double fill, int order,
-                                  int chunk_steps, double* series, int nlayers = 1, const int* layer_levels = nullptr) {
+// travels in the chunks next to u and v (same byte order as u, v).  The pass run on every chunk (K2+K3 for the series,
+// the section gather) is a HostPass; the pipeline stages its output of `values per time step` on the device and
+// copies all of it back at the end.
+
+// one chunk of n time steps on the device: u, v (and e3u, e3v) in native byte order, planes of ncell
+struct HostChunk {
+    const void* u;
+    const void* v;
+    const void* e3u;
+    const void* e3v;
+    int64_t e3_tstride;
+    const double* thickness;   // nullptr with e3u/e3v
+    const double* arc1;
+    const double* arc2;
+    int n;
+    int slot;                  // staging slot of the chunk (0 or 1)
+    double* out;               // device, n * values per time step
+};
+
+struct HostPass {
+    virtual ~HostPass() = default;
+    // argument checks that need the handle; returns the output values per time step (0: nothing to compute)
+    virtual int64_t begin(PliDev& p, int dtype, int nt, int nz) = 0;
+    // after the staging is sized, before the first chunk, on the compute stream
+    virtual void prepare(PliDev& p, int dtype, int nz, int chunk_steps, cudaStream_t ks) = 0;
+    virtual void chunk(PliDev& p, int dtype, int nz, const HostChunk& c, cudaStream_t ks) = 0;
+    // after both streams are synchronised
+    virtual void end(PliDev&, cudaStream_t) {}
+};
+
+static void host_pipeline(nfx_pli** self, const void* u, const void* v, int dtype_flags, const double* thickness,
+                          const void* e3u, const void* e3v, int e3_nt, int e3_on_device, const double* arc1,
+                          const double* arc2, int nt, int nz, int chunk_steps, double* result, HostPass& pass) {
     NFX_REQUIRE(self && *self, "NULL handle");
     const bool e3 = e3u != nullptr || e3v != nullptr;
-    NFX_REQUIRE(u && v && arc1 && arc2 && series, "NULL pointer");
+    NFX_REQUIRE(u && v && arc1 && arc2 && result, "NULL pointer");
     NFX_REQUIRE(e3 ? (e3u && e3v) : thickness != nullptr, "needs the layer thickness or both of e3u, e3v");
     NFX_REQUIRE(nt >= 0 && nz > 0, "bad sizes");
     NFX_REQUIRE(!e3 || e3_nt == 1 || e3_nt == nt, "e3u/e3v must hold 1 (time-invariant) or nt time steps");
@@ -1011,12 +1075,9 @@ static void flux_series_host_impl(nfx_pli** self, const void* u, const void* v, 
     PliDev& p = (*self)->d;
     NFX_REQUIRE(p.grid, "setGrid was not called");
     DeviceGuard g(p.grid->device);
-    const Csr& c = pick_csr(p, order, 1);
-    if (layer_levels) check_layers(p, dtype, nt, nz, nlayers, layer_levels);
+    const int64_t per_step = pass.begin(p, dtype, nt, nz);
     const int64_t ncell = p.grid->ncell;
-    const int M = p.ntransects;
-    const int64_t LM = (int64_t)nlayers * M;   // series values per time step
-    if (nt == 0 || M == 0) return;
+    if (nt == 0 || per_step == 0) return;
     const size_t esize = dtype == NFX_F64 ? 8 : 4;
     const size_t step_bytes = esize * (size_t)nz * (size_t)ncell;
     const bool e3_streamed = e3 && !e3_on_device && e3_nt == nt && nt > 1;
@@ -1041,11 +1102,10 @@ static void flux_series_host_impl(nfx_pli** self, const void* u, const void* v, 
             p.stage_e3v[i].ensure(step_bytes * chunk_steps);
         }
     }
-    p.stage_series.ensure((size_t)nt * LM);
+    p.stage_series.ensure((size_t)nt * per_step);
     p.stage_arc1.ensure(ncell);
     p.stage_arc2.ensure(ncell);
     cudaStream_t cs = p.copy_stream, ks = p.compute_stream;
-    const int* levels = layer_levels ? device_levels(p, nz, nlayers, layer_levels, ks) : nullptr;
     if (!e3) {
         p.stage_thick.ensure(nz);
         NFX_CUDA(cudaMemcpyAsync(p.stage_thick.p, thickness, sizeof(double) * nz, cudaMemcpyHostToDevice, ks));
@@ -1066,10 +1126,7 @@ static void flux_series_host_impl(nfx_pli** self, const void* u, const void* v, 
         d_e3u = p.stage_e3u[0].p;
         d_e3v = p.stage_e3v[0].p;
     }
-    const bool fused = e3 ? use_fused_e3(p, dtype, nullptr, nullptr, nullptr, nullptr, 0, ncell)
-                          : use_fused(p, dtype, nullptr, nullptr, ncell);
-    if (!fused)
-        for (int i = 0; i < 2; ++i) p.stage_eflux[i].ensure((size_t)chunk_steps * nlayers * 2 * ncell);
+    pass.prepare(p, dtype, nz, chunk_steps, ks);
     int slot = 0;
     bool used[2] = {false, false};
     for (int t0 = 0; t0 < nt; t0 += chunk_steps, slot ^= 1) {
@@ -1089,40 +1146,108 @@ static void flux_series_host_impl(nfx_pli** self, const void* u, const void* v, 
         }
         NFX_CUDA(cudaEventRecord(p.ev_ready[slot], cs));
         NFX_CUDA(cudaStreamWaitEvent(ks, p.ev_ready[slot], 0));
-        const void* ce3u = nullptr;
-        const void* ce3v = nullptr;
-        int64_t e3_tstride = 0;
+        HostChunk c{dst[0], dst[1], nullptr, nullptr, 0, e3 ? nullptr : p.stage_thick.p, p.stage_arc1.p,
+                    p.stage_arc2.p, n, slot, p.stage_series.p + (size_t)t0 * per_step};
         if (e3_streamed) {
-            ce3u = dst[2];
-            ce3v = dst[3];
-            e3_tstride = (int64_t)nz * ncell;
+            c.e3u = dst[2];
+            c.e3v = dst[3];
+            c.e3_tstride = (int64_t)nz * ncell;
         } else if (e3) {
-            const bool per_step = e3_on_device && e3_nt == nt && nt > 1;
-            e3_tstride = per_step ? (int64_t)nz * ncell : 0;
-            ce3u = (const unsigned char*)d_e3u + (per_step ? off : 0);
-            ce3v = (const unsigned char*)d_e3v + (per_step ? off : 0);
+            const bool per_step_e3 = e3_on_device && e3_nt == nt && nt > 1;
+            c.e3_tstride = per_step_e3 ? (int64_t)nz * ncell : 0;
+            c.e3u = (const unsigned char*)d_e3u + (per_step_e3 ? off : 0);
+            c.e3v = (const unsigned char*)d_e3v + (per_step_e3 ? off : 0);
         }
-        double* out = p.stage_series.p + (size_t)t0 * LM;
-        if (fused) {
-            flux_series_fast(p, dst[0], dst[1], dtype, e3 ? nullptr : p.stage_thick.p, p.stage_arc1.p, p.stage_arc2.p, n,
-                             nz, ncell, sverdrup, fill, order, out, ks, 0, -1, ce3u, ce3v, e3_tstride, nlayers, levels);
-        } else {
-            edgeflux_assemble_panel(dst[0], dst[1], dtype, e3 ? nullptr : p.stage_thick.p, p.stage_arc1.p,
-                                    p.stage_arc2.p, n, nz, ncell, ncell, sverdrup, fill, p.stage_eflux[slot].p, 0, g_k2opt,
-                                    ks, ce3u, ce3v, e3_tstride, nlayers, levels);
-            csr_integrate(c, M, p.stage_eflux[slot].p, ncell * 2, n * nlayers, out, ks);
-        }
+        pass.chunk(p, dtype, nz, c, ks);
         NFX_CUDA(cudaEventRecord(p.ev_done[slot], ks));
         used[slot] = true;
     }
-    NFX_CUDA(cudaMemcpyAsync(series, p.stage_series.p, sizeof(double) * (size_t)(nt * LM), cudaMemcpyDeviceToHost, ks));
+    NFX_CUDA(cudaMemcpyAsync(result, p.stage_series.p, sizeof(double) * (size_t)nt * per_step, cudaMemcpyDeviceToHost,
+                             ks));
     NFX_CUDA(cudaStreamSynchronize(ks));
     NFX_CUDA(cudaStreamSynchronize(cs));
-    g_last_series_fused = fused ? 1 : 0;
-    if (!fused) g_last_series_sparse = 0;
-    if (fused && fused_error_flag(p, ks) != 0)
-        throw Error(NFX_E_INTERNAL, "fused K2+K3 pass aborted (a bounded wait overflowed)");
+    pass.end(p, ks);
 }
+
+// the series: K2+K3 per chunk (the fused pass where the policy allows), series (nt, nlayers, M).  layer_levels (host,
+// nlayers + 1, NULL = the whole column): every chunk runs its nt_chunk * nlayers pseudo-steps.
+struct SeriesPass : HostPass {
+    bool e3 = false;
+    int sverdrup = 0, order = 0, nlayers = 1;
+    double fill = 0.0;
+    const int* layer_levels = nullptr;
+    const Csr* c = nullptr;
+    const int* levels = nullptr;
+    bool fused = false;
+    int64_t begin(PliDev& p, int dtype, int nt, int nz) override {
+        c = &pick_csr(p, order, 1);
+        if (layer_levels) check_layers(p, dtype, nt, nz, nlayers, layer_levels);
+        return (int64_t)nlayers * p.ntransects;
+    }
+    void prepare(PliDev& p, int dtype, int nz, int chunk_steps, cudaStream_t ks) override {
+        const int64_t ncell = p.grid->ncell;
+        levels = layer_levels ? device_levels(p, nz, nlayers, layer_levels, ks) : nullptr;
+        fused = e3 ? use_fused_e3(p, dtype, nullptr, nullptr, nullptr, nullptr, 0, ncell)
+                   : use_fused(p, dtype, nullptr, nullptr, ncell);
+        if (!fused)
+            for (int i = 0; i < 2; ++i) p.stage_eflux[i].ensure((size_t)chunk_steps * nlayers * 2 * ncell);
+    }
+    void chunk(PliDev& p, int dtype, int nz, const HostChunk& k, cudaStream_t ks) override {
+        const int64_t ncell = p.grid->ncell;
+        if (fused) {
+            flux_series_fast(p, k.u, k.v, dtype, k.thickness, k.arc1, k.arc2, k.n, nz, ncell, sverdrup, fill, order,
+                             k.out, ks, 0, -1, k.e3u, k.e3v, k.e3_tstride, nlayers, levels);
+        } else {
+            edgeflux_assemble_panel(k.u, k.v, dtype, k.thickness, k.arc1, k.arc2, k.n, nz, ncell, ncell, sverdrup, fill,
+                                    p.stage_eflux[k.slot].p, 0, g_k2opt, ks, k.e3u, k.e3v, k.e3_tstride, nlayers,
+                                    levels);
+            csr_integrate(*c, p.ntransects, p.stage_eflux[k.slot].p, ncell * 2, k.n * nlayers, k.out, ks);
+        }
+    }
+    void end(PliDev& p, cudaStream_t ks) override {
+        g_last_series_fused = fused ? 1 : 0;
+        if (!fused) g_last_series_sparse = 0;
+        if (fused && fused_error_flag(p, ks) != 0)
+            throw Error(NFX_E_INTERNAL, "fused K2+K3 pass aborted (a bounded wait overflowed)");
+    }
+};
+
+static void flux_series_host_impl(nfx_pli** self, const void* u, const void* v, int dtype_flags, const double* thickness,
+                                  const void* e3u, const void* e3v, int e3_nt, int e3_on_device, const double* arc1,
+                                  const double* arc2, int nt, int nz, int sverdrup, double fill, int order,
+                                  int chunk_steps, double* series, int nlayers = 1, const int* layer_levels = nullptr) {
+    SeriesPass pass;
+    pass.e3 = e3u != nullptr || e3v != nullptr;
+    pass.sverdrup = sverdrup;
+    pass.order = order;
+    pass.fill = fill;
+    pass.nlayers = nlayers;
+    pass.layer_levels = layer_levels;
+    host_pipeline(self, u, v, dtype_flags, thickness, e3u, e3v, e3_nt, e3_on_device, arc1, arc2, nt, nz, chunk_steps,
+                  series, pass);
+}
+
+// the section: one gather per chunk, section (nt, nlayers, nsub)
+struct SectionPass : HostPass {
+    int sverdrup = 0, nlayers = 1;
+    double fill = 0.0;
+    const int* layer_levels = nullptr;
+    const Csr* c = nullptr;
+    const int* levels = nullptr;
+    int64_t begin(PliDev& p, int, int, int nz) override {
+        check_layer_levels(nz, nlayers, layer_levels);
+        c = &section_csr(p);
+        return (int64_t)nlayers * p.nsub;
+    }
+    void prepare(PliDev& p, int, int nz, int, cudaStream_t ks) override {
+        levels = device_levels(p, nz, nlayers, layer_levels, ks);
+    }
+    void chunk(PliDev& p, int dtype, int nz, const HostChunk& k, cudaStream_t ks) override {
+        const int64_t ncell = p.grid->ncell;
+        flux_section(k.u, k.v, dtype, k.thickness, k.e3u, k.e3v, k.e3_tstride, k.arc1, k.arc2, c->idx.p, c->w, p.nsub,
+                     ncell, ncell, k.n, nz, nlayers, levels, sverdrup, fill, k.out, ks);
+    }
+};
 
 int nfx_flux_series_host(nfx_pli** self, const void* u, const void* v, int dtype_flags, const double* thickness,
                          const double* arc1, const double* arc2, int nt, int nz, int sverdrup, double fill, int order,
@@ -1155,6 +1280,23 @@ int nfx_flux_series_layers_host(nfx_pli** self, const void* u, const void* v, co
         NFX_REQUIRE(layer_levels, "layers: layer_levels is NULL");
         flux_series_host_impl(self, u, v, dtype_flags, thickness, e3u, e3v, e3_nt, e3_on_device, arc1, arc2, nt, nz,
                               sverdrup, fill, order, chunk_steps, series, nlayers, layer_levels);
+    });
+}
+
+int nfx_flux_section_host(nfx_pli** self, const void* u, const void* v, const void* e3u, const void* e3v,
+                          int dtype_flags, int e3_nt, int e3_on_device, const double* thickness, const double* arc1,
+                          const double* arc2, int nt, int nz, int nlayers, const int* layer_levels, int sverdrup,
+                          double fill, int chunk_steps, double* section) {
+    return guarded([&] {
+        NFX_REQUIRE((thickness != nullptr) != (e3u != nullptr || e3v != nullptr),
+                    "needs exactly one of thickness and (e3u, e3v)");
+        SectionPass pass;
+        pass.sverdrup = sverdrup;
+        pass.fill = fill;
+        pass.nlayers = nlayers;
+        pass.layer_levels = layer_levels;
+        host_pipeline(self, u, v, dtype_flags, thickness, e3u, e3v, e3_nt, e3_on_device, arc1, arc2, nt, nz,
+                      chunk_steps, section, pass);
     });
 }
 

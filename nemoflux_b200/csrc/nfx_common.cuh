@@ -276,4 +276,11 @@ double probe_read_bandwidth_groups(const void* buf, int64_t nbytes, const int32_
                                    double* sink, cudaStream_t s);   // nfx_probe.cu
 int k3_group_for(int64_t nnz, int64_t nrows);
 
+// transport section (nfx_section.cu): section (nt, nlayers, nsub) from the list-order compact CSR (idx, w: 4 entries per
+// sub-segment); exactly one of thickness and (e3u, e3v); levels: device (nlayers + 1), nullptr = one layer [0, nz)
+void flux_section(const void* u, const void* v, int dtype, const double* thickness, const void* e3u, const void* e3v,
+                  int64_t e3_tstride, const double* arc1, const double* arc2, const int32_t* idx, const double* w,
+                  int64_t nsub, int64_t ncell, int64_t ld, int nt, int nz, int nlayers, const int* levels, int sverdrup,
+                  double fill, double* section, cudaStream_t s);
+
 }  // namespace nfx

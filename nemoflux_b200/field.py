@@ -309,13 +309,14 @@ class Field(object):
                 return None
             return [nemoflux_gpu.H5DeviceReader(d, self.device) for d in readers]
 
-    def _flux_series_device_decode(self, readers, chunk_steps=0, prefetch=True, layers=None):
-        """flux series of chunked + deflated uo / vo: the COMPRESSED chunks cross PCIe and are inflated, unshuffled and
-        placed on the device (csrc/nfx_inflate.cu), then K2 + K3 run on the decoded slab.  A reader thread copies the
-        compressed chunks of block i + 1 from the memory-mapped files into pinned staging while block i is decoded."""
+    def _flux_series_device_decode(self, readers, chunk_steps, prefetch, fn, shape):
+        """fn over chunked + deflated uo / vo: the COMPRESSED chunks cross PCIe and are inflated, unshuffled and
+        placed on the device (csrc/nfx_inflate.cu), then fn (the series' K2 + K3, or the section) runs on the decoded
+        slab.  A reader thread copies the compressed chunks of block i + 1 from the memory-mapped files into pinned
+        staging while block i is decoded."""
         import threading
         import torch
-        out = numpy.zeros(self._series_shape(layers))
+        out = numpy.zeros(shape)
         esize = readers[0].ds.dtype.itemsize
         step_bytes = esize * self.nz * self.ny * self.nx
         # The decoder works on one chunk per warp and 20 warps fit an SM: a block of as many chunks as the device holds
@@ -353,8 +354,8 @@ class Field(object):
                 ud, vd = readers[0].decode(st[0]), readers[1].decode(st[1])
             if i + 1 < len(blocks) and not prefetch:
                 stage(i + 1)
-            ser = self.pli.fluxSeries(ud, vd, self._d_thickness, self._d_arc1, self._d_arc2, sverdrup=self.sverdrup,
-                                      fill=fill, e3u=self._d_e3u, e3v=self._d_e3v, layers=layers)
+            ser = fn(ud, vd, self._d_thickness, self._d_arc1, self._d_arc2, sverdrup=self.sverdrup, fill=fill,
+                     e3u=self._d_e3u, e3v=self._d_e3v)
             out[t0:t0 + m] = ser.cpu().numpy()
             if th is not None:
                 th.join()
@@ -383,15 +384,33 @@ class Field(object):
         (NFX_BIG_ENDIAN), so the host does no conversion pass.
         Chunked + deflated NetCDF-4 variables (device_decode=None: whenever possible, True: required, False: host zlib)
         travel COMPRESSED and are inflated / unshuffled on the device, see _flux_series_device_decode."""
+        def fn(*args, **kw):
+            return self.pli.fluxSeries(*args, layers=layers, **kw)
+        return self._over_chunks(fn, self._series_shape(layers), chunk_steps, prefetch, device_decode)
+
+    def fluxSection(self, layers=None, chunk_steps=0, prefetch=True, device_decode=None):
+        """(nt, nlayers, nsub) transport section: the flux across every cell crossing of every transect per layer of
+        model levels (layers: level boundaries, see levelsForDepths; None = one layer per level), see
+        PolylineIntegral.fluxSection and getSectionGeometry.  Reads the files as fluxSeries does."""
+        lev = list(range(self.nz + 1)) if layers is None else layers
+
+        def fn(*args, **kw):
+            return self.pli.fluxSection(*args, layers=lev, **kw)
+        return self._over_chunks(fn, (self.nt, len(lev) - 1, self.pli.getNumberOfSubsegments()), chunk_steps, prefetch,
+                                 device_decode)
+
+    def _over_chunks(self, fn, shape, chunk_steps, prefetch, device_decode):
+        """out (shape, time first) = fn(u, v, thickness, arc1, arc2, sverdrup=, fill=, e3u=, e3v=) over chunks of time
+        steps read from the files: the pipeline of fluxSeries"""
         import threading
         import torch
         if device_decode is not False:
             readers = self._device_readers()
             if readers is not None:
-                return self._flux_series_device_decode(readers, chunk_steps, prefetch, layers)
+                return self._flux_series_device_decode(readers, chunk_steps, prefetch, fn, shape)
             if device_decode is True:
                 raise RuntimeError('ERROR: uo / vo are not chunked HDF5 variables with a [shuffle,] [deflate] pipeline')
-        out = numpy.zeros(self._series_shape(layers))
+        out = numpy.zeros(shape)
         dtype = numpy.dtype(self.ncU['uo'].dtype).newbyteorder('=')
         step_bytes = dtype.itemsize * self.nz * self.ny * self.nx
         # ~300 MB per variable and chunk (sweep in profiles/r1_file_e2e_C3.json: 4 f64 / 8 f32 ORCA1 steps): small enough that reading chunk i+1 overlaps the upload of chunk i even
@@ -450,8 +469,8 @@ class Field(object):
                 th = threading.Thread(target=read, args=(i + 1, 1 - slot))
                 th.start()
             nu, nv = views[slot]                    # numpy views of the pinned buffers (kept alive by `bufs`)
-            out[t0:t0 + m] = self.pli.fluxSeries(nu[:m], nv[:m], self.thickness, arc1, arc2, sverdrup=self.sverdrup,
-                                                 fill=state.pop(i), e3u=self._d_e3u, e3v=self._d_e3v, layers=layers)
+            out[t0:t0 + m] = fn(nu[:m], nv[:m], self.thickness, arc1, arc2, sverdrup=self.sverdrup, fill=state.pop(i),
+                                e3u=self._d_e3u, e3v=self._d_e3v)
             if th is not None:
                 th.join()
             elif i + 1 < len(chunks):

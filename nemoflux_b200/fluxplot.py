@@ -1,7 +1,7 @@
 """fluxplot -- drop-in for nemoflux/fluxplot.py: flux time series of every transect (same flags).
 
     python -m nemoflux_b200.fluxplot -t T.nc -u U.nc -v V.nc -i "../data/nz/S*.txt" [-s] [--output series.csv]
-        [--layers "0,10,35,75" | --depthLayers "0,200,1000,6000"]
+        [--layers "0,10,35,75" | --depthLayers "0,200,1000,6000"] [--section section.nc]
 
 The reference loops ``for itime: fld.update(); for pli: pli.getIntegral(...)`` (fluxplot.py:51-59); here the
 whole (nt, M) series comes from Field.fluxSeries() (K2+K3 over chunks of time steps).  The series is printed
@@ -9,12 +9,16 @@ and optionally written as CSV; it is plotted only when matplotlib is importable 
 --layers (model-level boundaries) or --depthLayers (depths in metres, snapped to the nearest level interfaces) split
 every transect's flux by depth: one column per (transect, layer), transect-major, headed label[top-bottom m] with the
 interfaces that were integrated.
+--section FILE.nc also writes the transport section (Field.fluxSection): the flux across every cell crossing of every
+transect per layer (the layers of --layers / --depthLayers, else one per level) as a NetCDF classic (64-bit offset)
+file, see writeSection.
 """
 import argparse
 import os
 
 import numpy
 
+from . import ncio
 from .field import Field
 from .fluxviz import parseTransects
 
@@ -28,6 +32,40 @@ def parseList(text, kind=float):
     if len(vals) < 2:
         raise argparse.ArgumentTypeError(f'expected at least two boundaries, got {text!r}')
     return vals
+
+
+def writeSection(path, fld, layers, units):
+    """transport(time, layer, crossing) of fld.fluxSection(layers) with the crossings' geometry
+    (PolylineIntegral.getSectionGeometry), layer_top / layer_bottom in metres, transect_offsets and time (the record
+    dimension: only one record has to fit the 4 GB of the classic 64-bit-offset format).  Returns the number of
+    crossings."""
+    lev = list(range(fld.nz + 1)) if layers is None else list(layers)
+    sec = fld.fluxSection(layers=lev)
+    geo = fld.pli.getSectionGeometry()
+    iface = fld.layerInterfaces()
+    nsub = sec.shape[2]
+    w = ncio.Writer(path, classic=True)
+    w.createDimension('time', None)
+    w.createDimension('layer', len(lev) - 1)
+    w.createDimension('crossing', nsub)
+    w.createDimension('transect_edge', geo['offsets'].size)
+    tv = fld.timeObj.getValues() if fld.timeObj.getSize() == fld.nt else numpy.arange(fld.nt)
+    tattrs = {k: v for k, v in (('units', fld.timeObj.units), ('calendar', fld.timeObj.calendar)) if v} \
+        if fld.timeObj.getSize() == fld.nt else {'long_name': 'time index'}
+    w.createVariable('time', 'f8', ('time',), attrs=tattrs, data=numpy.asarray(tv, numpy.float64))
+    w.createVariable('transport', 'f8', ('time', 'layer', 'crossing'), data=sec,
+                     attrs={'units': units, 'long_name': 'flux across the cell crossing, per layer of model levels'})
+    w.createVariable('layer_top', 'f8', ('layer',), attrs={'units': 'm'}, data=iface[lev[:-1]])
+    w.createVariable('layer_bottom', 'f8', ('layer',), attrs={'units': 'm'}, data=iface[lev[1:]])
+    w.createVariable('transect_offsets', 'i4', ('transect_edge',), data=geo['offsets'].astype(numpy.int32))
+    for name, unit in (('transect', ''), ('segment', ''), ('cell_j', ''), ('cell_i', ''), ('lon0', 'degrees_east'),
+                       ('lat0', 'degrees_north'), ('lon1', 'degrees_east'), ('lat1', 'degrees_north'),
+                       ('length_km', 'km'), ('distance_km', 'km')):
+        a = geo[name]
+        kind = 'i4' if a.dtype.kind in 'iu' else 'f8'
+        w.createVariable(name, kind, ('crossing',), attrs={'units': unit} if unit else None, data=a.astype(kind))
+    w.close()
+    return nsub
 
 
 def main(argv=None):
@@ -46,6 +84,8 @@ def main(argv=None):
                      help='flux per layer of model levels: level boundaries "0,10,35,75"')
     lay.add_argument('--depthLayers', type=parseList, default=None,
                      help='flux per depth range: depths in metres "0,200,1000,6000", snapped to level interfaces')
+    ap.add_argument('--section', default='',
+                    help='write the transport section (flux per cell crossing and layer) to this NetCDF file')
     a = ap.parse_args(argv)
     pts, names = parseTransects(a.lonLatPoints, a.iFiles)
     print(f'target points:\n {pts}')
@@ -63,6 +103,9 @@ def main(argv=None):
     print('time,' + ','.join(labels) + f'   [{units}]')
     for t, row in zip(timeVals, rows):
         print(f'{t},' + ','.join(f'{x:.15g}' for x in row))
+    if a.section:
+        nsub = writeSection(a.section, fld, layers, units)
+        print(f'section: {nsub} crossings written to {a.section}')
     if a.output:
         with open(a.output, 'w') as f:
             f.write('time,' + ','.join(labels) + '\n')

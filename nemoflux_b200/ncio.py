@@ -270,10 +270,11 @@ def open_dataset(path):
 class Writer(object):
     """createDimension / createVariable subset of netCDF4.Dataset(path, 'w') used by datagen.py:168-208"""
 
-    def __init__(self, path):
+    def __init__(self, path, classic=False):
+        """classic: NetCDF classic with 64-bit offsets whatever the backend (without netCDF4 it always is)"""
         try:
             import netCDF4
-            self._nc4 = netCDF4.Dataset(path, 'w')
+            self._nc4 = netCDF4.Dataset(path, 'w', **({'format': 'NETCDF3_64BIT_OFFSET'} if classic else {}))
             self._h = None
         except ImportError:
             from scipy.io import netcdf_file

@@ -64,6 +64,7 @@ class Grid(object):
         self._h = ctypes.c_void_p()
         _lib.call('nfx_grid_new', ctypes.byref(self._h))
         self._points = None
+        self._cgrid = None
 
     def __del__(self):
         try:
@@ -83,6 +84,7 @@ class Grid(object):
     def setCGridShape(self, ny, nx):
         """structured shape behind the cell ids (cell = j*nx + i); enables the compact flux layout"""
         _lib.call('nfx_grid_set_cgrid_shape', ctypes.byref(self._h), int(ny), int(nx))
+        self._cgrid = (int(ny), int(nx))
 
     def getNumberOfCells(self):
         n = ctypes.c_int64()
@@ -114,6 +116,7 @@ class PolylineIntegral(object):
         _lib.call('nfx_pli_new', ctypes.byref(self._h))
         self._grid = None
         self._batched = False
+        self._polylines = []
 
     def __del__(self):
         try:
@@ -159,6 +162,7 @@ class PolylineIntegral(object):
         _lib.call('nfx_pli_compute_weights_batch', ctypes.byref(self._h), len(arrs), _np_ptr(offsets),
                   _np_ptr(allpts), int(bool(counterclock)))
         self._batched = not single
+        self._polylines = [a.copy() for a in arrs]      # for getSectionGeometry
         return 0
 
     def getIntegral(self, data, placement=CELL_BY_CELL_DATA, order='map'):
@@ -307,8 +311,76 @@ class PolylineIntegral(object):
             raise ValueError('batch_range needs CUDA tensors')
         return self._flux_series_host(u, v, thickness, arc1, arc2, sverdrup, fill, order, chunk_steps, e3u, e3v, lev)
 
-    def _flux_series_device(self, u, v, thickness, arc1, arc2, sverdrup, fill, order, eflux, out, batch_range=None,
-                            e3u=None, e3v=None, lev=None):
+    def fluxSection(self, u, v, thickness, arc1, arc2, sverdrup=False, fill=float('nan'), layers=None, out=None,
+                    chunk_steps=0, e3u=None, e3v=None):
+        """transport section: the flux across every sub-segment (cell crossing) of every transect, per layer of model
+        levels and time step -> (nt, N, nsub), float64.  getSubsegments()['offsets'] splits the last axis by transect
+        (emission order), getSectionGeometry() places every crossing along its transect.
+
+        Arguments as fluxSeries: CUDA tensors (device path, returns a CUDA tensor on the current stream; padded planes
+        and e3u/e3v of 1 or nt steps) or host arrays (chunked through the host-buffer pipeline, native or big-endian,
+        returns numpy).  layers: level boundaries [l0 < ... < lN] as in fluxSeries; None = one layer per level.
+
+        [t, i, s] = ((w0*E[idx0] + w1*E[idx1]) + w2*E[idx2]) + w3*E[idx3] over the 4 edge entries of sub-segment s, with
+        E the layer-i edge flux fluxSeries(layers=, eflux=) writes, bit for bit; a transect's crossings add up to its
+        layered series to rounding."""
+        torch = _torch()
+        lev = _layer_levels(layers)
+        nsub = self.getNumberOfSubsegments()
+        if isinstance(u, torch.Tensor) and u.is_cuda:
+            u, v, nt, nz, ncell, ld = self._device_inputs(u, v, thickness, arc1, arc2, e3u, e3v)
+            use_e3 = e3u is not None or e3v is not None
+            lev = numpy.arange(nz + 1, dtype=numpy.int32) if lev is None else lev
+            shape = (nt, lev.size - 1, nsub)
+            if out is None:
+                out = torch.empty(shape, dtype=torch.float64, device=u.device)
+            _require_cuda(out, torch.float64, 'out')
+            if out.numel() != nt * (lev.size - 1) * nsub:
+                raise ValueError(f'out must hold nt*nlayers*nsub = {nt * (lev.size - 1) * nsub} values')
+            if nt == 0 or nsub == 0:        # nothing to compute: no launch (empty tensors have no device address)
+                return out
+            e3_nt = _check_e3(e3u, e3v, u, nt, nz, ncell, ld) if use_e3 else 0
+            ptr = lambda t: _t_ptr(t) if t is not None else None   # noqa: E731
+            with torch.cuda.device(u.device):
+                _lib.call('nfx_flux_section', ctypes.byref(self._h), _t_ptr(u), _t_ptr(v), ptr(e3u), ptr(e3v),
+                          _dtype_code(str(u.dtype)), e3_nt, None if use_e3 else _t_ptr(thickness), _t_ptr(arc1),
+                          _t_ptr(arc2), nt, nz, ld, lev.size - 1, _np_ptr(lev), int(bool(sverdrup)), float(fill),
+                          _t_ptr(out), _stream_ptr())
+            return out
+        if out is not None:
+            raise ValueError('out is for CUDA inputs; host inputs return a new numpy array')
+        keep = (u, v, e3u, e3v)  # keep pinned tensors alive while numpy views are in use
+        h = _host_inputs(u, v, thickness, arc1, arc2, e3u, e3v)
+        lev = numpy.arange(h.nz + 1, dtype=numpy.int32) if lev is None else lev
+        res = numpy.zeros((h.nt, lev.size - 1, nsub), numpy.float64)
+        pu, pv, e3_nt, on_device = h.e3 if h.e3 is not None else (None, None, 0, False)
+        _lib.call('nfx_flux_section_host', ctypes.byref(self._h), _np_ptr(h.u), _np_ptr(h.v), pu, pv, h.code, e3_nt,
+                  int(on_device), None if h.th is None else _np_ptr(h.th), _np_ptr(h.a1), _np_ptr(h.a2), h.nt, h.nz,
+                  lev.size - 1, _np_ptr(lev), int(bool(sverdrup)), float(fill), int(chunk_steps), _np_ptr(res))
+        del keep
+        return res
+
+    def getNumberOfSubsegments(self):
+        n = ctypes.c_int64()
+        _lib.call('nfx_pli_get_num_subsegments', ctypes.byref(self._h), ctypes.byref(n))
+        return n.value
+
+    def getSectionGeometry(self):
+        """where every crossing of fluxSection lies, host numpy arrays per sub-segment (emission order):
+        transect, segment (index of the polyline segment), cell_j / cell_i (cell = j*nx + i), lon0/lat0 and lon1/lat1
+        (degrees: the crossing's end points on the polyline passed to computeWeights, x-period image shift undone),
+        length_km (great-circle distance between the end points) and distance_km (of the crossing's midpoint from the
+        transect's start: the great-circle lengths of the earlier segments plus the great-circle distance from the
+        segment's start to the midpoint); plus offsets (M+1), as getSubsegments.  Distances are on a sphere of radius
+        6371 km.  Where a transect runs along a grid line the two cells beside it both hold the crossing, with
+        duplicity coefficients getSubsegments()['coeff'] that add up to 1."""
+        if self._grid is None or self._grid._cgrid is None:
+            raise RuntimeError('getSectionGeometry needs Grid.setCGridShape before computeWeights')
+        return sectionGeometry(self.getSubsegments(), self._polylines, self._grid._cgrid[1])
+
+    def _device_inputs(self, u, v, thickness, arc1, arc2, e3u, e3v):
+        """checks of the CUDA-tensor inputs of fluxSeries / fluxSection -> (u, v, nt, nz, ncell, ld), u and v with a
+        time axis"""
         torch = _torch()
         ncells = self._grid.getNumberOfCells() if self._grid is not None else -1
         if u.dim() == 3 and u.shape[2] != ncells and u.shape[1] * u.shape[2] == ncells:
@@ -327,6 +399,13 @@ class PolylineIntegral(object):
             _require_cuda(t, torch.float64, name)
             if t.numel() != n:
                 raise ValueError(f'{name} must hold {n} values, got {t.numel()}')
+        return u, v, nt, nz, ncell, ld
+
+    def _flux_series_device(self, u, v, thickness, arc1, arc2, sverdrup, fill, order, eflux, out, batch_range=None,
+                            e3u=None, e3v=None, lev=None):
+        torch = _torch()
+        u, v, nt, nz, ncell, ld = self._device_inputs(u, v, thickness, arc1, arc2, e3u, e3v)
+        use_e3 = e3u is not None or e3v is not None
         m = self.getNumberOfTransects()
         shape = (nt, m) if lev is None else (nt, lev.size - 1, m)
         if nt == 0 or m == 0:       # nothing to integrate: no launch (empty tensors have no device address)
@@ -393,55 +472,13 @@ class PolylineIntegral(object):
 
     def _flux_series_host(self, u, v, thickness, arc1, arc2, sverdrup, fill, order, chunk_steps, e3u=None, e3v=None,
                           lev=None):
-        torch = _torch()
         keep = (u, v, e3u, e3v)  # keep pinned tensors alive while numpy views are in use
-        if isinstance(u, torch.Tensor):
-            u, v = u.numpy(), v.numpy()
-        u = numpy.asarray(u)
-        v = numpy.asarray(v)
-        if u.ndim == 3:
-            u, v = u[None], v[None]
-        if u.ndim != 4 or u.shape != v.shape or u.dtype != v.dtype:
-            raise ValueError("uo/vo shape does not match (t, z, y, x) or (z, y, x)")
-        code = _dtype_code(u.dtype.newbyteorder('=').name)
-        if not u.dtype.isnative:        # bytes as stored in a NetCDF classic file: swapped on the device
-            code |= _lib.NFX_BIG_ENDIAN
-        if not (u.flags.c_contiguous and v.flags.c_contiguous):
-            u, v = numpy.ascontiguousarray(u), numpy.ascontiguousarray(v)
-        nt, nz, ny, nx = u.shape
-        ncell = ny * nx
-        a1 = numpy.ascontiguousarray(_to_numpy(arc1), numpy.float64).reshape(-1)
-        a2 = numpy.ascontiguousarray(_to_numpy(arc2), numpy.float64).reshape(-1)
-        if a1.size != ncell or a2.size != ncell:
-            raise ValueError('arc1/arc2 sizes do not match uo')
+        h = _host_inputs(u, v, thickness, arc1, arc2, e3u, e3v)
+        u, v, code, nt, nz, a1, a2 = h.u, h.v, h.code, h.nt, h.nz, h.a1, h.a2
         m = self.getNumberOfTransects()
         out = numpy.zeros((nt, m) if lev is None else (nt, lev.size - 1, m), numpy.float64)
-        if e3u is not None or e3v is not None:
-            if e3u is None or e3v is None:
-                raise ValueError('e3u and e3v go together')
-            on_device = isinstance(e3u, torch.Tensor) and e3u.is_cuda
-            if on_device:
-                if not (isinstance(e3v, torch.Tensor) and e3v.is_cuda):
-                    raise ValueError('e3u and e3v must live on the same side')
-                want = torch.float64 if u.dtype.itemsize == 8 else torch.float32
-                for name, t in (('e3u', e3u), ('e3v', e3v)):
-                    if t.dtype != want or not t.is_contiguous():
-                        raise ValueError(f'{name} must be a contiguous CUDA tensor of the dtype of uo')
-                pu, pv = _t_ptr(e3u), _t_ptr(e3v)
-                # the host path runs on the handle's own streams: whatever produced e3u/e3v on the caller's stream
-                # must be complete before they are read there
-                torch.cuda.current_stream(e3u.device).synchronize()
-            else:
-                e3u, e3v = (numpy.asarray(x.numpy() if isinstance(x, torch.Tensor) else x) for x in (e3u, e3v))
-                for name, x in (('e3u', e3u), ('e3v', e3v)):
-                    if x.dtype != u.dtype:
-                        raise ValueError(f'{name} must have the dtype and byte order of uo ({u.dtype}), got {x.dtype}')
-                e3u, e3v = numpy.ascontiguousarray(e3u), numpy.ascontiguousarray(e3v)
-                pu, pv = _np_ptr(e3u), _np_ptr(e3v)
-            n3 = int(e3u.numel() if on_device else e3u.size)
-            if tuple(e3u.shape) != tuple(e3v.shape) or n3 not in (nz * ncell, nt * nz * ncell):
-                raise ValueError('e3u/e3v must hold (1 or nt, nz, ny*nx) values of the same shape')
-            e3_nt = n3 // (nz * ncell)
+        if h.e3 is not None:
+            pu, pv, e3_nt, on_device = h.e3
             if lev is not None:
                 _lib.call('nfx_flux_series_layers_host', ctypes.byref(self._h), _np_ptr(u), _np_ptr(v), pu, pv, code,
                           e3_nt, int(on_device), None, _np_ptr(a1), _np_ptr(a2), nt, nz, lev.size - 1, _np_ptr(lev),
@@ -453,9 +490,7 @@ class PolylineIntegral(object):
                       int(chunk_steps), _np_ptr(out))
             del keep
             return out
-        th = numpy.ascontiguousarray(_to_numpy(thickness), numpy.float64)
-        if th.size != nz:
-            raise ValueError('thickness size does not match uo')
+        th = h.th
         if lev is not None:
             _lib.call('nfx_flux_series_layers_host', ctypes.byref(self._h), _np_ptr(u), _np_ptr(v), None, None, code, 0, 0,
                       _np_ptr(th), _np_ptr(a1), _np_ptr(a2), nt, nz, lev.size - 1, _np_ptr(lev), int(bool(sverdrup)),
@@ -531,6 +566,108 @@ def _to_numpy(x):
     if isinstance(x, torch.Tensor):
         return x.detach().cpu().numpy()
     return numpy.asarray(x)
+
+
+def sectionGeometry(sub, polylines, nx):
+    """PolylineIntegral.getSectionGeometry from its pieces: sub = getSubsegments() (offsets, cell, seg, ta, tb), the
+    polylines (npoints, >= 2) of lon/lat degrees in transect order, nx = cells per grid row"""
+    offs = numpy.asarray(sub['offsets'], numpy.int64)
+    n = int(offs[-1]) if offs.size else 0
+    transect = numpy.repeat(numpy.arange(offs.size - 1, dtype=numpy.int32), numpy.diff(offs))
+    seg = numpy.asarray(sub['seg'], numpy.int64)
+    cell = numpy.asarray(sub['cell'], numpy.int64)
+    p0 = numpy.zeros((n, 2))
+    d = numpy.zeros((n, 2))
+    start_km = numpy.zeros(n)          # distance of the segment's start from the transect's start
+    for m, pts in enumerate(polylines):
+        a, b = offs[m], offs[m + 1]
+        if a == b:
+            continue
+        ll = numpy.asarray(pts, numpy.float64)[:, :2]
+        cum = numpy.concatenate([[0.], numpy.cumsum(_great_circle_km(ll[:-1], ll[1:]))])
+        sm = seg[a:b]
+        p0[a:b] = ll[sm]
+        d[a:b] = ll[sm + 1] - ll[sm]
+        start_km[a:b] = cum[sm]
+    ta, tb = numpy.asarray(sub['ta'], numpy.float64), numpy.asarray(sub['tb'], numpy.float64)
+    e0 = p0 + ta[:, None] * d
+    e1 = p0 + tb[:, None] * d
+    mid = p0 + (0.5 * (ta + tb))[:, None] * d
+    return dict(offsets=offs, transect=transect, segment=numpy.asarray(sub['seg'], numpy.int32), cell_j=cell // nx,
+                cell_i=cell % nx, lon0=e0[:, 0], lat0=e0[:, 1], lon1=e1[:, 0], lat1=e1[:, 1],
+                length_km=_great_circle_km(e0, e1), distance_km=start_km + _great_circle_km(p0, mid))
+
+
+def _great_circle_km(a, b):
+    """great-circle distance in km on a sphere of radius 6371 km between (n, 2) lon/lat points in degrees (haversine)"""
+    a, b = numpy.radians(numpy.asarray(a, numpy.float64)), numpy.radians(numpy.asarray(b, numpy.float64))
+    h = numpy.sin(0.5 * (b[..., 1] - a[..., 1])) ** 2 + \
+        numpy.cos(a[..., 1]) * numpy.cos(b[..., 1]) * numpy.sin(0.5 * (b[..., 0] - a[..., 0])) ** 2
+    return 2. * 6371. * numpy.arcsin(numpy.sqrt(numpy.clip(h, 0., 1.)))
+
+
+class _HostInputs(object):
+    pass
+
+
+def _host_inputs(u, v, thickness, arc1, arc2, e3u, e3v):
+    """checks of the host-array inputs of fluxSeries / fluxSection: u, v (C-contiguous, with a time axis), the dtype
+    code (| NFX_BIG_ENDIAN for big-endian bytes), nt, nz, arc1/arc2 as float64 arrays, and either th (the thickness)
+    or e3 = (pointer of e3u, pointer of e3v, e3_nt, on_device).  The arrays must stay alive for the call."""
+    torch = _torch()
+    if isinstance(u, torch.Tensor):
+        u, v = u.numpy(), v.numpy()
+    u = numpy.asarray(u)
+    v = numpy.asarray(v)
+    if u.ndim == 3:
+        u, v = u[None], v[None]
+    if u.ndim != 4 or u.shape != v.shape or u.dtype != v.dtype:
+        raise ValueError("uo/vo shape does not match (t, z, y, x) or (z, y, x)")
+    code = _dtype_code(u.dtype.newbyteorder('=').name)
+    if not u.dtype.isnative:        # bytes as stored in a NetCDF classic file: swapped on the device
+        code |= _lib.NFX_BIG_ENDIAN
+    if not (u.flags.c_contiguous and v.flags.c_contiguous):
+        u, v = numpy.ascontiguousarray(u), numpy.ascontiguousarray(v)
+    nt, nz, ny, nx = u.shape
+    ncell = ny * nx
+    a1 = numpy.ascontiguousarray(_to_numpy(arc1), numpy.float64).reshape(-1)
+    a2 = numpy.ascontiguousarray(_to_numpy(arc2), numpy.float64).reshape(-1)
+    if a1.size != ncell or a2.size != ncell:
+        raise ValueError('arc1/arc2 sizes do not match uo')
+    h = _HostInputs()
+    h.u, h.v, h.code, h.nt, h.nz, h.a1, h.a2, h.e3, h.th = u, v, code, nt, nz, a1, a2, None, None
+    if e3u is not None or e3v is not None:
+        if e3u is None or e3v is None:
+            raise ValueError('e3u and e3v go together')
+        on_device = isinstance(e3u, torch.Tensor) and e3u.is_cuda
+        if on_device:
+            if not (isinstance(e3v, torch.Tensor) and e3v.is_cuda):
+                raise ValueError('e3u and e3v must live on the same side')
+            want = torch.float64 if u.dtype.itemsize == 8 else torch.float32
+            for name, t in (('e3u', e3u), ('e3v', e3v)):
+                if t.dtype != want or not t.is_contiguous():
+                    raise ValueError(f'{name} must be a contiguous CUDA tensor of the dtype of uo')
+            pu, pv = _t_ptr(e3u), _t_ptr(e3v)
+            # the host path runs on the handle's own streams: whatever produced e3u/e3v on the caller's stream
+            # must be complete before they are read there
+            torch.cuda.current_stream(e3u.device).synchronize()
+        else:
+            e3u, e3v = (numpy.asarray(x.numpy() if isinstance(x, torch.Tensor) else x) for x in (e3u, e3v))
+            for name, x in (('e3u', e3u), ('e3v', e3v)):
+                if x.dtype != u.dtype:
+                    raise ValueError(f'{name} must have the dtype and byte order of uo ({u.dtype}), got {x.dtype}')
+            e3u, e3v = numpy.ascontiguousarray(e3u), numpy.ascontiguousarray(e3v)
+            pu, pv = _np_ptr(e3u), _np_ptr(e3v)
+            h.keep_e3 = (e3u, e3v)
+        n3 = int(e3u.numel() if on_device else e3u.size)
+        if tuple(e3u.shape) != tuple(e3v.shape) or n3 not in (nz * ncell, nt * nz * ncell):
+            raise ValueError('e3u/e3v must hold (1 or nt, nz, ny*nx) values of the same shape')
+        h.e3 = (pu, pv, n3 // (nz * ncell), on_device)
+        return h
+    h.th = numpy.ascontiguousarray(_to_numpy(thickness), numpy.float64)
+    if h.th.size != nz:
+        raise ValueError('thickness size does not match uo')
+    return h
 
 
 def _layer_levels(layers):
