@@ -229,6 +229,22 @@ int nfx_flux_section(nfx_pli** self, const void* u, const void* v, const void* e
                      int e3_nt, const double* thickness, const double* arc1, const double* arc2, int nt, int nz,
                      int64_t ld, int nlayers, const int* layer_levels, int sverdrup, double fill, double* section,
                      void* stream);
+/* Time-mean transport section (extension): the section of nfx_flux_section summed over windows of time steps.
+ * Arguments as nfx_flux_section, plus window_bounds (host, nwindows + 1 step indices relative to the steps passed,
+ * 0 <= b0 < b1 < ... < bK <= nt): window w covers the steps [b_w, b_{w+1}); steps outside [b0, bK) are not read.
+ * sums device (nwindows, nlayers, nsub):
+ *   sums[w, i, s] = (((+0 + sec[b_w, i, s]) + sec[b_w + 1, i, s]) + ...) + sec[b_{w+1} - 1, i, s]
+ * with sec exactly the value nfx_flux_section computes, every add a separate round-to-nearest double add in ascending
+ * step order (so a one-step window of -0 holds +0).  continue_first != 0: window 0 starts from the partial sums already
+ * in sums[0] instead of +0, so a window split over several calls (in step order) sums to the bits of one call.  The
+ * mean is sums / (b_{w+1} - b_w), left to the caller.  Launches split so that gridDim.y <= 65535; asynchronous on
+ * `stream`.  An invalid layering or window list (nt == 0 has none), nwindows * nlayers * nsub overflowing, or any
+ * refusal of nfx_flux_section returns NFX_E_INVALID before anything is launched; no sub-segment launches nothing. */
+int nfx_flux_section_window_sums(nfx_pli** self, const void* u, const void* v, const void* e3u, const void* e3v,
+                                 int dtype, int e3_nt, const double* thickness, const double* arc1, const double* arc2,
+                                 int nt, int nz, int64_t ld, int nlayers, const int* layer_levels, int sverdrup,
+                                 double fill, int nwindows, const int* window_bounds, int continue_first, double* sums,
+                                 void* stream);
 /* The device-path series calls (nfx_flux_series*, nfx_flux_series_range*) are asynchronous on `stream`.  Their fused
  * pass spins on per-batch counters with a bound; a pass that ever overflowed it aborts and leaves NaN in `series`.
  * nfx_pli_series_status synchronises `stream` and reports that: returns 0 with *status = 0 when every pass launched
@@ -317,6 +333,16 @@ int nfx_flux_section_host(nfx_pli** self, const void* u, const void* v, const vo
                           int dtype_flags, int e3_nt, int e3_on_device, const double* thickness, const double* arc1,
                           const double* arc2, int nt, int nz, int nlayers, const int* layer_levels, int sverdrup,
                           double fill, int chunk_steps, double* section);
+/* nfx_flux_section_window_sums from HOST buffers: arguments as nfx_flux_section_host plus nwindows, window_bounds,
+ * continue_first; sums host (nwindows, nlayers, nsub), read (window 0, continue_first) and written.  Only the steps
+ * [b0, bK) are uploaded.  The device stages the window sums a chunk touches (two slots of at most
+ * min(nwindows, chunk_steps + 1) windows, not nt steps) and copies back the windows every chunk completes.  The bits do
+ * not depend on chunk_steps or the byte order. */
+int nfx_flux_section_window_sums_host(nfx_pli** self, const void* u, const void* v, const void* e3u, const void* e3v,
+                                      int dtype_flags, int e3_nt, int e3_on_device, const double* thickness,
+                                      const double* arc1, const double* arc2, int nt, int nz, int nlayers,
+                                      const int* layer_levels, int sverdrup, double fill, int nwindows,
+                                      const int* window_bounds, int continue_first, int chunk_steps, double* sums);
 
 #ifdef __cplusplus
 }

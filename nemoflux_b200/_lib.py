@@ -106,6 +106,10 @@ SIGNATURES = {
                          c_vp, c_int, c_dbl, c_vp, c_vp],
     'nfx_flux_section_host': [P(c_vp), c_vp, c_vp, c_vp, c_vp, c_int, c_int, c_int, c_vp, c_vp, c_vp, c_int, c_int,
                               c_int, c_vp, c_int, c_dbl, c_int, c_vp],
+    'nfx_flux_section_window_sums': [P(c_vp), c_vp, c_vp, c_vp, c_vp, c_int, c_int, c_vp, c_vp, c_vp, c_int, c_int,
+                                     c_i64, c_int, c_vp, c_int, c_dbl, c_int, c_vp, c_int, c_vp, c_vp],
+    'nfx_flux_section_window_sums_host': [P(c_vp), c_vp, c_vp, c_vp, c_vp, c_int, c_int, c_int, c_vp, c_vp, c_vp,
+                                          c_int, c_int, c_int, c_vp, c_int, c_dbl, c_int, c_vp, c_int, c_int, c_vp],
 }
 
 _LIB = None

@@ -1,4 +1,5 @@
 // extern "C" entry points of libnemoflux_gpu.so -- see include/nemoflux_gpu.h.
+#include <algorithm>
 #include <atomic>
 #include <cstdlib>
 #include <cstring>
@@ -854,6 +855,57 @@ int nfx_flux_section(nfx_pli** self, const void* u, const void* v, const void* e
     });
 }
 
+// A window list handed in by the caller (host array): window w = steps [bounds[w], bounds[w+1]) of the nt passed.
+// Checked, with the size of the sums, before anything is launched.
+static void check_windows(int nt, int nwindows, const int* bounds, int nlayers, int64_t nsub) {
+    NFX_REQUIRE(nwindows >= 1, "windows: nwindows must be >= 1");
+    NFX_REQUIRE(bounds, "windows: window_bounds is NULL");
+    NFX_REQUIRE(bounds[0] >= 0 && bounds[nwindows] <= nt,
+                "windows: the step boundaries must lie in [0, nt = " + std::to_string(nt) + "]");
+    for (int i = 0; i < nwindows; ++i)
+        NFX_REQUIRE(bounds[i] < bounds[i + 1], "windows: the step boundaries must be strictly ascending (window " +
+                                                   std::to_string(i) + " is empty)");
+    const int64_t rows = (int64_t)nwindows * std::max(nlayers, 1);
+    NFX_REQUIRE(rows <= 2147483647ll && (nsub == 0 || rows <= (int64_t)(SIZE_MAX / sizeof(double)) / nsub),
+                "windows: nwindows * nlayers * nsub overflows");
+}
+
+// device copy of a (checked) window list, uploaded on `s`
+static const int* device_windows(PliDev& p, int nwindows, const int* bounds, cudaStream_t s) {
+    p.windows.ensure((size_t)nwindows + 1);
+    NFX_CUDA(cudaMemcpyAsync(p.windows.p, bounds, sizeof(int) * ((size_t)nwindows + 1), cudaMemcpyHostToDevice, s));
+    return p.windows.p;
+}
+
+int nfx_flux_section_window_sums(nfx_pli** self, const void* u, const void* v, const void* e3u, const void* e3v,
+                                 int dtype, int e3_nt, const double* thickness, const double* arc1, const double* arc2,
+                                 int nt, int nz, int64_t ld, int nlayers, const int* layer_levels, int sverdrup,
+                                 double fill, int nwindows, const int* window_bounds, int continue_first, double* sums,
+                                 void* stream) {
+    return guarded([&] {
+        NFX_REQUIRE(self && *self, "NULL handle");
+        PliDev& p = (*self)->d;
+        NFX_REQUIRE(p.grid, "setGrid was not called");
+        DeviceGuard g(p.grid->device);
+        NFX_REQUIRE(nt >= 0 && nz > 0, "bad sizes");
+        check_layer_levels(nz, nlayers, layer_levels);
+        const Csr& c = section_csr(p);
+        check_windows(nt, nwindows, window_bounds, nlayers, p.nsub);
+        NFX_REQUIRE(u && v && arc1 && arc2 && (sums || p.nsub == 0), "NULL pointer");
+        NFX_REQUIRE((e3u == nullptr) == (e3v == nullptr), "e3u and e3v go together");
+        NFX_REQUIRE((thickness != nullptr) != (e3u != nullptr), "needs exactly one of thickness and (e3u, e3v)");
+        NFX_REQUIRE(ld >= p.grid->ncell, "ld must be >= the number of cells");
+        NFX_REQUIRE(!e3u || e3_nt == 1 || e3_nt == nt, "e3u/e3v must hold 1 (time-invariant) or nt time steps");
+        if (p.nsub == 0) return;
+        const cudaStream_t s = (cudaStream_t)stream;
+        const int* levels = device_levels(p, nz, nlayers, layer_levels, s);
+        const int* bounds = device_windows(p, nwindows, window_bounds, s);
+        flux_section_windows(u, v, dtype, thickness, e3u, e3v, e3u && e3_nt != 1 ? (int64_t)nz * ld : 0, arc1, arc2,
+                             c.idx.p, c.w, p.nsub, p.grid->ncell, ld, nz, nlayers, levels, sverdrup, fill, bounds, 0,
+                             nwindows, 0, nt, continue_first ? 1 : 0, sums, s);
+    });
+}
+
 int nfx_edgeflux_to_cell_by_cell(const double* eflux, int nt, int ny, int nx, double* iv, void* stream) {
     return guarded([&] {
         int dev;
@@ -1031,8 +1083,8 @@ int nfx_flux_series(nfx_pli** self, const void* u, const void* v, int dtype, con
 // e3u/e3v (optional): per-column scale factors instead of `thickness`.  e3_on_device: borrowed device arrays
 // (e3_nt, nz, ncell) of the dtype of u, v; else host arrays -- e3_nt == 1 is uploaded once per call, e3_nt == nt
 // travels in the chunks next to u and v (same byte order as u, v).  The pass run on every chunk (K2+K3 for the series,
-// the section gather) is a HostPass; the pipeline stages its output of `values per time step` on the device and
-// copies all of it back at the end.
+// the section gather, the windowed section) is a HostPass, which stages its output on the device and copies it back:
+// the per-step passes all of it at the end, the windowed section the windows every chunk completes.
 
 // one chunk of n time steps on the device: u, v (and e3u, e3v) in native byte order, planes of ncell
 struct HostChunk {
@@ -1044,20 +1096,39 @@ struct HostChunk {
     const double* thickness;   // nullptr with e3u/e3v
     const double* arc1;
     const double* arc2;
+    int t0;                    // first time step of the chunk
     int n;
     int slot;                  // staging slot of the chunk (0 or 1)
-    double* out;               // device, n * values per time step
 };
 
 struct HostPass {
     virtual ~HostPass() = default;
-    // argument checks that need the handle; returns the output values per time step (0: nothing to compute)
-    virtual int64_t begin(PliDev& p, int dtype, int nt, int nz) = 0;
-    // after the staging is sized, before the first chunk, on the compute stream
-    virtual void prepare(PliDev& p, int dtype, int nz, int chunk_steps, cudaStream_t ks) = 0;
+    // argument checks that need the handle; false: nothing to compute
+    virtual bool begin(PliDev& p, int dtype, int nt, int nz) = 0;
+    // after the input staging is sized, before the first chunk, on the compute stream
+    virtual void prepare(PliDev& p, int dtype, int nt, int nz, int chunk_steps, double* result, cudaStream_t ks) = 0;
     virtual void chunk(PliDev& p, int dtype, int nz, const HostChunk& c, cudaStream_t ks) = 0;
+    // chunk c is launched (its ev_done recorded) and so is the one after it, if any: copy c's finished output back
+    virtual void retire(PliDev&, const HostChunk&, double* /*result*/, cudaStream_t /*cs*/) {}
+    // every chunk is launched and retired, before the streams are synchronised
+    virtual void finish(PliDev&, double* /*result*/, cudaStream_t /*ks*/) {}
     // after both streams are synchronised
     virtual void end(PliDev&, cudaStream_t) {}
+};
+
+// a pass with a fixed number of output values per time step: stage_series holds all of them, copied back at the end
+struct PerStepPass : HostPass {
+    int64_t per_step = 0;
+    int nt = 0;
+    double* out(PliDev& p, const HostChunk& c) const { return p.stage_series.p + (size_t)c.t0 * per_step; }
+    void stage(PliDev& p, int nt_) {
+        nt = nt_;
+        p.stage_series.ensure((size_t)nt * per_step);
+    }
+    void finish(PliDev& p, double* result, cudaStream_t ks) override {
+        NFX_CUDA(cudaMemcpyAsync(result, p.stage_series.p, sizeof(double) * (size_t)nt * per_step,
+                                 cudaMemcpyDeviceToHost, ks));
+    }
 };
 
 static void host_pipeline(nfx_pli** self, const void* u, const void* v, int dtype_flags, const double* thickness,
@@ -1075,9 +1146,9 @@ static void host_pipeline(nfx_pli** self, const void* u, const void* v, int dtyp
     PliDev& p = (*self)->d;
     NFX_REQUIRE(p.grid, "setGrid was not called");
     DeviceGuard g(p.grid->device);
-    const int64_t per_step = pass.begin(p, dtype, nt, nz);
+    const bool work = pass.begin(p, dtype, nt, nz);
     const int64_t ncell = p.grid->ncell;
-    if (nt == 0 || per_step == 0) return;
+    if (nt == 0 || !work) return;
     const size_t esize = dtype == NFX_F64 ? 8 : 4;
     const size_t step_bytes = esize * (size_t)nz * (size_t)ncell;
     const bool e3_streamed = e3 && !e3_on_device && e3_nt == nt && nt > 1;
@@ -1102,7 +1173,6 @@ static void host_pipeline(nfx_pli** self, const void* u, const void* v, int dtyp
             p.stage_e3v[i].ensure(step_bytes * chunk_steps);
         }
     }
-    p.stage_series.ensure((size_t)nt * per_step);
     p.stage_arc1.ensure(ncell);
     p.stage_arc2.ensure(ncell);
     cudaStream_t cs = p.copy_stream, ks = p.compute_stream;
@@ -1126,9 +1196,10 @@ static void host_pipeline(nfx_pli** self, const void* u, const void* v, int dtyp
         d_e3u = p.stage_e3u[0].p;
         d_e3v = p.stage_e3v[0].p;
     }
-    pass.prepare(p, dtype, nz, chunk_steps, ks);
+    pass.prepare(p, dtype, nt, nz, chunk_steps, result, ks);
     int slot = 0;
     bool used[2] = {false, false};
+    HostChunk prev{};
     for (int t0 = 0; t0 < nt; t0 += chunk_steps, slot ^= 1) {
         const int n = std::min(chunk_steps, nt - t0);
         if (used[slot]) NFX_CUDA(cudaStreamWaitEvent(cs, p.ev_done[slot], 0));
@@ -1147,7 +1218,7 @@ static void host_pipeline(nfx_pli** self, const void* u, const void* v, int dtyp
         NFX_CUDA(cudaEventRecord(p.ev_ready[slot], cs));
         NFX_CUDA(cudaStreamWaitEvent(ks, p.ev_ready[slot], 0));
         HostChunk c{dst[0], dst[1], nullptr, nullptr, 0, e3 ? nullptr : p.stage_thick.p, p.stage_arc1.p,
-                    p.stage_arc2.p, n, slot, p.stage_series.p + (size_t)t0 * per_step};
+                    p.stage_arc2.p, t0, n, slot};
         if (e3_streamed) {
             c.e3u = dst[2];
             c.e3v = dst[3];
@@ -1160,10 +1231,14 @@ static void host_pipeline(nfx_pli** self, const void* u, const void* v, int dtyp
         }
         pass.chunk(p, dtype, nz, c, ks);
         NFX_CUDA(cudaEventRecord(p.ev_done[slot], ks));
+        // the previous chunk's output goes back while this one runs (behind the previous chunk's ev_done, on the copy
+        // stream: the next chunk's inputs are queued behind it, and so is the next chunk that reuses its slot)
+        if (t0 > 0) pass.retire(p, prev, result, cs);
         used[slot] = true;
+        prev = c;
     }
-    NFX_CUDA(cudaMemcpyAsync(result, p.stage_series.p, sizeof(double) * (size_t)nt * per_step, cudaMemcpyDeviceToHost,
-                             ks));
+    pass.retire(p, prev, result, cs);
+    pass.finish(p, result, ks);
     NFX_CUDA(cudaStreamSynchronize(ks));
     NFX_CUDA(cudaStreamSynchronize(cs));
     pass.end(p, ks);
@@ -1171,7 +1246,7 @@ static void host_pipeline(nfx_pli** self, const void* u, const void* v, int dtyp
 
 // the series: K2+K3 per chunk (the fused pass where the policy allows), series (nt, nlayers, M).  layer_levels (host,
 // nlayers + 1, NULL = the whole column): every chunk runs its nt_chunk * nlayers pseudo-steps.
-struct SeriesPass : HostPass {
+struct SeriesPass : PerStepPass {
     bool e3 = false;
     int sverdrup = 0, order = 0, nlayers = 1;
     double fill = 0.0;
@@ -1179,13 +1254,15 @@ struct SeriesPass : HostPass {
     const Csr* c = nullptr;
     const int* levels = nullptr;
     bool fused = false;
-    int64_t begin(PliDev& p, int dtype, int nt, int nz) override {
+    bool begin(PliDev& p, int dtype, int nt_, int nz) override {
         c = &pick_csr(p, order, 1);
-        if (layer_levels) check_layers(p, dtype, nt, nz, nlayers, layer_levels);
-        return (int64_t)nlayers * p.ntransects;
+        if (layer_levels) check_layers(p, dtype, nt_, nz, nlayers, layer_levels);
+        per_step = (int64_t)nlayers * p.ntransects;
+        return per_step != 0;
     }
-    void prepare(PliDev& p, int dtype, int nz, int chunk_steps, cudaStream_t ks) override {
+    void prepare(PliDev& p, int dtype, int nt_, int nz, int chunk_steps, double*, cudaStream_t ks) override {
         const int64_t ncell = p.grid->ncell;
+        stage(p, nt_);
         levels = layer_levels ? device_levels(p, nz, nlayers, layer_levels, ks) : nullptr;
         fused = e3 ? use_fused_e3(p, dtype, nullptr, nullptr, nullptr, nullptr, 0, ncell)
                    : use_fused(p, dtype, nullptr, nullptr, ncell);
@@ -1196,12 +1273,12 @@ struct SeriesPass : HostPass {
         const int64_t ncell = p.grid->ncell;
         if (fused) {
             flux_series_fast(p, k.u, k.v, dtype, k.thickness, k.arc1, k.arc2, k.n, nz, ncell, sverdrup, fill, order,
-                             k.out, ks, 0, -1, k.e3u, k.e3v, k.e3_tstride, nlayers, levels);
+                             out(p, k), ks, 0, -1, k.e3u, k.e3v, k.e3_tstride, nlayers, levels);
         } else {
             edgeflux_assemble_panel(k.u, k.v, dtype, k.thickness, k.arc1, k.arc2, k.n, nz, ncell, ncell, sverdrup, fill,
                                     p.stage_eflux[k.slot].p, 0, g_k2opt, ks, k.e3u, k.e3v, k.e3_tstride, nlayers,
                                     levels);
-            csr_integrate(*c, p.ntransects, p.stage_eflux[k.slot].p, ncell * 2, k.n * nlayers, k.out, ks);
+            csr_integrate(*c, p.ntransects, p.stage_eflux[k.slot].p, ncell * 2, k.n * nlayers, out(p, k), ks);
         }
     }
     void end(PliDev& p, cudaStream_t ks) override {
@@ -1228,24 +1305,90 @@ static void flux_series_host_impl(nfx_pli** self, const void* u, const void* v, 
 }
 
 // the section: one gather per chunk, section (nt, nlayers, nsub)
-struct SectionPass : HostPass {
+struct SectionPass : PerStepPass {
     int sverdrup = 0, nlayers = 1;
     double fill = 0.0;
     const int* layer_levels = nullptr;
     const Csr* c = nullptr;
     const int* levels = nullptr;
-    int64_t begin(PliDev& p, int, int, int nz) override {
+    bool begin(PliDev& p, int, int, int nz) override {
         check_layer_levels(nz, nlayers, layer_levels);
         c = &section_csr(p);
-        return (int64_t)nlayers * p.nsub;
+        per_step = (int64_t)nlayers * p.nsub;
+        return per_step != 0;
     }
-    void prepare(PliDev& p, int, int nz, int, cudaStream_t ks) override {
+    void prepare(PliDev& p, int, int nt_, int nz, int, double*, cudaStream_t ks) override {
+        stage(p, nt_);
         levels = device_levels(p, nz, nlayers, layer_levels, ks);
     }
     void chunk(PliDev& p, int dtype, int nz, const HostChunk& k, cudaStream_t ks) override {
         const int64_t ncell = p.grid->ncell;
         flux_section(k.u, k.v, dtype, k.thickness, k.e3u, k.e3v, k.e3_tstride, k.arc1, k.arc2, c->idx.p, c->w, p.nsub,
-                     ncell, ncell, k.n, nz, nlayers, levels, sverdrup, fill, k.out, ks);
+                     ncell, ncell, k.n, nz, nlayers, levels, sverdrup, fill, out(p, k), ks);
+    }
+};
+
+// the windowed section: window sums (nwindows, nlayers, nsub), bounds relative to the steps the pipeline runs (the
+// entry point drops the steps before the first window and after the last, so bounds[0] == 0 and bounds[nw] == nt).
+// A chunk touches the windows [wa, wb) (wa: the window holding its first step); their sums are staged in the chunk's
+// slot of stage_windows, window wa in row 0.  When window wa began in an earlier chunk its partial sums are carried
+// over from the last row of the previous slot (or, for the first chunk with continue_first, from the host), and the
+// kernel continues them.  retire() copies back the windows a chunk completes.
+struct WindowPass : HostPass {
+    int sverdrup = 0, nlayers = 1, nwin = 0, continue_first = 0;
+    double fill = 0.0;
+    const int* layer_levels = nullptr;
+    std::vector<int> bounds;        // host, nwin + 1
+    const Csr* c = nullptr;
+    const int* levels = nullptr;
+    const int* d_bounds = nullptr;
+    int64_t row = 0;                // values per window: nlayers * nsub
+    int prev_wa = 0;                // first window of the previous chunk
+    // windows [wa, wb) touched by the steps [t0, t0 + n)
+    void touched(int t0, int n, int& wa, int& wb) const {
+        wa = (int)(std::upper_bound(bounds.begin(), bounds.end(), t0) - bounds.begin()) - 1;
+        wb = (int)(std::lower_bound(bounds.begin(), bounds.end(), t0 + n) - bounds.begin());
+    }
+    bool begin(PliDev& p, int, int, int nz) override {
+        check_layer_levels(nz, nlayers, layer_levels);
+        c = &section_csr(p);
+        row = (int64_t)nlayers * p.nsub;
+        return row != 0;
+    }
+    void prepare(PliDev& p, int, int nt, int nz, int chunk_steps, double* result, cudaStream_t ks) override {
+        int most = 1, wa, wb;
+        for (int t0 = 0; t0 < nt; t0 += chunk_steps) {
+            touched(t0, std::min(chunk_steps, nt - t0), wa, wb);
+            most = std::max(most, wb - wa);
+        }
+        for (int i = 0; i < 2; ++i) p.stage_windows[i].ensure((size_t)most * row);
+        levels = device_levels(p, nz, nlayers, layer_levels, ks);
+        d_bounds = device_windows(p, nwin, bounds.data(), ks);
+        if (continue_first)
+            NFX_CUDA(cudaMemcpyAsync(p.stage_windows[0].p, result, sizeof(double) * row, cudaMemcpyHostToDevice, ks));
+    }
+    void chunk(PliDev& p, int dtype, int nz, const HostChunk& k, cudaStream_t ks) override {
+        int wa, wb;
+        touched(k.t0, k.n, wa, wb);
+        const bool cont = k.t0 == 0 ? continue_first != 0 : bounds[wa] < k.t0;
+        if (cont && k.t0 > 0)          // window wa is the last one the previous chunk touched, in its row wa - prev_wa
+            NFX_CUDA(cudaMemcpyAsync(p.stage_windows[k.slot].p,
+                                     p.stage_windows[k.slot ^ 1].p + (size_t)(wa - prev_wa) * row, sizeof(double) * row,
+                                     cudaMemcpyDeviceToDevice, ks));
+        const int64_t ncell = p.grid->ncell;
+        flux_section_windows(k.u, k.v, dtype, k.thickness, k.e3u, k.e3v, k.e3_tstride, k.arc1, k.arc2, c->idx.p, c->w,
+                             p.nsub, ncell, ncell, nz, nlayers, levels, sverdrup, fill, d_bounds, wa, wb - wa, k.t0,
+                             k.t0 + k.n, cont ? 1 : 0, p.stage_windows[k.slot].p, ks);
+        prev_wa = wa;
+    }
+    void retire(PliDev& p, const HostChunk& k, double* result, cudaStream_t cs) override {
+        int wa, wb;
+        touched(k.t0, k.n, wa, wb);
+        const int done = bounds[wb] == k.t0 + k.n ? wb : wb - 1;     // the windows that end in this chunk: [wa, done)
+        if (done <= wa) return;
+        NFX_CUDA(cudaStreamWaitEvent(cs, p.ev_done[k.slot], 0));
+        NFX_CUDA(cudaMemcpyAsync(result + (size_t)wa * row, p.stage_windows[k.slot].p,
+                                 sizeof(double) * (size_t)(done - wa) * row, cudaMemcpyDeviceToHost, cs));
     }
 };
 
@@ -1297,6 +1440,43 @@ int nfx_flux_section_host(nfx_pli** self, const void* u, const void* v, const vo
         pass.layer_levels = layer_levels;
         host_pipeline(self, u, v, dtype_flags, thickness, e3u, e3v, e3_nt, e3_on_device, arc1, arc2, nt, nz,
                       chunk_steps, section, pass);
+    });
+}
+
+int nfx_flux_section_window_sums_host(nfx_pli** self, const void* u, const void* v, const void* e3u, const void* e3v,
+                                      int dtype_flags, int e3_nt, int e3_on_device, const double* thickness,
+                                      const double* arc1, const double* arc2, int nt, int nz, int nlayers,
+                                      const int* layer_levels, int sverdrup, double fill, int nwindows,
+                                      const int* window_bounds, int continue_first, int chunk_steps, double* sums) {
+    return guarded([&] {
+        NFX_REQUIRE(self && *self, "NULL handle");
+        NFX_REQUIRE((thickness != nullptr) != (e3u != nullptr || e3v != nullptr),
+                    "needs exactly one of thickness and (e3u, e3v)");
+        PliDev& p = (*self)->d;
+        NFX_REQUIRE(p.grid, "setGrid was not called");
+        NFX_REQUIRE(nt >= 0 && nz > 0, "bad sizes");
+        const int dtype = dtype_flags & ~NFX_BIG_ENDIAN;
+        NFX_REQUIRE(dtype == NFX_F64 || dtype == NFX_F32, "dtype must be NFX_F64 or NFX_F32 (optionally | NFX_BIG_ENDIAN)");
+        check_layer_levels(nz, nlayers, layer_levels);
+        check_windows(nt, nwindows, window_bounds, nlayers, p.nsub);
+        NFX_REQUIRE(u && v && sums, "NULL pointer");
+        // only the steps [b0, bK) are read: the pipeline runs on them, the bounds relative to b0
+        const int b0 = window_bounds[0], n = window_bounds[nwindows] - b0;
+        const size_t off = (size_t)b0 * (dtype == NFX_F64 ? 8 : 4) * (size_t)nz * (size_t)p.grid->ncell;
+        const bool e3_per_step = (e3u || e3v) && e3_nt == nt && nt > 1;
+        auto shift = [&](const void* x, bool by) { return x && by ? (const void*)((const unsigned char*)x + off) : x; };
+        WindowPass pass;
+        pass.sverdrup = sverdrup;
+        pass.fill = fill;
+        pass.nlayers = nlayers;
+        pass.layer_levels = layer_levels;
+        pass.nwin = nwindows;
+        pass.continue_first = continue_first;
+        pass.bounds.resize((size_t)nwindows + 1);
+        for (int i = 0; i <= nwindows; ++i) pass.bounds[i] = window_bounds[i] - b0;
+        host_pipeline(self, shift(u, true), shift(v, true), dtype_flags, thickness, shift(e3u, e3_per_step),
+                      shift(e3v, e3_per_step), e3_per_step ? n : e3_nt, e3_on_device, arc1, arc2, n, nz, chunk_steps,
+                      sums, pass);
     });
 }
 

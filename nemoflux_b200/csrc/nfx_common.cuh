@@ -193,11 +193,13 @@ struct PliDev {
     std::vector<int64_t> h_sub_offsets, h_map_offsets;
     DevBuf<int> levels;            // layered series: device copy of the layer boundaries of the last layered call
     std::vector<int> h_levels;     // ... and its host copy (the upload is skipped when they are unchanged)
+    DevBuf<int> windows;           // time-mean section: device copy of the window bounds of the last call
     // scratch reused by the host-buffer entry points
     DevBuf<double> scratch_data, scratch_res;
     // persistent staging of nfx_flux_series_host (two slots)
     DevBuf<unsigned char> stage_u[2], stage_v[2], stage_e3u[2], stage_e3v[2];
     DevBuf<double> stage_eflux[2], stage_series, stage_thick, stage_arc1, stage_arc2;
+    DevBuf<double> stage_windows[2];   // time-mean section: the window sums a chunk touches (two slots)
     cudaStream_t copy_stream = nullptr, compute_stream = nullptr;
     cudaEvent_t ev_ready[2] = {nullptr, nullptr}, ev_done[2] = {nullptr, nullptr};
 };
@@ -282,5 +284,14 @@ void flux_section(const void* u, const void* v, int dtype, const double* thickne
                   int64_t e3_tstride, const double* arc1, const double* arc2, const int32_t* idx, const double* w,
                   int64_t nsub, int64_t ncell, int64_t ld, int nt, int nz, int nlayers, const int* levels, int sverdrup,
                   double fill, double* section, cudaStream_t s);
+// ... summed over windows of time steps (nfx_section.cu): sums ((nwin, nlayers, nsub) from window w0 on) += the section
+// of the steps [bounds[w], bounds[w+1]) clipped to [t_first, t_end), in ascending step order; u, v (and per-step e3) hold
+// the steps from t_first on; bounds: device (all windows + 1); continue_first: window w0 continues the partial sums in
+// `sums`, else every window starts from +0
+void flux_section_windows(const void* u, const void* v, int dtype, const double* thickness, const void* e3u,
+                          const void* e3v, int64_t e3_tstride, const double* arc1, const double* arc2,
+                          const int32_t* idx, const double* w, int64_t nsub, int64_t ncell, int64_t ld, int nz,
+                          int nlayers, const int* levels, int sverdrup, double fill, const int* bounds, int w0, int nwin,
+                          int t_first, int t_end, int continue_first, double* sums, cudaStream_t s);
 
 }  // namespace nfx

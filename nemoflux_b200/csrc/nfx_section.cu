@@ -123,6 +123,123 @@ k_flux_section(const T* __restrict__ u, const T* __restrict__ v, const T* __rest
     }
 }
 
+// Time-mean section: the sums over windows of time steps of the section above.  One thread per (window, layer,
+// sub-segment), consecutive sub-segments in consecutive lanes; y = window * nlayers + layer.  Window w covers the steps
+// [bounds[w], bounds[w+1]) clipped to the steps [t_first, t_end) the arrays hold (u, v, e3 start at step t_first).
+// The thread walks the window's steps in ascending order; per step it sums the layer's levels into the 4 column sums,
+// forms the step's section value with the operations of k_flux_section and adds it to the running window sum:
+//   sum = (((+0 | the stored partial sum) + sec[t0]) + sec[t0 + 1]) + ...       (every add a __dadd_rn)
+// The first window the launch covers (w0) continues the partial sum stored in `sums` when continue_first is set.  One
+// streaming store per (window, layer, sub-segment); the loads per (step, level, edge) are those of k_flux_section.
+template <typename T, bool E3>
+__global__ void __launch_bounds__(kSectionBlock, SectionShape<T, E3>::ctas)
+k_flux_section_windows(const T* __restrict__ u, const T* __restrict__ v, const T* __restrict__ e3u,
+                       const T* __restrict__ e3v, int64_t e3_tstride, const double* __restrict__ dz,
+                       const double* __restrict__ arc1, const double* __restrict__ arc2,
+                       const int32_t* __restrict__ idx, const double* __restrict__ w, int64_t nsub, int64_t ncell,
+                       int64_t ld, int nz, int nlayers, const int* __restrict__ levels, double scale, int use_scale,
+                       T fill, int has_fill, const int* __restrict__ bounds, int w0, int t_first, int t_end,
+                       int continue_first, int64_t y0, double* __restrict__ sums) {
+    constexpr int UNROLL = SectionShape<T, E3>::unroll;
+    extern __shared__ double s_dz[];                        // [nz] dz (without E3), then [nlayers + 1] boundaries
+    int* s_lev = reinterpret_cast<int*>(s_dz + (E3 ? 0 : nz));
+    if constexpr (!E3)
+        for (int k = threadIdx.x; k < nz; k += kSectionBlock) s_dz[k] = dz[k];
+    for (int i = threadIdx.x; i <= nlayers; i += kSectionBlock)
+        s_lev[i] = levels ? levels[i] : (i == 0 ? 0 : nz);
+    __syncthreads();
+    const int64_t s = (int64_t)blockIdx.x * kSectionBlock + threadIdx.x;
+    if (s >= nsub) return;
+    const int64_t y = y0 + blockIdx.y;                      // (window - w0) * nlayers + layer
+    const int win = w0 + (int)(y / nlayers);
+    const int layer = (int)(y % nlayers);
+    const int tb = max(bounds[win], t_first) - t_first, te = min(bounds[win + 1], t_end) - t_first;
+    const int kbeg = s_lev[layer], kend = s_lev[layer + 1];
+    const T* pc[4];        // column of every edge at level kbeg of step 0
+    const T* pe[4];
+    double arc[4], wt[4];
+    bool live[4];
+#pragma unroll
+    for (int e = 0; e < 4; ++e) {
+        const int32_t j = idx[4 * s + e];
+        live[e] = j >= 0;
+        const bool isv = j >= ncell;
+        const int64_t col = !live[e] ? 0 : isv ? j - ncell : j;
+        pc[e] = (isv ? v : u) + (int64_t)kbeg * ld + col;
+        pe[e] = E3 ? (isv ? e3v : e3u) + (int64_t)kbeg * ld + col : nullptr;
+        arc[e] = !live[e] ? 0.0 : isv ? -arc2[col] : arc1[col];
+        wt[e] = w[4 * s + e];
+    }
+    double* out = sums + y * nsub + s;
+    double total = continue_first && y < nlayers ? __ldcs(out) : 0.0;
+    for (int t = tb; t < te; ++t) {
+        const int64_t tu = (int64_t)t * nz * ld, tx = (int64_t)t * e3_tstride;
+        double acc[4] = {0.0, 0.0, 0.0, 0.0};
+        auto level = [&](int kk, const T (&x)[4], const T (&ex)[4]) {
+            const double d = E3 ? 0.0 : s_dz[kk];
+#pragma unroll
+            for (int e = 0; e < 4; ++e) {
+                const double de = E3 ? clean<T>(ex[e], fill, has_fill) : d;
+                acc[e] = __dadd_rn(acc[e], __dmul_rn(de, clean<T>(x[e], fill, has_fill)));
+            }
+        };
+        int k = kbeg;
+        for (; k + UNROLL <= kend; k += UNROLL) {
+            T x[UNROLL][4], ex[UNROLL][4];
+#pragma unroll
+            for (int q = 0; q < UNROLL; ++q)
+#pragma unroll
+                for (int e = 0; e < 4; ++e) {
+                    x[q][e] = __ldg(pc[e] + tu + (int64_t)(k - kbeg + q) * ld);
+                    if constexpr (E3) ex[q][e] = __ldg(pe[e] + tx + (int64_t)(k - kbeg + q) * ld);
+                }
+#pragma unroll
+            for (int q = 0; q < UNROLL; ++q) level(k + q, x[q], ex[q]);
+        }
+        for (; k < kend; ++k) {
+            T x[4], ex[4];
+#pragma unroll
+            for (int e = 0; e < 4; ++e) {
+                x[e] = __ldg(pc[e] + tu + (int64_t)(k - kbeg) * ld);
+                if constexpr (E3) ex[e] = __ldg(pe[e] + tx + (int64_t)(k - kbeg) * ld);
+            }
+            level(k, x, ex);
+        }
+        double r = 0.0;
+#pragma unroll
+        for (int e = 0; e < 4; ++e) {
+            double f = __dmul_rn(acc[e], arc[e]);
+            if (use_scale) f = __dmul_rn(f, scale);
+            f = live[e] ? f : 0.0;
+            r = e == 0 ? __dmul_rn(wt[0], f) : __dadd_rn(r, __dmul_rn(wt[e], f));
+        }
+        total = __dadd_rn(total, r);
+    }
+    __stcs(out, total);
+}
+
+template <typename T, bool E3>
+void launch_section_windows(const void* u, const void* v, const void* e3u, const void* e3v, int64_t e3_tstride,
+                            const double* dz, const double* arc1, const double* arc2, const int32_t* idx,
+                            const double* w, int64_t nsub, int64_t ncell, int64_t ld, int nz, int nlayers,
+                            const int* levels, int sverdrup, double fill, const int* bounds, int w0, int nwin,
+                            int t_first, int t_end, int continue_first, double* sums, cudaStream_t s) {
+    const double scale = 6371000.0 / 1.e6;
+    const int has_fill = !(fill != fill);
+    const size_t smem = (E3 ? 0 : sizeof(double) * nz) + sizeof(int) * (nlayers + 1);
+    const unsigned gx = (unsigned)((nsub + kSectionBlock - 1) / kSectionBlock);
+    const int64_t ny = (int64_t)nwin * nlayers;
+    for (int64_t y0 = 0; y0 < ny; y0 += 65535) {
+        dim3 grid(gx, (unsigned)std::min<int64_t>(65535, ny - y0));
+        k_flux_section_windows<T, E3><<<grid, kSectionBlock, smem, s>>>(
+            (const T*)u, (const T*)v, (const T*)e3u, (const T*)e3v, e3_tstride, dz, arc1, arc2, idx, w, nsub, ncell,
+            ld, nz, nlayers, levels, scale, sverdrup, (T)fill, has_fill, bounds, w0, t_first, t_end, continue_first,
+            y0, sums);
+        count_launch();
+        NFX_CUDA(cudaGetLastError());
+    }
+}
+
 template <typename T, bool E3>
 void launch_section(const void* u, const void* v, const void* e3u, const void* e3v, int64_t e3_tstride,
                     const double* dz, const double* arc1, const double* arc2, const int32_t* idx, const double* w,
@@ -171,6 +288,37 @@ void flux_section(const void* u, const void* v, int dtype, const double* thickne
             launch_section<float, false>(u, v, e3u, e3v, e3_tstride, thickness, arc1, arc2, idx, w, nsub, ncell, ld, nt,
                                          nz, nlayers, levels, sverdrup, fill, section, s);
     }
+}
+
+void flux_section_windows(const void* u, const void* v, int dtype, const double* thickness, const void* e3u,
+                          const void* e3v, int64_t e3_tstride, const double* arc1, const double* arc2,
+                          const int32_t* idx, const double* w, int64_t nsub, int64_t ncell, int64_t ld, int nz,
+                          int nlayers, const int* levels, int sverdrup, double fill, const int* bounds, int w0, int nwin,
+                          int t_first, int t_end, int continue_first, double* sums, cudaStream_t s) {
+    NFX_REQUIRE(u && v && arc1 && arc2 && idx && w && bounds && sums, "section windows: NULL pointer");
+    NFX_REQUIRE((e3u == nullptr) == (e3v == nullptr) && (thickness != nullptr) != (e3u != nullptr),
+                "section windows: needs exactly one of thickness and (e3u, e3v)");
+    NFX_REQUIRE(nz > 0 && nz <= 3000 && nwin >= 0 && t_first <= t_end && ld >= ncell, "section windows: bad sizes");
+    NFX_REQUIRE(nsub / kSectionBlock < 2147483647ll, "section windows: too many sub-segments");
+    if (nwin == 0 || nsub == 0) return;
+    const bool e3 = e3u != nullptr;
+#define NFX_SECTION_WINDOWS(T, E3)                                                                                    \
+    launch_section_windows<T, E3>(u, v, e3u, e3v, e3_tstride, thickness, arc1, arc2, idx, w, nsub, ncell, ld, nz,     \
+                                  nlayers, levels, sverdrup, fill, bounds, w0, nwin, t_first, t_end, continue_first,  \
+                                  sums, s)
+    if (dtype == NFX_F64) {
+        if (e3)
+            NFX_SECTION_WINDOWS(double, true);
+        else
+            NFX_SECTION_WINDOWS(double, false);
+    } else {
+        NFX_REQUIRE(dtype == NFX_F32, "section windows: dtype must be NFX_F64 or NFX_F32");
+        if (e3)
+            NFX_SECTION_WINDOWS(float, true);
+        else
+            NFX_SECTION_WINDOWS(float, false);
+    }
+#undef NFX_SECTION_WINDOWS
 }
 
 }  // namespace nfx

@@ -309,14 +309,15 @@ class Field(object):
                 return None
             return [nemoflux_gpu.H5DeviceReader(d, self.device) for d in readers]
 
-    def _flux_series_device_decode(self, readers, chunk_steps, prefetch, fn, shape):
+    def _flux_series_device_decode(self, readers, chunk_steps, prefetch, fn, steps):
         """fn over chunked + deflated uo / vo: the COMPRESSED chunks cross PCIe and are inflated, unshuffled and
         placed on the device (csrc/nfx_inflate.cu), then fn (the series' K2 + K3, or the section) runs on the decoded
         slab.  A reader thread copies the compressed chunks of block i + 1 from the memory-mapped files into pinned
         staging while block i is decoded."""
         import threading
         import torch
-        out = numpy.zeros(shape)
+        t_lo, t_hi = steps
+        nt = t_hi - t_lo
         esize = readers[0].ds.dtype.itemsize
         step_bytes = esize * self.nz * self.ny * self.nx
         # The decoder works on one chunk per warp and 20 warps fit an SM: a block of as many chunks as the device holds
@@ -326,12 +327,12 @@ class Field(object):
         chunks_per_step = len(readers[0].dss) * len(readers) * max(1, int(numpy.prod(
             [-(-ext // c) for ext, c in zip(ds.shape[1:], ds.chunk_dims[1:])]))) // max(1, ds.chunk_dims[0])
         wave = 20 * torch.cuda.get_device_properties(self.device).multi_processor_count
-        n = chunk_steps if chunk_steps > 0 else max(1, min(self.nt, wave // max(chunks_per_step, 1),
+        n = chunk_steps if chunk_steps > 0 else max(1, min(nt, wave // max(chunks_per_step, 1),
                                                            (3 << 30) // max(2 * step_bytes, 1)))
         if chunk_steps <= 0:                            # blocks of equal size: a short last block costs a full chunk latency
-            nblk = -(-self.nt // n)
-            n = -(-self.nt // nblk)
-        blocks = [(t0, min(n, self.nt - t0)) for t0 in range(0, self.nt, n)]
+            nblk = -(-nt // n)
+            n = -(-nt // nblk)
+        blocks = [(t0, min(n, t_hi - t0)) for t0 in range(t_lo, t_hi, n)]
         fill = self._fill(self.ncU, 'uo')
         staged = {}
 
@@ -354,14 +355,12 @@ class Field(object):
                 ud, vd = readers[0].decode(st[0]), readers[1].decode(st[1])
             if i + 1 < len(blocks) and not prefetch:
                 stage(i + 1)
-            ser = fn(ud, vd, self._d_thickness, self._d_arc1, self._d_arc2, sverdrup=self.sverdrup, fill=fill,
-                     e3u=self._d_e3u, e3v=self._d_e3v)
-            out[t0:t0 + m] = ser.cpu().numpy()
+            fn(t0, m, ud, vd, self._d_thickness, self._d_arc1, self._d_arc2, sverdrup=self.sverdrup, fill=fill,
+               e3u=self._d_e3u, e3v=self._d_e3v)
             if th is not None:
                 th.join()
         self.last_ingest = dict(path='device decode', bytes_compressed=sum(r.bytes_compressed for r in readers),
                                 bytes_decoded=sum(r.bytes_decoded for r in readers))
-        return out
 
     def _series_shape(self, layers):
         return (self.nt, len(self.plis)) if layers is None else (self.nt, len(layers) - 1, len(self.plis))
@@ -384,49 +383,87 @@ class Field(object):
         (NFX_BIG_ENDIAN), so the host does no conversion pass.
         Chunked + deflated NetCDF-4 variables (device_decode=None: whenever possible, True: required, False: host zlib)
         travel COMPRESSED and are inflated / unshuffled on the device, see _flux_series_device_decode."""
-        def fn(*args, **kw):
-            return self.pli.fluxSeries(*args, layers=layers, **kw)
-        return self._over_chunks(fn, self._series_shape(layers), chunk_steps, prefetch, device_decode)
+        out = numpy.zeros(self._series_shape(layers))
 
-    def fluxSection(self, layers=None, chunk_steps=0, prefetch=True, device_decode=None):
+        def fn(t0, m, *args, **kw):
+            out[t0:t0 + m] = _host(self.pli.fluxSeries(*args, layers=layers, **kw))
+        self._over_chunks(fn, chunk_steps, prefetch, device_decode)
+        return out
+
+    def fluxSection(self, layers=None, chunk_steps=0, prefetch=True, device_decode=None, windows=None):
         """(nt, nlayers, nsub) transport section: the flux across every cell crossing of every transect per layer of
         model levels (layers: level boundaries, see levelsForDepths; None = one layer per level), see
-        PolylineIntegral.fluxSection and getSectionGeometry.  Reads the files as fluxSeries does."""
+        PolylineIntegral.fluxSection and getSectionGeometry.  Reads the files as fluxSeries does.
+
+        windows: step boundaries [b0 < ... < bK] (see timeobj.timeWindows) -> (K, nlayers, nsub), the time mean of
+        every window, PolylineIntegral.fluxSection(windows=) of the whole record bit for bit.  Only the steps
+        [b0, bK) are read; one (K, nlayers, nsub) array of sums is kept, each block of steps read from the files
+        continues the windows it shares with the block before, and the sums are divided at the end."""
         lev = list(range(self.nz + 1)) if layers is None else layers
+        nsub = self.pli.getNumberOfSubsegments()
+        if windows is None:
+            out = numpy.zeros((self.nt, len(lev) - 1, nsub))
 
-        def fn(*args, **kw):
-            return self.pli.fluxSection(*args, layers=lev, **kw)
-        return self._over_chunks(fn, (self.nt, len(lev) - 1, self.pli.getNumberOfSubsegments()), chunk_steps, prefetch,
-                                 device_decode)
+            def fn(t0, m, *args, **kw):
+                out[t0:t0 + m] = _host(self.pli.fluxSection(*args, layers=lev, **kw))
+            self._over_chunks(fn, chunk_steps, prefetch, device_decode)
+            return out
+        b = numpy.asarray(windows).reshape(-1)
+        if b.size < 2 or b.dtype.kind not in 'iu' or b[0] < 0 or b[-1] > self.nt or numpy.any(numpy.diff(b) <= 0):
+            raise ValueError(f'windows must be strictly ascending step indices in [0, nt = {self.nt}], got {windows!r}')
+        b = b.astype(numpy.int64)
+        sums = numpy.zeros((b.size - 1, len(lev) - 1, nsub))
 
-    def _over_chunks(self, fn, shape, chunk_steps, prefetch, device_decode):
-        """out (shape, time first) = fn(u, v, thickness, arc1, arc2, sverdrup=, fill=, e3u=, e3v=) over chunks of time
-        steps read from the files: the pipeline of fluxSeries"""
+        def fn(t0, m, u, v, *args, **kw):
+            # the windows [wa, wb) this block touches, their bounds inside the block; window wa continues its sums when
+            # it began in an earlier block
+            wa = max(int(numpy.searchsorted(b, t0, 'right')) - 1, 0)
+            wb = min(int(numpy.searchsorted(b, t0 + m, 'left')), b.size - 1)
+            if wa >= wb:
+                return
+            local = numpy.clip(b[wa:wb + 1] - t0, 0, m)
+            if isinstance(u, numpy.ndarray):
+                self.pli.sectionWindowSums(u, v, *args, windows=local, layers=lev, sums=sums[wa:wb],
+                                           continue_first=b[wa] < t0, **kw)
+            else:
+                import torch
+                part = torch.from_numpy(sums[wa:wb]).to(u.device)
+                self.pli.sectionWindowSums(u, v, *args, windows=local, layers=lev, sums=part,
+                                           continue_first=b[wa] < t0, **kw)
+                sums[wa:wb] = part.cpu().numpy()
+        self._over_chunks(fn, chunk_steps, prefetch, device_decode, steps=(int(b[0]), int(b[-1])))
+        sums /= numpy.diff(b).astype(numpy.float64)[:, None, None]
+        return sums
+
+    def _over_chunks(self, fn, chunk_steps, prefetch, device_decode, steps=None):
+        """fn(t0, m, u, v, thickness, arc1, arc2, sverdrup=, fill=, e3u=, e3v=) over blocks [t0, t0 + m) of the time
+        steps [steps[0], steps[1]) (default: all) read from the files: the pipeline of fluxSeries"""
         import threading
         import torch
+        steps = (0, self.nt) if steps is None else steps
         if device_decode is not False:
             readers = self._device_readers()
             if readers is not None:
-                return self._flux_series_device_decode(readers, chunk_steps, prefetch, fn, shape)
+                return self._flux_series_device_decode(readers, chunk_steps, prefetch, fn, steps)
             if device_decode is True:
                 raise RuntimeError('ERROR: uo / vo are not chunked HDF5 variables with a [shuffle,] [deflate] pipeline')
-        out = numpy.zeros(shape)
+        t_lo, t_hi = steps
         dtype = numpy.dtype(self.ncU['uo'].dtype).newbyteorder('=')
         step_bytes = dtype.itemsize * self.nz * self.ny * self.nx
         # ~300 MB per variable and chunk (sweep in profiles/r1_file_e2e_C3.json: 4 f64 / 8 f32 ORCA1 steps): small enough that reading chunk i+1 overlaps the upload of chunk i even
         # for a short series, large enough for full-rate PCIe copies
-        n = chunk_steps if chunk_steps > 0 else max(1, min(self.nt, (300 << 20) // max(step_bytes, 1)))
+        n = chunk_steps if chunk_steps > 0 else max(1, min(t_hi - t_lo, (300 << 20) // max(step_bytes, 1)))
         arc1, arc2 = self.arcLengths[:, 1].copy(), self.arcLengths[:, 2].copy()
         tdtype = {4: torch.float32, 8: torch.float64}[dtype.itemsize]
         shape = (n, self.nz, self.ny, self.nx)
-        nbuf = 2 if prefetch and self.nt > n else 1
+        nbuf = 2 if prefetch and t_hi - t_lo > n else 1
         cache = getattr(self, '_pinned', None)      # page-locked allocations are slow (~0.1 s/GB): keep them
         if cache is None or cache[0] != (shape, tdtype) or len(cache[1]) < nbuf:
             cache = ((shape, tdtype), [(torch.empty(shape, dtype=tdtype, pin_memory=True),
                                         torch.empty(shape, dtype=tdtype, pin_memory=True)) for _ in range(nbuf)])
             self._pinned = cache
         bufs = cache[1][:nbuf]
-        chunks = [(t0, min(n, self.nt - t0)) for t0 in range(0, self.nt, n)]
+        chunks = [(t0, min(n, t_hi - t0)) for t0 in range(t_lo, t_hi, n)]
         state = {}
         raw_u, raw_v = numpy.dtype(self.ncU['uo'].dtype), numpy.dtype(self.ncV['vo'].dtype)
         as_stored = raw_u == raw_v and not raw_u.isnative       # both files big-endian: no conversion on the host
@@ -469,18 +506,22 @@ class Field(object):
                 th = threading.Thread(target=read, args=(i + 1, 1 - slot))
                 th.start()
             nu, nv = views[slot]                    # numpy views of the pinned buffers (kept alive by `bufs`)
-            out[t0:t0 + m] = fn(nu[:m], nv[:m], self.thickness, arc1, arc2, sverdrup=self.sverdrup, fill=state.pop(i),
-                                e3u=self._d_e3u, e3v=self._d_e3v)
+            fn(t0, m, nu[:m], nv[:m], self.thickness, arc1, arc2, sverdrup=self.sverdrup, fill=state.pop(i),
+               e3u=self._d_e3u, e3v=self._d_e3v)
             if th is not None:
                 th.join()
             elif i + 1 < len(chunks):
                 read(i + 1, slot)
         pool.shutdown()
-        return out
 
     def close(self):
         self.ncU.close()
         self.ncV.close()
+
+
+def _host(x):
+    """a result of PolylineIntegral as numpy (CUDA tensors of the device-decode path are copied back)"""
+    return x if isinstance(x, numpy.ndarray) else x.cpu().numpy()
 
 
 def layerInterfaces(bounds_depth):

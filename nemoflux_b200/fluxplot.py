@@ -1,7 +1,7 @@
 """fluxplot -- drop-in for nemoflux/fluxplot.py: flux time series of every transect (same flags).
 
     python -m nemoflux_b200.fluxplot -t T.nc -u U.nc -v V.nc -i "../data/nz/S*.txt" [-s] [--output series.csv]
-        [--layers "0,10,35,75" | --depthLayers "0,200,1000,6000"] [--section section.nc]
+        [--layers "0,10,35,75" | --depthLayers "0,200,1000,6000"] [--section section.nc] [--timeMean N|month|year]
 
 The reference loops ``for itime: fld.update(); for pli: pli.getIntegral(...)`` (fluxplot.py:51-59); here the
 whole (nt, M) series comes from Field.fluxSeries() (K2+K3 over chunks of time steps).  The series is printed
@@ -12,6 +12,10 @@ interfaces that were integrated.
 --section FILE.nc also writes the transport section (Field.fluxSection): the flux across every cell crossing of every
 transect per layer (the layers of --layers / --depthLayers, else one per level) as a NetCDF classic (64-bit offset)
 file, see writeSection.
+--timeMean N|month|year averages over windows of N steps, or of the steps of each calendar month / year
+(timeobj.timeWindows): the printed and CSV series become window means (windowMeans), one row per window labelled
+first/last (the dates of its first and last step), and the --section file holds window means computed on the device
+(Field.fluxSection(windows=)) with time_bnds and cell_methods = "time: mean".
 """
 import argparse
 import os
@@ -21,6 +25,7 @@ import numpy
 from . import ncio
 from .field import Field
 from .fluxviz import parseTransects
+from .timeobj import timeWindows
 
 
 def parseList(text, kind=float):
@@ -34,13 +39,39 @@ def parseList(text, kind=float):
     return vals
 
 
-def writeSection(path, fld, layers, units):
+def parseTimeMean(text):
+    """'--timeMean' value: a number of steps >= 1, 'month' or 'year'"""
+    t = text.strip().lower()
+    if t in ('month', 'year'):
+        return t
+    if t.isdigit() and int(t) >= 1:
+        return int(t)
+    raise argparse.ArgumentTypeError(f"expected a number of steps >= 1, 'month' or 'year', got {text!r}")
+
+
+def windowMeans(x, bounds):
+    """(K, ...) means over the windows [b_w, b_{w+1}) of the first axis of x: the sum in ascending step order from
+    +0, divided by the window's length (the definition of fluxSection(windows=))"""
+    x = numpy.asarray(x, numpy.float64)
+    out = numpy.empty((len(bounds) - 1,) + x.shape[1:])
+    for w in range(len(bounds) - 1):
+        acc = numpy.zeros(x.shape[1:])
+        for t in range(bounds[w], bounds[w + 1]):
+            acc = acc + x[t]
+        out[w] = acc / (bounds[w + 1] - bounds[w])
+    return out
+
+
+def writeSection(path, fld, layers, units, windows=None):
     """transport(time, layer, crossing) of fld.fluxSection(layers) with the crossings' geometry
     (PolylineIntegral.getSectionGeometry), layer_top / layer_bottom in metres, transect_offsets and time (the record
     dimension: only one record has to fit the 4 GB of the classic 64-bit-offset format).  Returns the number of
-    crossings."""
+    crossings.
+    windows (step bounds, see timeobj.timeWindows): window means instead, cell_methods = "time: mean"; time is the mean
+    of the window's time values and time_bnds (time, 2) its extent: from the time variable's bounds variable (NEMO's
+    time_centered_bounds) when the file has one, else the first and last time stamps."""
     lev = list(range(fld.nz + 1)) if layers is None else list(layers)
-    sec = fld.fluxSection(layers=lev)
+    sec = fld.fluxSection(layers=lev) if windows is None else fld.fluxSection(layers=lev, windows=windows)
     geo = fld.pli.getSectionGeometry()
     iface = fld.layerInterfaces()
     nsub = sec.shape[2]
@@ -52,9 +83,21 @@ def writeSection(path, fld, layers, units):
     tv = fld.timeObj.getValues() if fld.timeObj.getSize() == fld.nt else numpy.arange(fld.nt)
     tattrs = {k: v for k, v in (('units', fld.timeObj.units), ('calendar', fld.timeObj.calendar)) if v} \
         if fld.timeObj.getSize() == fld.nt else {'long_name': 'time index'}
-    w.createVariable('time', 'f8', ('time',), attrs=tattrs, data=numpy.asarray(tv, numpy.float64))
-    w.createVariable('transport', 'f8', ('time', 'layer', 'crossing'), data=sec,
-                     attrs={'units': units, 'long_name': 'flux across the cell crossing, per layer of model levels'})
+    tv = numpy.asarray(tv, numpy.float64)
+    tattrs_sec = {'units': units, 'long_name': 'flux across the cell crossing, per layer of model levels'}
+    if windows is not None:
+        b = list(windows)
+        bnds = fld.timeObj.getBounds() if fld.timeObj.getSize() == fld.nt else None
+        lo = numpy.array([bnds[b0, 0] if bnds is not None else tv[b0] for b0 in b[:-1]], numpy.float64)
+        hi = numpy.array([bnds[b1 - 1, 1] if bnds is not None else tv[b1 - 1] for b1 in b[1:]], numpy.float64)
+        tv = numpy.array([tv[b0:b1].mean() for b0, b1 in zip(b[:-1], b[1:])], numpy.float64)
+        tattrs = dict(tattrs, bounds='time_bnds')
+        tattrs_sec['cell_methods'] = 'time: mean'
+        w.createDimension('nv', 2)
+    w.createVariable('time', 'f8', ('time',), attrs=tattrs, data=tv)
+    if windows is not None:
+        w.createVariable('time_bnds', 'f8', ('time', 'nv'), data=numpy.stack([lo, hi], 1))
+    w.createVariable('transport', 'f8', ('time', 'layer', 'crossing'), data=sec, attrs=tattrs_sec)
     w.createVariable('layer_top', 'f8', ('layer',), attrs={'units': 'm'}, data=iface[lev[:-1]])
     w.createVariable('layer_bottom', 'f8', ('layer',), attrs={'units': 'm'}, data=iface[lev[1:]])
     w.createVariable('transect_offsets', 'i4', ('transect_edge',), data=geo['offsets'].astype(numpy.int32))
@@ -86,6 +129,8 @@ def main(argv=None):
                      help='flux per depth range: depths in metres "0,200,1000,6000", snapped to level interfaces')
     ap.add_argument('--section', default='',
                     help='write the transport section (flux per cell crossing and layer) to this NetCDF file')
+    ap.add_argument('--timeMean', type=parseTimeMean, default=None,
+                    help='average over windows of N steps, or per calendar month / year: N|month|year')
     a = ap.parse_args(argv)
     pts, names = parseTransects(a.lonLatPoints, a.iFiles)
     print(f'target points:\n {pts}')
@@ -93,18 +138,23 @@ def main(argv=None):
     layers = fld.levelsForDepths(a.depthLayers) if a.depthLayers is not None else a.layers
     series = fld.fluxSeries(layers=layers)
     timeVals = [fld.timeObj.getTimeAsDate(i) for i in range(fld.nt)]
+    windows = None
+    if a.timeMean is not None:
+        windows = timeWindows(fld.timeObj, fld.nt, a.timeMean)
+        series = windowMeans(series, windows)
+        timeVals = [f'{timeVals[b0]}/{timeVals[b1 - 1]}' for b0, b1 in zip(windows[:-1], windows[1:])]
     units = 'Sv' if a.sverdrup else 'A m^2/s'
     labels = [os.path.basename(n) for n in names]
     rows = series
     if layers is not None:
         iface = fld.layerInterfaces()
         labels = [f'{lab}[{iface[k0]:g}-{iface[k1]:g} m]' for lab in labels for k0, k1 in zip(layers[:-1], layers[1:])]
-        rows = numpy.asarray(series).transpose(0, 2, 1).reshape(fld.nt, -1)      # (time, transect-major layers)
+        rows = numpy.asarray(series).transpose(0, 2, 1).reshape(len(series), -1)   # (time, transect-major layers)
     print('time,' + ','.join(labels) + f'   [{units}]')
     for t, row in zip(timeVals, rows):
         print(f'{t},' + ','.join(f'{x:.15g}' for x in row))
     if a.section:
-        nsub = writeSection(a.section, fld, layers, units)
+        nsub = writeSection(a.section, fld, layers, units, windows)
         print(f'section: {nsub} crossings written to {a.section}')
     if a.output:
         with open(a.output, 'w') as f:

@@ -312,7 +312,7 @@ class PolylineIntegral(object):
         return self._flux_series_host(u, v, thickness, arc1, arc2, sverdrup, fill, order, chunk_steps, e3u, e3v, lev)
 
     def fluxSection(self, u, v, thickness, arc1, arc2, sverdrup=False, fill=float('nan'), layers=None, out=None,
-                    chunk_steps=0, e3u=None, e3v=None):
+                    chunk_steps=0, e3u=None, e3v=None, windows=None):
         """transport section: the flux across every sub-segment (cell crossing) of every transect, per layer of model
         levels and time step -> (nt, N, nsub), float64.  getSubsegments()['offsets'] splits the last axis by transect
         (emission order), getSectionGeometry() places every crossing along its transect.
@@ -323,14 +323,86 @@ class PolylineIntegral(object):
 
         [t, i, s] = ((w0*E[idx0] + w1*E[idx1]) + w2*E[idx2]) + w3*E[idx3] over the 4 edge entries of sub-segment s, with
         E the layer-i edge flux fluxSeries(layers=, eflux=) writes, bit for bit; a transect's crossings add up to its
-        layered series to rounding."""
+        layered series to rounding.
+
+        windows: step boundaries [b0 < b1 < ... < bK] (0 <= b0, bK <= nt) -> the time mean over every window of steps
+        [b_w, b_{w+1}), (K, N, nsub) (out: CUDA float64 of that shape).  The sum of the window is taken in ascending
+        step order from +0 (a one-step window of -0 gives +0), every add rounded on its own, then divided by the
+        window's length: numpy reproduces it bit for bit from the per-step section with a sequential loop over t.  Steps
+        outside [b0, bK) are not read.  The memory is that of the K windows, whatever nt; see sectionWindowSums."""
+        wins = _window_bounds(windows)
+        if wins is None:
+            return self._section(u, v, thickness, arc1, arc2, sverdrup, fill, layers, out, chunk_steps, e3u, e3v)
+        sums = self.sectionWindowSums(u, v, thickness, arc1, arc2, wins, sverdrup=sverdrup, fill=fill, layers=layers,
+                                      sums=out, chunk_steps=chunk_steps, e3u=e3u, e3v=e3v)
+        lengths = numpy.diff(wins).astype(numpy.float64)
+        if isinstance(sums, numpy.ndarray):
+            sums /= lengths[:, None, None]
+            return sums
+        # a CUDA tensor of lengths, not a Python scalar: torch divides by a host scalar through its reciprocal
+        return sums.div_(_torch().from_numpy(lengths).to(sums.device).view(-1, 1, 1))
+
+    def sectionWindowSums(self, u, v, thickness, arc1, arc2, windows, sverdrup=False, fill=float('nan'), layers=None,
+                          sums=None, continue_first=False, chunk_steps=0, e3u=None, e3v=None):
+        """sums over windows of time steps of fluxSection(layers=): (K, N, nsub) float64, window w the steps
+        [b_w, b_{w+1}) of the steps passed, added in ascending step order from +0.  fluxSection(windows=) divides these
+        by the window lengths.  sums: the output (CUDA tensor for CUDA inputs, C-contiguous float64 numpy array for
+        host inputs; None = a new one).  continue_first: window 0 continues the partial sums already in sums[0], so a
+        record read in blocks of steps (a window split over several calls, in step order) gives the bits of one call."""
+        torch = _torch()
+        wins = _window_bounds(windows)
+        if wins is None:
+            raise ValueError('windows is required')
+        lev = _layer_levels(layers)
+        nsub = self.getNumberOfSubsegments()
+        if isinstance(u, torch.Tensor) and u.is_cuda:
+            u, v, nt, nz, ncell, ld, lev = self._section_device_inputs(u, v, thickness, arc1, arc2, e3u, e3v, lev)
+            use_e3 = e3u is not None or e3v is not None
+            e3_nt = _check_e3(e3u, e3v, u, nt, nz, ncell, ld) if use_e3 and nt else 0
+            shape = (wins.size - 1, lev.size - 1, nsub)
+            if sums is None:
+                sums = (torch.zeros if continue_first else torch.empty)(shape, dtype=torch.float64, device=u.device)
+            _require_cuda(sums, torch.float64, 'out')
+            if tuple(sums.shape) != shape or not sums.is_contiguous():
+                raise ValueError(f'out must be a contiguous CUDA tensor of shape (K, nlayers, nsub) = {shape}')
+            ptr = lambda t: _t_ptr(t) if t is not None and t.numel() else None   # noqa: E731
+            with torch.cuda.device(u.device):
+                _lib.call('nfx_flux_section_window_sums', ctypes.byref(self._h), ptr(u), ptr(v), ptr(e3u), ptr(e3v),
+                          _dtype_code(str(u.dtype)), e3_nt, None if use_e3 else _t_ptr(thickness), _t_ptr(arc1),
+                          _t_ptr(arc2), nt, nz, ld, lev.size - 1, _np_ptr(lev), int(bool(sverdrup)), float(fill),
+                          wins.size - 1, _np_ptr(wins), int(bool(continue_first)), ptr(sums), _stream_ptr())
+            return sums
+        keep = (u, v, e3u, e3v)  # keep pinned tensors alive while numpy views are in use
+        h = _host_inputs(u, v, thickness, arc1, arc2, e3u, e3v)
+        lev = numpy.arange(h.nz + 1, dtype=numpy.int32) if lev is None else lev
+        shape = (wins.size - 1, lev.size - 1, nsub)
+        if sums is None:
+            sums = numpy.zeros(shape, numpy.float64)
+        if not isinstance(sums, numpy.ndarray) or sums.dtype != numpy.float64 or sums.shape != shape or \
+                not sums.flags.c_contiguous or not sums.flags.writeable:
+            raise ValueError(f'out must be a C-contiguous float64 numpy array of shape (K, nlayers, nsub) = {shape}')
+        pu, pv, e3_nt, on_device = h.e3 if h.e3 is not None else (None, None, 0, False)
+        _lib.call('nfx_flux_section_window_sums_host', ctypes.byref(self._h), _np_ptr(h.u), _np_ptr(h.v), pu, pv,
+                  h.code, e3_nt, int(on_device), None if h.th is None else _np_ptr(h.th), _np_ptr(h.a1), _np_ptr(h.a2),
+                  h.nt, h.nz, lev.size - 1, _np_ptr(lev), int(bool(sverdrup)), float(fill), wins.size - 1,
+                  _np_ptr(wins), int(bool(continue_first)), int(chunk_steps), _np_ptr(sums))
+        del keep
+        return sums
+
+    def _section_device_inputs(self, u, v, thickness, arc1, arc2, e3u, e3v, lev):
+        """checks of the CUDA inputs of fluxSection / sectionWindowSums -> (u, v, nt, nz, ncell, ld, levels), the
+        levels of one layer per level when lev is None"""
+        u, v, nt, nz, ncell, ld = self._device_inputs(u, v, thickness, arc1, arc2, e3u, e3v)
+        lev = numpy.arange(nz + 1, dtype=numpy.int32) if lev is None else lev
+        return u, v, nt, nz, ncell, ld, lev
+
+    def _section(self, u, v, thickness, arc1, arc2, sverdrup, fill, layers, out, chunk_steps, e3u, e3v):
         torch = _torch()
         lev = _layer_levels(layers)
         nsub = self.getNumberOfSubsegments()
         if isinstance(u, torch.Tensor) and u.is_cuda:
-            u, v, nt, nz, ncell, ld = self._device_inputs(u, v, thickness, arc1, arc2, e3u, e3v)
+            u, v, nt, nz, ncell, ld, lev = self._section_device_inputs(u, v, thickness, arc1, arc2, e3u, e3v, lev)
             use_e3 = e3u is not None or e3v is not None
-            lev = numpy.arange(nz + 1, dtype=numpy.int32) if lev is None else lev
             shape = (nt, lev.size - 1, nsub)
             if out is None:
                 out = torch.empty(shape, dtype=torch.float64, device=u.device)
@@ -682,6 +754,21 @@ def _layer_levels(layers):
         raise ValueError('layers must hold integer level indices')
     if numpy.any(numpy.abs(a) > 2 ** 31 - 1):
         raise ValueError('layers: level index out of range')
+    return numpy.ascontiguousarray(a, numpy.int32)
+
+
+def _window_bounds(windows):
+    """windows -> contiguous int32 array of step boundaries (None stays None).  Only the form is checked here; the
+    library rejects boundaries that are not strictly ascending inside [0, nt]."""
+    if windows is None:
+        return None
+    a = numpy.asarray(_to_numpy(windows))
+    if a.ndim != 1 or a.size < 2:
+        raise ValueError(f'windows must be a 1-D sequence of at least 2 step boundaries, got shape {a.shape}')
+    if a.dtype.kind not in 'iu' and not (a.dtype.kind == 'f' and numpy.all(a == numpy.round(a))):
+        raise ValueError('windows must hold integer step indices')
+    if numpy.any(numpy.abs(a) > 2 ** 31 - 1):
+        raise ValueError('windows: step index out of range')
     return numpy.ascontiguousarray(a, numpy.int32)
 
 

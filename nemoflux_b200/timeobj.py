@@ -53,10 +53,13 @@ class TimeObj(object):
 
     def __init__(self, nc):
         self.timeVarName, self.timeVar, self.units, self.calendar = '', [], '', 'standard'
+        self.boundsVar = None
         for name, var in nc.items():
             if _is_time_axis(var):          # the last match wins, as in the reference
                 self.timeVarName, self.timeVar, self.units = name, var[:], str(getattr(var, 'units', ''))
                 self.calendar = str(getattr(var, 'calendar', 'standard')).lower()
+                bnds = str(getattr(var, 'bounds', ''))
+                self.boundsVar = nc[bnds][:] if bnds and bnds in nc else None
         since = _SINCE.match(self.units)
         self._origin = datetime.datetime(*(int(since.group(k)) for k in (2, 3, 4))) if since else None
         self._unit_s = _SECONDS[since.group(1)] if since else None
@@ -76,8 +79,35 @@ class TimeObj(object):
             return _fixed_calendar_date(self._origin, seconds, self.calendar)
         return (self._origin + datetime.timedelta(seconds=seconds)).date()
 
+    def getBounds(self):
+        """(n, 2) values of the time variable's CF `bounds` variable (NEMO: time_centered_bounds), or None"""
+        if self.boundsVar is None or len(self.boundsVar) != len(self.timeVar):
+            return None
+        return self.boundsVar[:]
+
     def getTimeAsString(self, timeIndex):
         when = self.getTimeAsDate(timeIndex)
         if isinstance(when, (datetime.date, CalendarDate)):
             return f'{when.year}-{when.month}-{when.day}'
         return f'time index {when}'
+
+
+def timeWindows(timeObj, nt, spec):
+    """window bounds [b0 = 0 < b1 < ... < bK = nt] of the nt steps for time means (fluxSection(windows=)):
+    spec an int N -> windows of N steps (the last one holds what is left); 'month' / 'year' -> runs of consecutive
+    steps with the same (year, month) / year of getTimeAsDate, in every calendar it decodes (standard, noleap /
+    365_day, 360_day).  Calendar windows need a time axis of nt values with CF units '<unit> since Y-M-D'."""
+    if isinstance(spec, str) and spec.strip().isdigit():
+        spec = int(spec)
+    if isinstance(spec, int) and not isinstance(spec, bool):
+        if spec < 1:
+            raise ValueError(f'a time window holds at least 1 step, got {spec}')
+        return list(range(0, nt, spec)) + [nt] if nt > 0 else [0]
+    if spec not in ('month', 'year'):
+        raise ValueError(f"time windows: expected a number of steps, 'month' or 'year', got {spec!r}")
+    if timeObj is None or timeObj._origin is None or timeObj.getSize() != nt or nt == 0:
+        raise ValueError(f"time windows by {spec} need a time axis of {nt} steps with CF units '<unit> since Y-M-D' "
+                         "(this file has none): give a number of steps instead")
+    dates = [timeObj.getTimeAsDate(i) for i in range(nt)]
+    keys = [(d.year, d.month) if spec == 'month' else d.year for d in dates]
+    return [0] + [i for i in range(1, nt) if keys[i] != keys[i - 1]] + [nt]
