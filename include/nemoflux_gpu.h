@@ -245,6 +245,26 @@ int nfx_flux_section_window_sums(nfx_pli** self, const void* u, const void* v, c
                                  int nt, int nz, int64_t ld, int nlayers, const int* layer_levels, int sverdrup,
                                  double fill, int nwindows, const int* window_bounds, int continue_first, double* sums,
                                  void* stream);
+/* Class transport (extension): the flux across every transect binned by a T-grid field c (temperature, salinity,
+ * density...).  Arguments as nfx_flux_section with one layer per level, plus the class field cfield (device, c_nt x nz
+ * planes of ld values, the dtype of u, v; c_nt = 1: time-invariant, or nt), its missing-value marker cfill (NaN = none;
+ * compared in the storage type, as fill) and class_bounds (host, nclasses + 1 strictly ascending doubles, +-inf
+ * allowed, no NaN; 1 <= nclasses <= 96).  classes device (nt, nclasses, M):
+ *   classes[t, j, m] = sum over the crossings s of transect m and the levels k with b_j <= c[t|0, k, cell(s)] < b_{j+1}
+ *                      of f[t, k, s], the value nfx_flux_section computes for the one-level layer k
+ * A level whose class value is NaN, the marker, below b0 or at or above bK counts nowhere.  Sum order: per crossing
+ * and class the levels in ascending order from +0; the crossings of a transect in tiles of 32 in emission order, each
+ * folded by a fixed shuffle tree (lane l + lane l + o, o = 16, 8, 4, 2, 1); the tiles in ascending order from +0.  The
+ * bits depend only on the inputs.  Asynchronous on `stream`, except that the bounds (and, on the first call after
+ * computeWeights, the crossing tiles) are copied from pageable host memory, which waits for the work already queued on
+ * `stream`.  The bounds, tiles and partial sums are scratch of the handle: calls on one handle must not run
+ * concurrently on different streams.  Invalid bounds, too many classes, a NULL pointer, or
+ * transects computed without nfx_grid_set_cgrid_shape return NFX_E_INVALID before anything is launched; nt == 0 or no
+ * crossing launches nothing and leaves `classes` as it is. */
+int nfx_flux_classes(nfx_pli** self, const void* u, const void* v, const void* e3u, const void* e3v, int dtype,
+                     int e3_nt, const double* thickness, const double* arc1, const double* arc2, int nt, int nz,
+                     int64_t ld, const void* cfield, int c_nt, double cfill, int nclasses, const double* class_bounds,
+                     int sverdrup, double fill, double* classes, void* stream);
 /* The device-path series calls (nfx_flux_series*, nfx_flux_series_range*) are asynchronous on `stream`.  Their fused
  * pass spins on per-batch counters with a bound; a pass that ever overflowed it aborts and leaves NaN in `series`.
  * nfx_pli_series_status synchronises `stream` and reports that: returns 0 with *status = 0 when every pass launched
@@ -343,6 +363,14 @@ int nfx_flux_section_window_sums_host(nfx_pli** self, const void* u, const void*
                                       const double* arc1, const double* arc2, int nt, int nz, int nlayers,
                                       const int* layer_levels, int sverdrup, double fill, int nwindows,
                                       const int* window_bounds, int continue_first, int chunk_steps, double* sums);
+/* nfx_flux_classes from HOST buffers: arguments as nfx_flux_section_host plus cfield (host, c_nt x nz x ncell in the
+ * dtype and byte order of u, v: streamed with them when c_nt == nt, uploaded once when c_nt == 1), cfill, nclasses,
+ * class_bounds; classes host (nt, nclasses, M).  The bits do not depend on chunk_steps or the byte order and are
+ * those of nfx_flux_classes. */
+int nfx_flux_classes_host(nfx_pli** self, const void* u, const void* v, const void* e3u, const void* e3v,
+                          int dtype_flags, int e3_nt, int e3_on_device, const double* thickness, const double* arc1,
+                          const double* arc2, int nt, int nz, const void* cfield, int c_nt, double cfill, int nclasses,
+                          const double* class_bounds, int sverdrup, double fill, int chunk_steps, double* classes);
 
 #ifdef __cplusplus
 }

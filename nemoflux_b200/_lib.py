@@ -110,6 +110,10 @@ SIGNATURES = {
                                      c_i64, c_int, c_vp, c_int, c_dbl, c_int, c_vp, c_int, c_vp, c_vp],
     'nfx_flux_section_window_sums_host': [P(c_vp), c_vp, c_vp, c_vp, c_vp, c_int, c_int, c_int, c_vp, c_vp, c_vp,
                                           c_int, c_int, c_int, c_vp, c_int, c_dbl, c_int, c_vp, c_int, c_int, c_vp],
+    'nfx_flux_classes': [P(c_vp), c_vp, c_vp, c_vp, c_vp, c_int, c_int, c_vp, c_vp, c_vp, c_int, c_int, c_i64, c_vp,
+                         c_int, c_dbl, c_int, c_vp, c_int, c_dbl, c_vp, c_vp],
+    'nfx_flux_classes_host': [P(c_vp), c_vp, c_vp, c_vp, c_vp, c_int, c_int, c_int, c_vp, c_vp, c_vp, c_int, c_int,
+                              c_vp, c_int, c_dbl, c_int, c_vp, c_int, c_dbl, c_int, c_vp],
 }
 
 _LIB = None

@@ -906,6 +906,88 @@ int nfx_flux_section_window_sums(nfx_pli** self, const void* u, const void* v, c
     });
 }
 
+// Class bounds handed in by the caller (host array): K + 1 strictly ascending doubles, +-inf allowed, no NaN.  Checked
+// before anything is launched.
+static void check_class_bounds(int nclasses, const double* bounds) {
+    NFX_REQUIRE(nclasses >= 1 && nclasses <= kClassMax,
+                "classes: the number of classes must be in [1, " + std::to_string(kClassMax) + "]");
+    NFX_REQUIRE(bounds, "classes: class_bounds is NULL");
+    for (int j = 0; j <= nclasses; ++j) NFX_REQUIRE(bounds[j] == bounds[j], "classes: a class bound is NaN");
+    for (int j = 0; j < nclasses; ++j)
+        NFX_REQUIRE(bounds[j] < bounds[j + 1], "classes: the class bounds must be strictly ascending (class " +
+                                                   std::to_string(j) + " is empty)");
+}
+
+// the warp tiles of k_flux_classes: at most 32 consecutive crossings of one transect each, in emission order
+static void class_tiles(PliDev& p, cudaStream_t s) {
+    if (p.class_ntiles >= 0) return;
+    p.h_class_tiles.clear();
+    p.h_class_tr_tiles.assign((size_t)p.ntransects + 1, 0);
+    for (int m = 0; m < p.ntransects; ++m) {
+        for (int64_t a = p.h_sub_offsets[m]; a < p.h_sub_offsets[m + 1]; a += 32) p.h_class_tiles.push_back(a);
+        p.h_class_tr_tiles[m + 1] = (int64_t)p.h_class_tiles.size();
+    }
+    p.h_class_tiles.push_back(p.nsub);
+    const int64_t ntiles = (int64_t)p.h_class_tiles.size() - 1;
+    p.class_tiles.ensure(p.h_class_tiles.size());
+    p.class_tr_tiles.ensure(p.h_class_tr_tiles.size());
+    NFX_CUDA(cudaMemcpyAsync(p.class_tiles.p, p.h_class_tiles.data(), sizeof(int64_t) * p.h_class_tiles.size(),
+                             cudaMemcpyHostToDevice, s));
+    // copies from pageable memory: the source is read before they return, so the vectors may change afterwards
+    NFX_CUDA(cudaMemcpyAsync(p.class_tr_tiles.p, p.h_class_tr_tiles.data(),
+                             sizeof(int64_t) * p.h_class_tr_tiles.size(), cudaMemcpyHostToDevice, s));
+    p.class_ntiles = ntiles;
+}
+
+// tiles, bounds and the partial sums of a class call of up to nt steps (the partial sums: at most 64 MB, or one step)
+static int prepare_classes(PliDev& p, int nclasses, const double* bounds, int nt, cudaStream_t s) {
+    class_tiles(p, s);
+    p.class_bounds.ensure((size_t)nclasses + 1);
+    NFX_CUDA(cudaMemcpyAsync(p.class_bounds.p, bounds, sizeof(double) * ((size_t)nclasses + 1), cudaMemcpyHostToDevice,
+                             s));
+    const int64_t per_step = std::max<int64_t>(1, p.class_ntiles * nclasses);
+    const int steps = (int)std::max<int64_t>(1, std::min<int64_t>(nt, ((int64_t)64 << 20) / 8 / per_step));
+    p.class_partial.ensure((size_t)steps * per_step);
+    return steps;
+}
+
+static void run_classes(PliDev& p, const void* u, const void* v, int dtype, const double* thickness, const void* e3u,
+                        const void* e3v, int64_t e3_tstride, const double* arc1, const double* arc2, const void* cfield,
+                        int64_t c_tstride, double cfill, int nclasses, int64_t ld, int nt, int nz, int sverdrup,
+                        double fill, int partial_steps, double* classes, cudaStream_t s) {
+    const Csr& c = section_csr(p);
+    flux_classes(u, v, dtype, thickness, e3u, e3v, e3_tstride, arc1, arc2, c.idx.p, c.w, p.cell.p, cfield, c_tstride,
+                 cfill, p.class_bounds.p, nclasses, p.class_tiles.p, p.class_ntiles, p.class_tr_tiles.p, p.ntransects,
+                 p.grid->ncell, ld, nt, nz, sverdrup, fill, p.class_partial.p, partial_steps, classes, s);
+}
+
+int nfx_flux_classes(nfx_pli** self, const void* u, const void* v, const void* e3u, const void* e3v, int dtype,
+                     int e3_nt, const double* thickness, const double* arc1, const double* arc2, int nt, int nz,
+                     int64_t ld, const void* cfield, int c_nt, double cfill, int nclasses, const double* class_bounds,
+                     int sverdrup, double fill, double* classes, void* stream) {
+    return guarded([&] {
+        NFX_REQUIRE(self && *self, "NULL handle");
+        PliDev& p = (*self)->d;
+        NFX_REQUIRE(p.grid, "setGrid was not called");
+        DeviceGuard g(p.grid->device);
+        NFX_REQUIRE(u && v && arc1 && arc2 && cfield && classes, "NULL pointer");
+        NFX_REQUIRE((e3u == nullptr) == (e3v == nullptr), "e3u and e3v go together");
+        NFX_REQUIRE((thickness != nullptr) != (e3u != nullptr), "needs exactly one of thickness and (e3u, e3v)");
+        NFX_REQUIRE(nt >= 0 && nz > 0 && nz <= 3000, "bad sizes");
+        NFX_REQUIRE(dtype == NFX_F64 || dtype == NFX_F32, "dtype must be NFX_F64 or NFX_F32");
+        NFX_REQUIRE(ld >= p.grid->ncell, "ld must be >= the number of cells");
+        NFX_REQUIRE(!e3u || e3_nt == 1 || e3_nt == nt, "e3u/e3v must hold 1 (time-invariant) or nt time steps");
+        NFX_REQUIRE(c_nt == 1 || c_nt == nt, "the class field must hold 1 (time-invariant) or nt time steps");
+        check_class_bounds(nclasses, class_bounds);
+        section_csr(p);
+        if (nt == 0 || p.nsub == 0) return;
+        const cudaStream_t s = (cudaStream_t)stream;
+        const int steps = prepare_classes(p, nclasses, class_bounds, nt, s);
+        run_classes(p, u, v, dtype, thickness, e3u, e3v, e3u && e3_nt != 1 ? (int64_t)nz * ld : 0, arc1, arc2, cfield,
+                    c_nt != 1 ? (int64_t)nz * ld : 0, cfill, nclasses, ld, nt, nz, sverdrup, fill, steps, classes, s);
+    });
+}
+
 int nfx_edgeflux_to_cell_by_cell(const double* eflux, int nt, int ny, int nx, double* iv, void* stream) {
     return guarded([&] {
         int dev;
@@ -1099,6 +1181,8 @@ struct HostChunk {
     int t0;                    // first time step of the chunk
     int n;
     int slot;                  // staging slot of the chunk (0 or 1)
+    const void* cf;            // class field at the chunk's first step (nullptr without one)
+    int64_t c_tstride;         // its step stride (0: time-invariant)
 };
 
 struct HostPass {
@@ -1133,7 +1217,8 @@ struct PerStepPass : HostPass {
 
 static void host_pipeline(nfx_pli** self, const void* u, const void* v, int dtype_flags, const double* thickness,
                           const void* e3u, const void* e3v, int e3_nt, int e3_on_device, const double* arc1,
-                          const double* arc2, int nt, int nz, int chunk_steps, double* result, HostPass& pass) {
+                          const double* arc2, int nt, int nz, int chunk_steps, double* result, HostPass& pass,
+                          const void* cf = nullptr, int c_nt = 0) {
     NFX_REQUIRE(self && *self, "NULL handle");
     const bool e3 = e3u != nullptr || e3v != nullptr;
     NFX_REQUIRE(u && v && arc1 && arc2 && result, "NULL pointer");
@@ -1152,6 +1237,7 @@ static void host_pipeline(nfx_pli** self, const void* u, const void* v, int dtyp
     const size_t esize = dtype == NFX_F64 ? 8 : 4;
     const size_t step_bytes = esize * (size_t)nz * (size_t)ncell;
     const bool e3_streamed = e3 && !e3_on_device && e3_nt == nt && nt > 1;
+    const bool cf_streamed = cf && c_nt == nt && nt > 1;   // else uploaded once, as e3 of one step
     if (chunk_steps <= 0) {
         const size_t target = (size_t)256 << 20;  // per variable and slot
         chunk_steps = (int)std::max<size_t>(1, target / step_bytes);
@@ -1172,6 +1258,7 @@ static void host_pipeline(nfx_pli** self, const void* u, const void* v, int dtyp
             p.stage_e3u[i].ensure(step_bytes * chunk_steps);
             p.stage_e3v[i].ensure(step_bytes * chunk_steps);
         }
+        if (cf_streamed) p.stage_cf[i].ensure(step_bytes * chunk_steps);
     }
     p.stage_arc1.ensure(ncell);
     p.stage_arc2.ensure(ncell);
@@ -1196,6 +1283,11 @@ static void host_pipeline(nfx_pli** self, const void* u, const void* v, int dtyp
         d_e3u = p.stage_e3u[0].p;
         d_e3v = p.stage_e3v[0].p;
     }
+    if (cf && !cf_streamed) {
+        p.stage_cf[0].ensure(step_bytes);
+        NFX_CUDA(cudaMemcpyAsync(p.stage_cf[0].p, cf, step_bytes, cudaMemcpyHostToDevice, ks));
+        if (big_endian) bswap_inplace(p.stage_cf[0].p, step_bytes / esize, (int)esize, ks);
+    }
     pass.prepare(p, dtype, nt, nz, chunk_steps, result, ks);
     int slot = 0;
     bool used[2] = {false, false};
@@ -1204,12 +1296,13 @@ static void host_pipeline(nfx_pli** self, const void* u, const void* v, int dtyp
         const int n = std::min(chunk_steps, nt - t0);
         if (used[slot]) NFX_CUDA(cudaStreamWaitEvent(cs, p.ev_done[slot], 0));
         const size_t off = (size_t)t0 * step_bytes;
-        const void* src[4] = {(const unsigned char*)u + off, (const unsigned char*)v + off,
+        const void* src[5] = {(const unsigned char*)u + off, (const unsigned char*)v + off,
                               e3_streamed ? (const unsigned char*)e3u + off : nullptr,
-                              e3_streamed ? (const unsigned char*)e3v + off : nullptr};
-        unsigned char* dst[4] = {p.stage_u[slot].p, p.stage_v[slot].p, e3_streamed ? p.stage_e3u[slot].p : nullptr,
-                                 e3_streamed ? p.stage_e3v[slot].p : nullptr};
-        for (int q = 0; q < 4; ++q) {
+                              e3_streamed ? (const unsigned char*)e3v + off : nullptr,
+                              cf_streamed ? (const unsigned char*)cf + off : nullptr};
+        unsigned char* dst[5] = {p.stage_u[slot].p, p.stage_v[slot].p, e3_streamed ? p.stage_e3u[slot].p : nullptr,
+                                 e3_streamed ? p.stage_e3v[slot].p : nullptr, cf_streamed ? p.stage_cf[slot].p : nullptr};
+        for (int q = 0; q < 5; ++q) {
             if (!src[q]) continue;
             NFX_CUDA(cudaMemcpyAsync(dst[q], src[q], step_bytes * n, cudaMemcpyHostToDevice, cs));
             if (big_endian)   // file bytes as stored: swap on the device, behind the copy on the copy stream
@@ -1218,7 +1311,11 @@ static void host_pipeline(nfx_pli** self, const void* u, const void* v, int dtyp
         NFX_CUDA(cudaEventRecord(p.ev_ready[slot], cs));
         NFX_CUDA(cudaStreamWaitEvent(ks, p.ev_ready[slot], 0));
         HostChunk c{dst[0], dst[1], nullptr, nullptr, 0, e3 ? nullptr : p.stage_thick.p, p.stage_arc1.p,
-                    p.stage_arc2.p, t0, n, slot};
+                    p.stage_arc2.p, t0, n, slot, nullptr, 0};
+        if (cf) {
+            c.cf = cf_streamed ? dst[4] : p.stage_cf[0].p;
+            c.c_tstride = cf_streamed ? (int64_t)nz * ncell : 0;
+        }
         if (e3_streamed) {
             c.e3u = dst[2];
             c.e3v = dst[3];
@@ -1392,6 +1489,27 @@ struct WindowPass : HostPass {
     }
 };
 
+// class transport: one class pass per chunk, classes (nt, K, M)
+struct ClassPass : PerStepPass {
+    int sverdrup = 0, nclasses = 1, partial_steps = 1;
+    double fill = 0.0, cfill = 0.0;
+    const double* bounds = nullptr;
+    bool begin(PliDev& p, int, int, int) override {
+        section_csr(p);
+        per_step = (int64_t)nclasses * p.ntransects;
+        return p.nsub != 0;
+    }
+    void prepare(PliDev& p, int, int nt_, int, int chunk_steps, double*, cudaStream_t ks) override {
+        stage(p, nt_);
+        partial_steps = prepare_classes(p, nclasses, bounds, chunk_steps, ks);
+    }
+    void chunk(PliDev& p, int dtype, int nz, const HostChunk& k, cudaStream_t ks) override {
+        const int64_t ncell = p.grid->ncell;
+        run_classes(p, k.u, k.v, dtype, k.thickness, k.e3u, k.e3v, k.e3_tstride, k.arc1, k.arc2, k.cf, k.c_tstride,
+                    cfill, nclasses, ncell, k.n, nz, sverdrup, fill, partial_steps, out(p, k), ks);
+    }
+};
+
 int nfx_flux_series_host(nfx_pli** self, const void* u, const void* v, int dtype_flags, const double* thickness,
                          const double* arc1, const double* arc2, int nt, int nz, int sverdrup, double fill, int order,
                          int chunk_steps, double* series) {
@@ -1477,6 +1595,28 @@ int nfx_flux_section_window_sums_host(nfx_pli** self, const void* u, const void*
         host_pipeline(self, shift(u, true), shift(v, true), dtype_flags, thickness, shift(e3u, e3_per_step),
                       shift(e3v, e3_per_step), e3_per_step ? n : e3_nt, e3_on_device, arc1, arc2, n, nz, chunk_steps,
                       sums, pass);
+    });
+}
+
+int nfx_flux_classes_host(nfx_pli** self, const void* u, const void* v, const void* e3u, const void* e3v,
+                          int dtype_flags, int e3_nt, int e3_on_device, const double* thickness, const double* arc1,
+                          const double* arc2, int nt, int nz, const void* cfield, int c_nt, double cfill, int nclasses,
+                          const double* class_bounds, int sverdrup, double fill, int chunk_steps, double* classes) {
+    return guarded([&] {
+        NFX_REQUIRE((thickness != nullptr) != (e3u != nullptr || e3v != nullptr),
+                    "needs exactly one of thickness and (e3u, e3v)");
+        NFX_REQUIRE(cfield, "NULL pointer");
+        NFX_REQUIRE(nz <= 3000, "bad sizes");
+        NFX_REQUIRE(c_nt == 1 || c_nt == nt, "the class field must hold 1 (time-invariant) or nt time steps");
+        check_class_bounds(nclasses, class_bounds);
+        ClassPass pass;
+        pass.sverdrup = sverdrup;
+        pass.fill = fill;
+        pass.cfill = cfill;
+        pass.nclasses = nclasses;
+        pass.bounds = class_bounds;
+        host_pipeline(self, u, v, dtype_flags, thickness, e3u, e3v, e3_nt, e3_on_device, arc1, arc2, nt, nz,
+                      chunk_steps, classes, pass, cfield, c_nt);
     });
 }
 

@@ -200,6 +200,13 @@ struct PliDev {
     DevBuf<unsigned char> stage_u[2], stage_v[2], stage_e3u[2], stage_e3v[2];
     DevBuf<double> stage_eflux[2], stage_series, stage_thick, stage_arc1, stage_arc2;
     DevBuf<double> stage_windows[2];   // time-mean section: the window sums a chunk touches (two slots)
+    DevBuf<unsigned char> stage_cf[2];  // class transport: the class field of a chunk (two slots), or of every step
+    // class transport: warp tiles of the crossings (class_ntiles + 1 starts, per transect the range of its tiles), built
+    // on first use after computeWeights (class_ntiles < 0: not built); the bounds of the last call; partial sums
+    int64_t class_ntiles = -1;
+    std::vector<int64_t> h_class_tiles, h_class_tr_tiles;
+    DevBuf<int64_t> class_tiles, class_tr_tiles;
+    DevBuf<double> class_bounds, class_partial;
     cudaStream_t copy_stream = nullptr, compute_stream = nullptr;
     cudaEvent_t ev_ready[2] = {nullptr, nullptr}, ev_done[2] = {nullptr, nullptr};
 };
@@ -293,5 +300,17 @@ void flux_section_windows(const void* u, const void* v, int dtype, const double*
                           const int32_t* idx, const double* w, int64_t nsub, int64_t ncell, int64_t ld, int nz,
                           int nlayers, const int* levels, int sverdrup, double fill, const int* bounds, int w0, int nwin,
                           int t_first, int t_end, int continue_first, double* sums, cudaStream_t s);
+// class transport (nfx_section.cu): classes (nt, K, M), the per-level section flux of every crossing binned by the class
+// field at its cell (cfield (1 or nt, nz, ld) of the dtype of u, v; c_tstride 0 or nz * ld) into the classes
+// [bounds[j], bounds[j+1]) (device, K + 1 ascending doubles).  tile_start (ntiles + 1): the warp tiles of at most 32
+// crossings of one transect, tr_tiles (M + 1) the tiles of every transect; partial: scratch of
+// partial_steps * ntiles * K doubles, the steps are run in batches of at most partial_steps.
+constexpr int kClassMax = 96;   // the per-thread class sums of a 256-thread CTA: 2 KB of shared memory per class
+void flux_classes(const void* u, const void* v, int dtype, const double* thickness, const void* e3u, const void* e3v,
+                  int64_t e3_tstride, const double* arc1, const double* arc2, const int32_t* idx, const double* w,
+                  const int32_t* cell, const void* cfield, int64_t c_tstride, double cfill, const double* bounds, int K,
+                  const int64_t* tile_start, int64_t ntiles, const int64_t* tr_tiles, int ntransects, int64_t ncell,
+                  int64_t ld, int nt, int nz, int sverdrup, double fill, double* partial, int partial_steps,
+                  double* classes, cudaStream_t s);
 
 }  // namespace nfx

@@ -1012,6 +1012,7 @@ void pli_compute_weights(PliDev& p, int ntransects, const int* offsets, const do
     p.h_map_offsets.assign(ntransects + 1, 0);
     p.has_compact = (g.ny > 0 && g.nx > 0);
     p.plan[0].built = p.plan[1].built = false;
+    p.class_ntiles = -1;
     for (int o = 0; o < 2; ++o)
         for (int l = 0; l < 2; ++l) p.csr[o][l].nnz = 0;
     p.sub_offsets.ensure(ntransects + 1);

@@ -37,6 +37,66 @@ struct SectionShape {
     static constexpr int ctas = E3 ? 2 : 3;
 };
 
+// The operation sequence of one crossing, shared by the section kernels.  section_edges: the column of u or v every
+// edge of sub-segment s reads (at offset `off`, its scale factor at `e3_off`), the factor that turns a column sum into
+// K2's edge flux, its weight, and whether it is live (idx -1: the south edge of row 0, whose flux is 0).
+template <typename T, bool E3>
+__device__ __forceinline__ void section_edges(const T* __restrict__ u, const T* __restrict__ v, const T* __restrict__ e3u,
+                                              const T* __restrict__ e3v, const double* __restrict__ arc1,
+                                              const double* __restrict__ arc2, const int32_t* __restrict__ idx,
+                                              const double* __restrict__ w, int64_t s, int64_t ncell, int64_t off,
+                                              int64_t e3_off, const T* (&pc)[4], const T* (&pe)[4], double (&arc)[4],
+                                              double (&wt)[4], bool (&live)[4]) {
+#pragma unroll
+    for (int e = 0; e < 4; ++e) {
+        const int32_t j = idx[4 * s + e];
+        live[e] = j >= 0;
+        const bool isv = j >= ncell;
+        const int64_t col = !live[e] ? 0 : isv ? j - ncell : j;   // idx < 0: a harmless address, the flux is 0
+        pc[e] = (isv ? v : u) + off + col;
+        pe[e] = E3 ? (isv ? e3v : e3u) + e3_off + col : nullptr;
+        arc[e] = !live[e] ? 0.0 : isv ? -arc2[col] : arc1[col];   // eV = (-sum) * arc2: the negation is exact
+        wt[e] = w[4 * s + e];
+    }
+}
+
+// the 4 columns (and, with E3, their scale factors) of one level, `off` / `e3_off` past the pointers of section_edges
+template <typename T, bool E3>
+__device__ __forceinline__ void section_load(const T* const (&pc)[4], const T* const (&pe)[4], int64_t off,
+                                             int64_t e3_off, T (&x)[4], T (&ex)[4]) {
+#pragma unroll
+    for (int e = 0; e < 4; ++e) {
+        x[e] = __ldg(pc[e] + off);
+        if constexpr (E3) ex[e] = __ldg(pe[e] + e3_off);
+    }
+}
+
+// one level into the 4 column sums: acc += dz (or e3) * u, NaN and the marker as 0
+template <typename T, bool E3>
+__device__ __forceinline__ void section_level(double (&acc)[4], double d, const T (&x)[4], const T (&ex)[4], T fill,
+                                              int has_fill) {
+#pragma unroll
+    for (int e = 0; e < 4; ++e) {
+        const double de = E3 ? clean<T>(ex[e], fill, has_fill) : d;
+        acc[e] = __dadd_rn(acc[e], __dmul_rn(de, clean<T>(x[e], fill, has_fill)));
+    }
+}
+
+// the section value of 4 column sums: the eflux value of K2 per edge ((sum * arc) [* 6.371], -sum * arc2 for eV; 0 for
+// the south edge of row 0), their weighted sum in edge order
+__device__ __forceinline__ double section_value(const double (&acc)[4], const double (&arc)[4], const double (&wt)[4],
+                                                const bool (&live)[4], double scale, int use_scale) {
+    double r = 0.0;
+#pragma unroll
+    for (int e = 0; e < 4; ++e) {
+        double f = __dmul_rn(acc[e], arc[e]);
+        if (use_scale) f = __dmul_rn(f, scale);
+        f = live[e] ? f : 0.0;
+        r = e == 0 ? __dmul_rn(wt[0], f) : __dadd_rn(r, __dmul_rn(wt[e], f));
+    }
+    return r;
+}
+
 template <typename T, bool E3>
 __global__ void __launch_bounds__(kSectionBlock, SectionShape<T, E3>::ctas)
 k_flux_section(const T* __restrict__ u, const T* __restrict__ v, const T* __restrict__ e3u, const T* __restrict__ e3v,
@@ -57,44 +117,22 @@ k_flux_section(const T* __restrict__ u, const T* __restrict__ v, const T* __rest
     const int64_t t = t0 + blockIdx.y;
     const T* pc[4];        // column of every edge at level 0 of step t
     const T* pe[4];        // E3: its scale factors
-    double arc[4], wt[4], acc[4];
+    double arc[4], wt[4], acc[4] = {0.0, 0.0, 0.0, 0.0};
     bool live[4];
-#pragma unroll
-    for (int e = 0; e < 4; ++e) {
-        const int32_t j = idx[4 * s + e];
-        live[e] = j >= 0;
-        const bool isv = j >= ncell;
-        const int64_t col = !live[e] ? 0 : isv ? j - ncell : j;   // idx < 0: a harmless address, the flux is 0
-        pc[e] = (isv ? v : u) + t * nz * ld + col;
-        pe[e] = E3 ? (isv ? e3v : e3u) + t * e3_tstride + col : nullptr;
-        arc[e] = !live[e] ? 0.0 : isv ? -arc2[col] : arc1[col];   // eV = (-sum) * arc2: the negation is exact
-        wt[e] = w[4 * s + e];
-        acc[e] = 0.0;
-    }
+    section_edges<T, E3>(u, v, e3u, e3v, arc1, arc2, idx, w, s, ncell, t * nz * ld, t * e3_tstride, pc, pe, arc, wt,
+                         live);
     double* out = section + (t * nlayers) * nsub + s;
     int layer = 0, next = s_lev[1];
     const int kend = s_lev[nlayers];
     int k = s_lev[0];
-    // level kk into the 4 column sums; after the last level of a layer: the 4 edge fluxes, their weighted sum in
-    // edge order, one streaming store (the layering is the same for every thread: the branch does not diverge)
+    // level kk into the 4 column sums; after the last level of a layer: the section value, one streaming store (the
+    // layering is the same for every thread: the branch does not diverge)
     auto step = [&](int kk, const T (&x)[4], const T (&ex)[4]) {
-        const double d = E3 ? 0.0 : s_dz[kk];
-#pragma unroll
-        for (int e = 0; e < 4; ++e) {
-            const double de = E3 ? clean<T>(ex[e], fill, has_fill) : d;
-            acc[e] = __dadd_rn(acc[e], __dmul_rn(de, clean<T>(x[e], fill, has_fill)));
-        }
+        section_level<T, E3>(acc, E3 ? 0.0 : s_dz[kk], x, ex, fill, has_fill);
         if (kk + 1 == next) {
-            double r = 0.0;
+            const double r = section_value(acc, arc, wt, live, scale, use_scale);
 #pragma unroll
-            for (int e = 0; e < 4; ++e) {
-                // the eflux value of K2: (sum * arc) [* 6.371], -sum * arc2 for eV; 0 for the south edge of row 0
-                double f = __dmul_rn(acc[e], arc[e]);
-                if (use_scale) f = __dmul_rn(f, scale);
-                f = live[e] ? f : 0.0;
-                r = e == 0 ? __dmul_rn(wt[0], f) : __dadd_rn(r, __dmul_rn(wt[e], f));
-                acc[e] = 0.0;
-            }
+            for (int e = 0; e < 4; ++e) acc[e] = 0.0;
             __stcs(out + (int64_t)layer * nsub, r);
             ++layer;
             next = layer < nlayers ? s_lev[layer + 1] : -1;
@@ -103,22 +141,13 @@ k_flux_section(const T* __restrict__ u, const T* __restrict__ v, const T* __rest
     for (; k + UNROLL <= kend; k += UNROLL) {
         T x[UNROLL][4], ex[UNROLL][4];
 #pragma unroll
-        for (int q = 0; q < UNROLL; ++q)
-#pragma unroll
-            for (int e = 0; e < 4; ++e) {
-                x[q][e] = __ldg(pc[e] + (int64_t)(k + q) * ld);
-                if constexpr (E3) ex[q][e] = __ldg(pe[e] + (int64_t)(k + q) * ld);
-            }
+        for (int q = 0; q < UNROLL; ++q) section_load<T, E3>(pc, pe, (int64_t)(k + q) * ld, (int64_t)(k + q) * ld, x[q], ex[q]);
 #pragma unroll
         for (int q = 0; q < UNROLL; ++q) step(k + q, x[q], ex[q]);
     }
     for (; k < kend; ++k) {
         T x[4], ex[4];
-#pragma unroll
-        for (int e = 0; e < 4; ++e) {
-            x[e] = __ldg(pc[e] + (int64_t)k * ld);
-            if constexpr (E3) ex[e] = __ldg(pe[e] + (int64_t)k * ld);
-        }
+        section_load<T, E3>(pc, pe, (int64_t)k * ld, (int64_t)k * ld, x, ex);
         step(k, x, ex);
     }
 }
@@ -159,63 +188,166 @@ k_flux_section_windows(const T* __restrict__ u, const T* __restrict__ v, const T
     const T* pe[4];
     double arc[4], wt[4];
     bool live[4];
-#pragma unroll
-    for (int e = 0; e < 4; ++e) {
-        const int32_t j = idx[4 * s + e];
-        live[e] = j >= 0;
-        const bool isv = j >= ncell;
-        const int64_t col = !live[e] ? 0 : isv ? j - ncell : j;
-        pc[e] = (isv ? v : u) + (int64_t)kbeg * ld + col;
-        pe[e] = E3 ? (isv ? e3v : e3u) + (int64_t)kbeg * ld + col : nullptr;
-        arc[e] = !live[e] ? 0.0 : isv ? -arc2[col] : arc1[col];
-        wt[e] = w[4 * s + e];
-    }
+    section_edges<T, E3>(u, v, e3u, e3v, arc1, arc2, idx, w, s, ncell, (int64_t)kbeg * ld, (int64_t)kbeg * ld, pc, pe,
+                         arc, wt, live);
     double* out = sums + y * nsub + s;
     double total = continue_first && y < nlayers ? __ldcs(out) : 0.0;
     for (int t = tb; t < te; ++t) {
         const int64_t tu = (int64_t)t * nz * ld, tx = (int64_t)t * e3_tstride;
         double acc[4] = {0.0, 0.0, 0.0, 0.0};
-        auto level = [&](int kk, const T (&x)[4], const T (&ex)[4]) {
-            const double d = E3 ? 0.0 : s_dz[kk];
-#pragma unroll
-            for (int e = 0; e < 4; ++e) {
-                const double de = E3 ? clean<T>(ex[e], fill, has_fill) : d;
-                acc[e] = __dadd_rn(acc[e], __dmul_rn(de, clean<T>(x[e], fill, has_fill)));
-            }
-        };
         int k = kbeg;
         for (; k + UNROLL <= kend; k += UNROLL) {
             T x[UNROLL][4], ex[UNROLL][4];
 #pragma unroll
             for (int q = 0; q < UNROLL; ++q)
+                section_load<T, E3>(pc, pe, tu + (int64_t)(k - kbeg + q) * ld, tx + (int64_t)(k - kbeg + q) * ld, x[q],
+                                    ex[q]);
 #pragma unroll
-                for (int e = 0; e < 4; ++e) {
-                    x[q][e] = __ldg(pc[e] + tu + (int64_t)(k - kbeg + q) * ld);
-                    if constexpr (E3) ex[q][e] = __ldg(pe[e] + tx + (int64_t)(k - kbeg + q) * ld);
-                }
-#pragma unroll
-            for (int q = 0; q < UNROLL; ++q) level(k + q, x[q], ex[q]);
+            for (int q = 0; q < UNROLL; ++q)
+                section_level<T, E3>(acc, E3 ? 0.0 : s_dz[k + q], x[q], ex[q], fill, has_fill);
         }
         for (; k < kend; ++k) {
             T x[4], ex[4];
-#pragma unroll
-            for (int e = 0; e < 4; ++e) {
-                x[e] = __ldg(pc[e] + tu + (int64_t)(k - kbeg) * ld);
-                if constexpr (E3) ex[e] = __ldg(pe[e] + tx + (int64_t)(k - kbeg) * ld);
-            }
-            level(k, x, ex);
+            section_load<T, E3>(pc, pe, tu + (int64_t)(k - kbeg) * ld, tx + (int64_t)(k - kbeg) * ld, x, ex);
+            section_level<T, E3>(acc, E3 ? 0.0 : s_dz[k], x, ex, fill, has_fill);
         }
-        double r = 0.0;
-#pragma unroll
-        for (int e = 0; e < 4; ++e) {
-            double f = __dmul_rn(acc[e], arc[e]);
-            if (use_scale) f = __dmul_rn(f, scale);
-            f = live[e] ? f : 0.0;
-            r = e == 0 ? __dmul_rn(wt[0], f) : __dadd_rn(r, __dmul_rn(wt[e], f));
-        }
-        total = __dadd_rn(total, r);
+        total = __dadd_rn(total, section_value(acc, arc, wt, live, scale, use_scale));
     }
     __stcs(out, total);
+}
+
+// Class transport: the flux across every transect binned by a T-grid field c (temperature, salinity, density...).
+// One thread per (time step, crossing), the crossings of one transect in warp tiles of at most 32 consecutive
+// crossings (tile_start, K1's emission order; a tile never spans two transects), 8 tiles per CTA.  Per level the
+// thread gathers its 4 columns as k_flux_section does, forms the crossing's level flux with the section's operations
+// (a one-level layer: the bits of fluxSection(layers=range(nz+1))), loads c at its cell and level, finds the class
+// j with b_j <= c < b_{j+1} by a search over the bounds in shared memory and adds the flux to its own sum of class j
+// in shared memory (s_acc[j][thread]: no two threads share a word).  NaN, the marker cfill and values outside
+// [b0, bK) count nowhere.  After the last level each warp folds its 32 per-crossing sums of every class with a fixed
+// shuffle tree into one partial value per (step, tile, class); k_reduce_class_tiles adds a transect's tiles in
+// ascending order.  No atomics: the bits depend on nothing but the inputs.
+// levels in flight of k_flux_classes (5 loads per level, 9 with E3) and CTAs per SM: the section's, one level fewer
+// without E3 (4 levels spill at 80 registers, profiles/r7_classes_ptxas.md)
+template <typename T, bool E3>
+struct ClassShape {
+    static constexpr int unroll = E3 ? SectionShape<T, E3>::unroll : 3;
+    static constexpr int ctas = SectionShape<T, E3>::ctas;
+};
+
+template <typename T, bool E3>
+__global__ void __launch_bounds__(kSectionBlock, ClassShape<T, E3>::ctas)
+k_flux_classes(const T* __restrict__ u, const T* __restrict__ v, const T* __restrict__ e3u, const T* __restrict__ e3v,
+               int64_t e3_tstride, const double* __restrict__ dz, const double* __restrict__ arc1,
+               const double* __restrict__ arc2, const int32_t* __restrict__ idx, const double* __restrict__ w,
+               const int32_t* __restrict__ cell, const T* __restrict__ cf, int64_t c_tstride, T cfill, int has_cfill,
+               const double* __restrict__ bounds, int K, const int64_t* __restrict__ tile_start, int64_t ntiles,
+               int64_t ncell, int64_t ld, int nz, double scale, int use_scale, T fill, int has_fill, int64_t t0,
+               double* __restrict__ partial) {
+    constexpr int UNROLL = ClassShape<T, E3>::unroll;
+    extern __shared__ double s_mem[];
+    double* s_acc = s_mem;                                  // [K][kSectionBlock] per-thread class sums
+    double* s_b = s_acc + (size_t)K * kSectionBlock;        // [K + 1] bounds
+    double* s_dz = s_b + K + 1;                             // [nz] dz (without E3)
+    for (int i = threadIdx.x; i <= K; i += kSectionBlock) s_b[i] = bounds[i];
+    if constexpr (!E3)
+        for (int k = threadIdx.x; k < nz; k += kSectionBlock) s_dz[k] = dz[k];
+    for (int j = 0; j < K; ++j) s_acc[j * kSectionBlock + threadIdx.x] = 0.0;
+    __syncthreads();
+    const int64_t tile = (int64_t)blockIdx.x * (kSectionBlock / 32) + threadIdx.x / 32;
+    if (tile >= ntiles) return;                             // the whole warp
+    const int lane = threadIdx.x & 31;
+    const int64_t t = t0 + blockIdx.y;
+    const int64_t s = tile_start[tile] + lane;
+    double* acc_j = s_acc + threadIdx.x;                    // this thread's sum of class j: acc_j[j * kSectionBlock]
+    if (s < tile_start[tile + 1]) {
+        const T* pc[4];
+        const T* pe[4];
+        double arc[4], wt[4];
+        bool live[4];
+        section_edges<T, E3>(u, v, e3u, e3v, arc1, arc2, idx, w, s, ncell, t * nz * ld, t * e3_tstride, pc, pe, arc,
+                             wt, live);
+        const T* pcl = cf + t * c_tstride + cell[s];
+        int top = 1;                                        // the largest power of two <= K + 1
+        while (2 * top <= K + 1) top *= 2;
+        auto level = [&](int kk, const T (&x)[4], const T (&ex)[4], T c) {
+            double acc[4] = {0.0, 0.0, 0.0, 0.0};
+            section_level<T, E3>(acc, E3 ? 0.0 : s_dz[kk], x, ex, fill, has_fill);
+            const double f = section_value(acc, arc, wt, live, scale, use_scale);
+            const double xc = (double)c;
+            if (xc != xc || (has_cfill && c == cfill)) return;
+            int pos = 0;                                    // the number of bounds <= xc
+            for (int h = top; h > 0; h >>= 1)
+                if (pos + h <= K + 1 && s_b[pos + h - 1] <= xc) pos += h;
+            if (pos >= 1 && pos <= K) acc_j[(pos - 1) * kSectionBlock] = __dadd_rn(acc_j[(pos - 1) * kSectionBlock], f);
+        };
+        int k = 0;
+        for (; k + UNROLL <= nz; k += UNROLL) {
+            T x[UNROLL][4], ex[UNROLL][4], c[UNROLL];
+#pragma unroll
+            for (int q = 0; q < UNROLL; ++q) {
+                section_load<T, E3>(pc, pe, (int64_t)(k + q) * ld, (int64_t)(k + q) * ld, x[q], ex[q]);
+                c[q] = __ldg(pcl + (int64_t)(k + q) * ld);
+            }
+#pragma unroll
+            for (int q = 0; q < UNROLL; ++q) level(k + q, x[q], ex[q], c[q]);
+        }
+        for (; k < nz; ++k) {
+            T x[4], ex[4];
+            section_load<T, E3>(pc, pe, (int64_t)k * ld, (int64_t)k * ld, x, ex);
+            level(k, x, ex, __ldg(pcl + (int64_t)k * ld));
+        }
+    }
+    __syncwarp();
+    // lane l adds lane l + o for o = 16, 8, 4, 2, 1 (absent crossings hold +0): one value per (step, tile, class)
+    double* out = partial + ((int64_t)blockIdx.y * ntiles + tile) * K;
+    for (int j = 0; j < K; ++j) {
+        double a = acc_j[j * kSectionBlock];
+#pragma unroll
+        for (int o = 16; o > 0; o >>= 1) a = __dadd_rn(a, __shfl_down_sync(0xffffffffu, a, o));
+        if (lane == 0) out[j] = a;
+    }
+}
+
+// classes[t, j, m] = the tiles of transect m added in ascending order from +0 (partial: the steps from t0 on)
+__global__ void k_reduce_class_tiles(const double* __restrict__ partial, int nt, int64_t ntiles, int K,
+                                     const int64_t* __restrict__ tr_tiles, int ntransects, int64_t t0,
+                                     double* __restrict__ classes) {
+    const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= (int64_t)nt * ntransects * K) return;
+    const int j = (int)(i % K);
+    const int m = (int)(i / K % ntransects);
+    const int64_t t = i / ((int64_t)K * ntransects);
+    double a = 0.0;
+    for (int64_t g = tr_tiles[m]; g < tr_tiles[m + 1]; ++g) a = __dadd_rn(a, partial[(t * ntiles + g) * K + j]);
+    classes[((t0 + t) * K + j) * ntransects + m] = a;
+}
+
+template <typename T, bool E3>
+void launch_classes(const void* u, const void* v, const void* e3u, const void* e3v, int64_t e3_tstride,
+                    const double* dz, const double* arc1, const double* arc2, const int32_t* idx, const double* w,
+                    const int32_t* cell, const void* cfield, int64_t c_tstride, double cfill, const double* bounds,
+                    int K, const int64_t* tile_start, int64_t ntiles, const int64_t* tr_tiles, int ntransects,
+                    int64_t ncell, int64_t ld, int nt, int nz, int sverdrup, double fill, double* partial,
+                    int partial_steps, double* classes, cudaStream_t s) {
+    const double scale = 6371000.0 / 1.e6;
+    const size_t smem = sizeof(double) * ((size_t)K * kSectionBlock + K + 1 + (E3 ? 0 : nz));
+    NFX_CUDA(cudaFuncSetAttribute(k_flux_classes<T, E3>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    const unsigned gx = (unsigned)((ntiles + kSectionBlock / 32 - 1) / (kSectionBlock / 32));
+    const int batch = std::min(partial_steps, 65535);
+    for (int t0 = 0; t0 < nt; t0 += batch) {
+        const int n = std::min(batch, nt - t0);
+        k_flux_classes<T, E3><<<dim3(gx, (unsigned)n), kSectionBlock, smem, s>>>(
+            (const T*)u, (const T*)v, (const T*)e3u, (const T*)e3v, e3_tstride, dz, arc1, arc2, idx, w, cell,
+            (const T*)cfield, c_tstride, (T)cfill, !(cfill != cfill), bounds, K, tile_start, ntiles, ncell, ld, nz, scale,
+            sverdrup, (T)fill, !(fill != fill), t0, partial);
+        count_launch();
+        NFX_CUDA(cudaGetLastError());
+        const int64_t nr = (int64_t)n * ntransects * K;
+        k_reduce_class_tiles<<<(unsigned)((nr + 255) / 256), 256, 0, s>>>(partial, n, ntiles, K, tr_tiles, ntransects,
+                                                                         t0, classes);
+        count_launch();
+        NFX_CUDA(cudaGetLastError());
+    }
 }
 
 template <typename T, bool E3>
@@ -319,6 +451,40 @@ void flux_section_windows(const void* u, const void* v, int dtype, const double*
             NFX_SECTION_WINDOWS(float, false);
     }
 #undef NFX_SECTION_WINDOWS
+}
+
+void flux_classes(const void* u, const void* v, int dtype, const double* thickness, const void* e3u, const void* e3v,
+                  int64_t e3_tstride, const double* arc1, const double* arc2, const int32_t* idx, const double* w,
+                  const int32_t* cell, const void* cfield, int64_t c_tstride, double cfill, const double* bounds, int K,
+                  const int64_t* tile_start, int64_t ntiles, const int64_t* tr_tiles, int ntransects, int64_t ncell,
+                  int64_t ld, int nt, int nz, int sverdrup, double fill, double* partial, int partial_steps,
+                  double* classes, cudaStream_t s) {
+    NFX_REQUIRE(u && v && arc1 && arc2 && idx && w && cell && cfield && bounds && tile_start && tr_tiles && partial &&
+                    classes, "classes: NULL pointer");
+    NFX_REQUIRE((e3u == nullptr) == (e3v == nullptr) && (thickness != nullptr) != (e3u != nullptr),
+                "classes: needs exactly one of thickness and (e3u, e3v)");
+    NFX_REQUIRE(nz > 0 && nz <= 3000 && nt >= 0 && ld >= ncell && partial_steps >= 1, "classes: bad sizes");
+    NFX_REQUIRE(K >= 1 && K <= kClassMax, "classes: K must be in [1, " + std::to_string(kClassMax) + "]");
+    NFX_REQUIRE(ntiles / (kSectionBlock / 32) < 2147483647ll, "classes: too many sub-segments");
+    if (nt == 0 || ntiles == 0) return;
+    const bool e3 = e3u != nullptr;
+#define NFX_CLASSES(T, E3)                                                                                            \
+    launch_classes<T, E3>(u, v, e3u, e3v, e3_tstride, thickness, arc1, arc2, idx, w, cell, cfield, c_tstride, cfill,  \
+                          bounds, K, tile_start, ntiles, tr_tiles, ntransects, ncell, ld, nt, nz, sverdrup, fill,     \
+                          partial, partial_steps, classes, s)
+    if (dtype == NFX_F64) {
+        if (e3)
+            NFX_CLASSES(double, true);
+        else
+            NFX_CLASSES(double, false);
+    } else {
+        NFX_REQUIRE(dtype == NFX_F32, "classes: dtype must be NFX_F64 or NFX_F32");
+        if (e3)
+            NFX_CLASSES(float, true);
+        else
+            NFX_CLASSES(float, false);
+    }
+#undef NFX_CLASSES
 }
 
 }  // namespace nfx

@@ -47,6 +47,7 @@ class Field(object):
     def __init__(self, tFile, uFile, vFile, lonLatZPoints, sverdrup=False, verbose=True, meshFile=None):
         import torch
         self.sverdrup = sverdrup
+        self.tFile = tFile
         with ncio.open_dataset(tFile) as nc:
             bounds_lat = nc['bounds_lat'][:]
             bounds_lon = nc['bounds_lon'][:]
@@ -309,7 +310,7 @@ class Field(object):
                 return None
             return [nemoflux_gpu.H5DeviceReader(d, self.device) for d in readers]
 
-    def _flux_series_device_decode(self, readers, chunk_steps, prefetch, fn, steps):
+    def _flux_series_device_decode(self, readers, chunk_steps, prefetch, fn, steps, aux=None):
         """fn over chunked + deflated uo / vo: the COMPRESSED chunks cross PCIe and are inflated, unshuffled and
         placed on the device (csrc/nfx_inflate.cu), then fn (the series' K2 + K3, or the section) runs on the decoded
         slab.  A reader thread copies the compressed chunks of block i + 1 from the memory-mapped files into pinned
@@ -339,6 +340,8 @@ class Field(object):
         def stage(i):
             t0, m = blocks[i]
             staged[i] = tuple(r.stage([t0, 0, 0, 0], [t0 + m, self.nz, self.ny, self.nx]) for r in readers)
+            if aux is not None:
+                staged[('aux', i)] = aux(t0, m, numpy.dtype(str(readers[0].tdtype).replace('torch.', '')))
 
         # stage() ends by sending its bytes to one of the reader's two device buffers; the reader thread prepares block
         # i + 1 (file -> pinned -> device) while block i is inflated and integrated
@@ -355,8 +358,9 @@ class Field(object):
                 ud, vd = readers[0].decode(st[0]), readers[1].decode(st[1])
             if i + 1 < len(blocks) and not prefetch:
                 stage(i + 1)
+            more = {} if aux is None else dict(aux=staged.pop(('aux', i)))
             fn(t0, m, ud, vd, self._d_thickness, self._d_arc1, self._d_arc2, sverdrup=self.sverdrup, fill=fill,
-               e3u=self._d_e3u, e3v=self._d_e3v)
+               e3u=self._d_e3u, e3v=self._d_e3v, **more)
             if th is not None:
                 th.join()
         self.last_ingest = dict(path='device decode', bytes_compressed=sum(r.bytes_compressed for r in readers),
@@ -435,16 +439,59 @@ class Field(object):
         sums /= numpy.diff(b).astype(numpy.float64)[:, None, None]
         return sums
 
-    def _over_chunks(self, fn, chunk_steps, prefetch, device_decode, steps=None):
+    def fluxClasses(self, var, bounds, file=None, chunk_steps=0, prefetch=True, device_decode=None):
+        """(nt, K, M) class transport: every transect's flux binned by the T-grid variable `var` (thetao, so, sigma0...)
+        into the classes [b_j, b_{j+1}) of bounds, see PolylineIntegral.fluxClasses.  var is read from `file` (default:
+        the T file), (nt, nz, ny, nx) or time-invariant (nz, ny, nx), with its _FillValue, block by block next to uo/vo
+        on the pipeline of fluxSeries, and converted to the storage type of uo/vo."""
+        import torch
+        b = numpy.asarray(bounds, numpy.float64).reshape(-1)
+        nc = ncio.open_dataset(file or self.tFile)
+        try:
+            cv = nc[var]
+            shape = tuple(cv.shape)
+            if shape[-3:] != (self.nz, self.ny, self.nx) or len(shape) not in (3, 4) or \
+                    (len(shape) == 4 and shape[0] not in (1, self.nt)):
+                raise RuntimeError(f'ERROR: {var} has shape {shape}, expected (nt, nz, ny, nx) or (nz, ny, nx) = '
+                                   f'({self.nt}, {self.nz}, {self.ny}, {self.nx})')
+            steady = len(shape) == 3 or shape[0] == 1
+            cfill = self._fill(nc, var)
+            fixed = self._slab(nc, var, 0, 1) if steady else None
+            once = {}                       # the time-invariant field, converted (and uploaded) once per form
+            out = numpy.zeros((self.nt, b.size - 1, len(self.plis)))
+
+            def read(t0, m, dtype):
+                """on the reader thread, next to uo/vo: the block in the storage type and byte order of uo/vo"""
+                return numpy.ascontiguousarray(self._slab(nc, var, t0, m).astype(dtype))
+
+            def fn(t0, m, u, v, *args, aux=None, **kw):
+                on_host = isinstance(u, numpy.ndarray)
+                if steady:
+                    key = u.dtype if on_host else (u.device, u.dtype)
+                    if key not in once:
+                        c = numpy.ascontiguousarray(fixed.astype(u.dtype if on_host else fixed.dtype.newbyteorder('=')))
+                        once[key] = c if on_host else torch.from_numpy(c).to(u.device, u.dtype).reshape(1, self.nz, -1)
+                    c = once[key]
+                else:
+                    c = aux if on_host else torch.from_numpy(aux).to(u.device).reshape(m, self.nz, -1)
+                out[t0:t0 + m] = _host(self.pli.fluxClasses(u, v, *args, cfield=c, bounds=b, cfill=cfill, **kw))
+            self._over_chunks(fn, chunk_steps, prefetch, device_decode, aux=None if steady else read)
+        finally:
+            nc.close()
+        return out
+
+    def _over_chunks(self, fn, chunk_steps, prefetch, device_decode, steps=None, aux=None):
         """fn(t0, m, u, v, thickness, arc1, arc2, sverdrup=, fill=, e3u=, e3v=) over blocks [t0, t0 + m) of the time
-        steps [steps[0], steps[1]) (default: all) read from the files: the pipeline of fluxSeries"""
+        steps [steps[0], steps[1]) (default: all) read from the files: the pipeline of fluxSeries.  aux(t0, m, dtype)
+        (optional) reads one more array per block on the reader thread, dtype the numpy type of the block's uo/vo;
+        fn gets it as aux="""
         import threading
         import torch
         steps = (0, self.nt) if steps is None else steps
         if device_decode is not False:
             readers = self._device_readers()
             if readers is not None:
-                return self._flux_series_device_decode(readers, chunk_steps, prefetch, fn, steps)
+                return self._flux_series_device_decode(readers, chunk_steps, prefetch, fn, steps, aux)
             if device_decode is True:
                 raise RuntimeError('ERROR: uo / vo are not chunked HDF5 variables with a [shuffle,] [deflate] pipeline')
         t_lo, t_hi = steps
@@ -483,6 +530,8 @@ class Field(object):
             """file -> pinned buffer, one task per (variable, time step): byte-order conversion in parallel"""
             t0, m = chunks[i]
             nu, nv = views[slot]
+            if aux is not None:
+                state[('aux', i)] = aux(t0, m, nu.dtype)
             if four_d and (fill_v != fill_v or fill_v == fill_u):
                 # one task per (variable, time step, slab of levels): enough tasks to keep every worker copying
                 nsplit = max(1, min(self.nz, -(-2 * workers // (2 * m))))
@@ -506,8 +555,9 @@ class Field(object):
                 th = threading.Thread(target=read, args=(i + 1, 1 - slot))
                 th.start()
             nu, nv = views[slot]                    # numpy views of the pinned buffers (kept alive by `bufs`)
+            more = {} if aux is None else dict(aux=state.pop(('aux', i)))
             fn(t0, m, nu[:m], nv[:m], self.thickness, arc1, arc2, sverdrup=self.sverdrup, fill=state.pop(i),
-               e3u=self._d_e3u, e3v=self._d_e3v)
+               e3u=self._d_e3u, e3v=self._d_e3v, **more)
             if th is not None:
                 th.join()
             elif i + 1 < len(chunks):

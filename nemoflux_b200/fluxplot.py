@@ -1,7 +1,8 @@
 """fluxplot -- drop-in for nemoflux/fluxplot.py: flux time series of every transect (same flags).
 
     python -m nemoflux_b200.fluxplot -t T.nc -u U.nc -v V.nc -i "../data/nz/S*.txt" [-s] [--output series.csv]
-        [--layers "0,10,35,75" | --depthLayers "0,200,1000,6000"] [--section section.nc] [--timeMean N|month|year]
+        [--layers "0,10,35,75" | --depthLayers "0,200,1000,6000" | --classField NAME[:FILE] --classBounds=b0,b1,...]
+        [--section section.nc] [--timeMean N|month|year]
 
 The reference loops ``for itime: fld.update(); for pli: pli.getIntegral(...)`` (fluxplot.py:51-59); here the
 whole (nt, M) series comes from Field.fluxSeries() (K2+K3 over chunks of time steps).  The series is printed
@@ -12,6 +13,10 @@ interfaces that were integrated.
 --section FILE.nc also writes the transport section (Field.fluxSection): the flux across every cell crossing of every
 transect per layer (the layers of --layers / --depthLayers, else one per level) as a NetCDF classic (64-bit offset)
 file, see writeSection.
+--classField NAME[:FILE] --classBounds=b0,b1,... split every transect's flux by the class of a T-grid variable
+(thetao, so, sigma0...; from the T file unless FILE is given): one column per (transect, class), headed
+label[b_j–b_{j+1}), the water with b_j <= value < b_{j+1} (Field.fluxClasses).  Not combined with --layers /
+--depthLayers.
 --timeMean N|month|year averages over windows of N steps, or of the steps of each calendar month / year
 (timeobj.timeWindows): the printed and CSV series become window means (windowMeans), one row per window labelled
 first/last (the dates of its first and last step), and the --section file holds window means computed on the device
@@ -60,6 +65,11 @@ def windowMeans(x, bounds):
             acc = acc + x[t]
         out[w] = acc / (bounds[w + 1] - bounds[w])
     return out
+
+
+def classLabels(labels, bounds):
+    """column headings of a class series, transect-major: label[b_j–b_{j+1})"""
+    return [f'{lab}[{b0:g}–{b1:g})' for lab in labels for b0, b1 in zip(bounds[:-1], bounds[1:])]
 
 
 def writeSection(path, fld, layers, units, windows=None):
@@ -127,16 +137,26 @@ def main(argv=None):
                      help='flux per layer of model levels: level boundaries "0,10,35,75"')
     lay.add_argument('--depthLayers', type=parseList, default=None,
                      help='flux per depth range: depths in metres "0,200,1000,6000", snapped to level interfaces')
+    lay.add_argument('--classField', default=None,
+                     help='flux per class of a T-grid variable: NAME or NAME:FILE (default file: the T file)')
+    ap.add_argument('--classBounds', type=parseList, default=None,
+                    help='class bounds of --classField, ascending, -inf/inf allowed: --classBounds=-2,0,4,10,inf')
     ap.add_argument('--section', default='',
                     help='write the transport section (flux per cell crossing and layer) to this NetCDF file')
     ap.add_argument('--timeMean', type=parseTimeMean, default=None,
                     help='average over windows of N steps, or per calendar month / year: N|month|year')
     a = ap.parse_args(argv)
+    if (a.classField is None) != (a.classBounds is None):
+        ap.error('--classField and --classBounds go together')
     pts, names = parseTransects(a.lonLatPoints, a.iFiles)
     print(f'target points:\n {pts}')
     fld = Field(a.tFile, a.uFile, a.vFile, pts, a.sverdrup, meshFile=a.meshFile or None)
     layers = fld.levelsForDepths(a.depthLayers) if a.depthLayers is not None else a.layers
-    series = fld.fluxSeries(layers=layers)
+    if a.classField is not None:
+        var, _, cfile = a.classField.partition(':')
+        series = fld.fluxClasses(var, a.classBounds, file=cfile or None)
+    else:
+        series = fld.fluxSeries(layers=layers)
     timeVals = [fld.timeObj.getTimeAsDate(i) for i in range(fld.nt)]
     windows = None
     if a.timeMean is not None:
@@ -150,6 +170,9 @@ def main(argv=None):
         iface = fld.layerInterfaces()
         labels = [f'{lab}[{iface[k0]:g}-{iface[k1]:g} m]' for lab in labels for k0, k1 in zip(layers[:-1], layers[1:])]
         rows = numpy.asarray(series).transpose(0, 2, 1).reshape(len(series), -1)   # (time, transect-major layers)
+    elif a.classField is not None:
+        labels = classLabels(labels, a.classBounds)
+        rows = numpy.asarray(series).transpose(0, 2, 1).reshape(len(series), -1)   # (time, transect-major classes)
     print('time,' + ','.join(labels) + f'   [{units}]')
     for t, row in zip(timeVals, rows):
         print(f'{t},' + ','.join(f'{x:.15g}' for x in row))
@@ -157,7 +180,7 @@ def main(argv=None):
         nsub = writeSection(a.section, fld, layers, units, windows)
         print(f'section: {nsub} crossings written to {a.section}')
     if a.output:
-        with open(a.output, 'w') as f:
+        with open(a.output, 'w', encoding='utf-8') as f:
             f.write('time,' + ','.join(labels) + '\n')
             for t, row in zip(timeVals, rows):
                 f.write(f'{t},' + ','.join(repr(float(x)) for x in row) + '\n')

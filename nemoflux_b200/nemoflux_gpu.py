@@ -389,6 +389,64 @@ class PolylineIntegral(object):
         del keep
         return sums
 
+    def fluxClasses(self, u, v, thickness, arc1, arc2, cfield, bounds, cfill=float('nan'), sverdrup=False,
+                    fill=float('nan'), e3u=None, e3v=None, chunk_steps=0):
+        """class transport: the flux across every transect binned by a T-grid field (temperature, salinity, density...)
+        -> (nt, K, M) float64: [t, j, m] is transect m's flux at step t carried by the levels of its crossings whose
+        class value lies in [b_j, b_{j+1}).
+
+        Arguments as fluxSection (CUDA tensors on the current stream, or host arrays through the chunk pipeline), plus:
+        cfield, the class field at the T points, with the dtype, byte order and plane layout of uo/vo, (1 or nt, nz,
+        ...) (a (nz, ny, nx) field is time-invariant); cfill its missing-value marker (compared in the storage type;
+        NaN = none); bounds, K + 1 strictly ascending class bounds (1 <= K <= 96, +-inf allowed, no NaN).
+
+        Every level k of crossing s adds fluxSection(layers=range(nz + 1))[t, k, s] to the class of
+        c = cfield[t or 0, k, cell(s)]; NaN, cfill, c < b0 and c >= bK count nowhere.  The sum order is fixed (per
+        crossing ascending levels, 32-crossing tiles by a fixed tree, tiles in order): the bits depend only on the
+        inputs, whatever chunk_steps, the byte order or the side of the inputs."""
+        torch = _torch()
+        b = numpy.ascontiguousarray(_to_numpy(bounds), numpy.float64).reshape(-1)
+        if b.size < 2:
+            raise ValueError(f'bounds must hold at least 2 class bounds, got {b.size}')
+        m = self.getNumberOfTransects()
+        nsub = self.getNumberOfSubsegments()
+        if isinstance(u, torch.Tensor) and u.is_cuda:
+            u, v, nt, nz, ncell, ld = self._device_inputs(u, v, thickness, arc1, arc2, e3u, e3v)
+            use_e3 = e3u is not None or e3v is not None
+            cfield, c_nt = _class_field_device(cfield, u, nt, nz, ncell, ld)
+            out = torch.zeros((nt, b.size - 1, m), dtype=torch.float64, device=u.device)
+            if nt == 0 or nsub == 0:        # nothing to compute: no launch (empty tensors have no device address)
+                return out
+            e3_nt = _check_e3(e3u, e3v, u, nt, nz, ncell, ld) if use_e3 else 0
+            ptr = lambda t: _t_ptr(t) if t is not None else None   # noqa: E731
+            with torch.cuda.device(u.device):
+                _lib.call('nfx_flux_classes', ctypes.byref(self._h), _t_ptr(u), _t_ptr(v), ptr(e3u), ptr(e3v),
+                          _dtype_code(str(u.dtype)), e3_nt, None if use_e3 else _t_ptr(thickness), _t_ptr(arc1),
+                          _t_ptr(arc2), nt, nz, ld, _t_ptr(cfield), c_nt, float(cfill), b.size - 1, _np_ptr(b),
+                          int(bool(sverdrup)), float(fill), _t_ptr(out), _stream_ptr())
+            return out
+        keep = (u, v, e3u, e3v)  # keep pinned tensors alive while numpy views are in use
+        h = _host_inputs(u, v, thickness, arc1, arc2, e3u, e3v)
+        c = numpy.asarray(cfield.numpy() if isinstance(cfield, torch.Tensor) else cfield)
+        if c.dtype != h.u.dtype:
+            raise ValueError(f'cfield must have the dtype and byte order of uo ({h.u.dtype}), got {c.dtype}')
+        nz, ny, nx = h.u.shape[1:]
+        if c.ndim == 3 and c.shape == (nz, ny, nx):
+            c = c[None]
+        if c.ndim == 3:
+            c = c.reshape(c.shape[0], c.shape[1], ny, nx) if c.shape[2] == ny * nx else c
+        if c.ndim != 4 or c.shape[1:] != (nz, ny, nx) or c.shape[0] not in (1, h.nt):
+            raise ValueError(f'cfield must be (1 or nt, nz, ny, nx) or (nz, ny, nx), got shape {c.shape}')
+        c = numpy.ascontiguousarray(c)
+        res = numpy.zeros((h.nt, b.size - 1, m), numpy.float64)
+        pu, pv, e3_nt, on_device = h.e3 if h.e3 is not None else (None, None, 0, False)
+        _lib.call('nfx_flux_classes_host', ctypes.byref(self._h), _np_ptr(h.u), _np_ptr(h.v), pu, pv, h.code, e3_nt,
+                  int(on_device), None if h.th is None else _np_ptr(h.th), _np_ptr(h.a1), _np_ptr(h.a2), h.nt, h.nz,
+                  _np_ptr(c), c.shape[0], float(cfill), b.size - 1, _np_ptr(b), int(bool(sverdrup)), float(fill),
+                  int(chunk_steps), _np_ptr(res))
+        del keep
+        return res
+
     def _section_device_inputs(self, u, v, thickness, arc1, arc2, e3u, e3v, lev):
         """checks of the CUDA inputs of fluxSection / sectionWindowSums -> (u, v, nt, nz, ncell, ld, levels), the
         levels of one layer per level when lev is None"""
@@ -800,11 +858,29 @@ def _check_e3(e3u, e3v, u, nt, nz, ncell, ld):
         if not isinstance(t, torch.Tensor) or not t.is_cuda or t.dtype != u.dtype:
             raise TypeError(f'{name} must be a CUDA tensor with the dtype of uo/vo')
         ent, enz, encell, eld = _plane_layout(t, name)
-        if (enz, encell) != (nz, ncell) or ent not in (1, nt) or (eld != ld and enz > 1):
+        # the kernels step levels by ld and time steps by nz * ld, the layout of uo/vo
+        if (enz, encell) != (nz, ncell) or ent not in (1, nt) or (eld != ld and enz > 1) or \
+                (ent > 1 and t.stride(0) != nz * ld):
             raise ValueError(f'{name} must be (1 or nt, nz, cells) with the plane layout of uo/vo')
     if e3u.shape[0] != e3v.shape[0]:
         raise ValueError('e3u and e3v must hold the same number of time steps')
     return int(e3u.shape[0])
+
+
+def _class_field_device(c, u, nt, nz, ncell, ld):
+    """the class field of fluxClasses on the device: a CUDA tensor with the dtype and plane layout of uo, (1 or nt, nz,
+    ny, nx), (1 or nt, nz, cells) or (nz, ny, nx) -> (c with a time axis, its number of time steps)"""
+    torch = _torch()
+    if not isinstance(c, torch.Tensor) or not c.is_cuda or c.dtype != u.dtype:
+        raise TypeError('cfield must be a CUDA tensor with the dtype of uo/vo')
+    if c.dim() == 3 and c.shape[0] == nz and c.shape[1] * c.shape[2] == ncell and c.shape[2] != ncell:
+        c = c.unsqueeze(0)                                  # (z, y, x): time-invariant
+    cnt, cnz, cncell, cld = _plane_layout(c, 'cfield')
+    # the kernel steps levels by ld and time steps by nz * ld, the layout of uo/vo
+    if (cnz, cncell) != (nz, ncell) or cnt not in (1, nt) or (cld != ld and cnz > 1) or \
+            (cnt > 1 and c.stride(0) != nz * ld):
+        raise ValueError('cfield must be (1 or nt, nz, cells) with the plane layout of uo/vo')
+    return c, int(cnt)
 
 
 def _require_cuda(t, dtype, name):
