@@ -265,6 +265,34 @@ int nfx_flux_classes(nfx_pli** self, const void* u, const void* v, const void* e
                      int e3_nt, const double* thickness, const double* arc1, const double* arc2, int nt, int nz,
                      int64_t ld, const void* cfield, int c_nt, double cfill, int nclasses, const double* class_bounds,
                      int sverdrup, double fill, double* classes, void* stream);
+/* Tracer transport (extension): heat, salt, freshwater... carried across every transect, per layer of model levels.
+ * Arguments as nfx_flux_section, plus the tracer (device, tr_nt x nz planes of ld values at the T points, the dtype of
+ * u, v; tr_nt = 1: time-invariant, or nt), its missing-value marker tfill (NaN = none; compared in the storage type, as
+ * fill; NaN is always missing) and a reference value ref.  Every edge is one C-grid face between two T cells: E eU[c]
+ * (c, east(c)), W eU[west(c)] (west(c), c), N eV[c] (c, north(c); none in the top row), S eV[south(c)] (south(c), c);
+ * east / west wrap x-periodically.  At level k the face value is
+ *   q = 0.5 * (tau_a + tau_b) - ref (both sides present), tau_a - ref (one side present), 0 (neither)
+ * and per crossing, layer and edge A_e = sum over the layer's levels in ascending order from +0 of (d_k * u_e,k) * q_e,k
+ * (d_k: thickness or e3u/e3v; u with NaN and `fill` as 0).  The crossing's value is nfx_flux_section's operations on
+ * the 4 sums A_e (arcs, sverdrup, the sign of eV, the weights in edge order); every operation is rounded on its own, in
+ * double.  With tau == 1 and ref == 0 it is nfx_flux_section's value bit for bit.
+ *   section device (nt, nlayers, nsub) or NULL: that value;
+ *   series  device (nt, nlayers, M) or NULL: the crossings of every transect in tiles of 32 in emission order, each
+ *           folded by a fixed shuffle tree (lane l + lane l + o, o = 16, 8, 4, 2, 1), the tiles in ascending order
+ *           from +0 (the sum order of nfx_flux_classes).
+ * One of series, section may be NULL, not both.  The bits depend only on the inputs.  Asynchronous on `stream`, except
+ * that the layering (when it differs from the previous call's) and, on the first call after computeWeights, the
+ * crossing tiles are copied from pageable host memory, which waits for the work already queued on `stream`.  The tiles
+ * and partial sums are scratch of the handle: calls on one handle must not run concurrently on different streams.  A
+ * NULL pointer, tr_nt not in {1, nt}, a bad layering, or transects computed without nfx_grid_set_cgrid_shape return
+ * NFX_E_INVALID before anything is launched; nt == 0 or no crossing launches nothing and leaves the outputs as they
+ * are.  Units: tracer units x flux units (heat in W: rho0 * cp x the result with metre metrics; freshwater:
+ * -1 / S_ref x the result with ref = S_ref). */
+int nfx_flux_tracer(nfx_pli** self, const void* u, const void* v, const void* e3u, const void* e3v, int dtype,
+                    int e3_nt, const double* thickness, const double* arc1, const double* arc2, int nt, int nz,
+                    int64_t ld, const void* tracer, int tr_nt, double tfill, double ref, int nlayers,
+                    const int* layer_levels, int sverdrup, double fill, double* series, double* section,
+                    void* stream);
 /* The device-path series calls (nfx_flux_series*, nfx_flux_series_range*) are asynchronous on `stream`.  Their fused
  * pass spins on per-batch counters with a bound; a pass that ever overflowed it aborts and leaves NaN in `series`.
  * nfx_pli_series_status synchronises `stream` and reports that: returns 0 with *status = 0 when every pass launched
@@ -371,6 +399,15 @@ int nfx_flux_classes_host(nfx_pli** self, const void* u, const void* v, const vo
                           int dtype_flags, int e3_nt, int e3_on_device, const double* thickness, const double* arc1,
                           const double* arc2, int nt, int nz, const void* cfield, int c_nt, double cfill, int nclasses,
                           const double* class_bounds, int sverdrup, double fill, int chunk_steps, double* classes);
+/* nfx_flux_tracer from HOST buffers: arguments as nfx_flux_section_host plus tracer (host, tr_nt x nz x ncell in the
+ * dtype and byte order of u, v: streamed with them when tr_nt == nt, uploaded once when tr_nt == 1), tfill, ref;
+ * series host (nt, nlayers, M) and / or section host (nt, nlayers, nsub), one of them may be NULL.  The bits do not
+ * depend on chunk_steps or the byte order and are those of nfx_flux_tracer. */
+int nfx_flux_tracer_host(nfx_pli** self, const void* u, const void* v, const void* e3u, const void* e3v,
+                         int dtype_flags, int e3_nt, int e3_on_device, const double* thickness, const double* arc1,
+                         const double* arc2, int nt, int nz, const void* tracer, int tr_nt, double tfill, double ref,
+                         int nlayers, const int* layer_levels, int sverdrup, double fill, int chunk_steps,
+                         double* series, double* section);
 
 #ifdef __cplusplus
 }

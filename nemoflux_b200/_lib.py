@@ -114,6 +114,10 @@ SIGNATURES = {
                          c_int, c_dbl, c_int, c_vp, c_int, c_dbl, c_vp, c_vp],
     'nfx_flux_classes_host': [P(c_vp), c_vp, c_vp, c_vp, c_vp, c_int, c_int, c_int, c_vp, c_vp, c_vp, c_int, c_int,
                               c_vp, c_int, c_dbl, c_int, c_vp, c_int, c_dbl, c_int, c_vp],
+    'nfx_flux_tracer': [P(c_vp), c_vp, c_vp, c_vp, c_vp, c_int, c_int, c_vp, c_vp, c_vp, c_int, c_int, c_i64, c_vp,
+                        c_int, c_dbl, c_dbl, c_int, c_vp, c_int, c_dbl, c_vp, c_vp, c_vp],
+    'nfx_flux_tracer_host': [P(c_vp), c_vp, c_vp, c_vp, c_vp, c_int, c_int, c_int, c_vp, c_vp, c_vp, c_int, c_int,
+                             c_vp, c_int, c_dbl, c_dbl, c_int, c_vp, c_int, c_dbl, c_int, c_vp, c_vp],
 }
 
 _LIB = None

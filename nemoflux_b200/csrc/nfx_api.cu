@@ -939,15 +939,22 @@ static void class_tiles(PliDev& p, cudaStream_t s) {
     p.class_ntiles = ntiles;
 }
 
-// tiles, bounds and the partial sums of a class call of up to nt steps (the partial sums: at most 64 MB, or one step)
-static int prepare_classes(PliDev& p, int nclasses, const double* bounds, int nt, cudaStream_t s) {
+// the warp tiles and the partial sums of `per_tile` values per (step, tile) of a call of up to nt steps (the partial
+// sums: at most 64 MB, or one step); returns the steps per batch
+static int tile_partials(PliDev& p, int per_tile, int nt, cudaStream_t s) {
     class_tiles(p, s);
+    const int64_t per_step = std::max<int64_t>(1, p.class_ntiles * per_tile);
+    const int steps = (int)std::max<int64_t>(1, std::min<int64_t>(nt, ((int64_t)64 << 20) / 8 / per_step));
+    p.class_partial.ensure((size_t)steps * per_step);
+    return steps;
+}
+
+// tiles, bounds and the partial sums of a class call of up to nt steps
+static int prepare_classes(PliDev& p, int nclasses, const double* bounds, int nt, cudaStream_t s) {
+    const int steps = tile_partials(p, nclasses, nt, s);
     p.class_bounds.ensure((size_t)nclasses + 1);
     NFX_CUDA(cudaMemcpyAsync(p.class_bounds.p, bounds, sizeof(double) * ((size_t)nclasses + 1), cudaMemcpyHostToDevice,
                              s));
-    const int64_t per_step = std::max<int64_t>(1, p.class_ntiles * nclasses);
-    const int steps = (int)std::max<int64_t>(1, std::min<int64_t>(nt, ((int64_t)64 << 20) / 8 / per_step));
-    p.class_partial.ensure((size_t)steps * per_step);
     return steps;
 }
 
@@ -985,6 +992,52 @@ int nfx_flux_classes(nfx_pli** self, const void* u, const void* v, const void* e
         const int steps = prepare_classes(p, nclasses, class_bounds, nt, s);
         run_classes(p, u, v, dtype, thickness, e3u, e3v, e3u && e3_nt != 1 ? (int64_t)nz * ld : 0, arc1, arc2, cfield,
                     c_nt != 1 ? (int64_t)nz * ld : 0, cfill, nclasses, ld, nt, nz, sverdrup, fill, steps, classes, s);
+    });
+}
+
+static void run_tracer(PliDev& p, const void* u, const void* v, int dtype, const double* thickness, const void* e3u,
+                       const void* e3v, int64_t e3_tstride, const double* arc1, const double* arc2, const void* tracer,
+                       int64_t tr_tstride, double tfill, double ref, int64_t ld, int nt, int nz, int nlayers,
+                       const int* levels, int sverdrup, double fill, int partial_steps, double* series, double* section,
+                       cudaStream_t s) {
+    const Csr& c = section_csr(p);
+    flux_tracer(u, v, dtype, thickness, e3u, e3v, e3_tstride, arc1, arc2, c.idx.p, c.w, p.cell.p, tracer, tr_tstride,
+                tfill, ref, p.class_tiles.p, p.class_ntiles, p.class_tr_tiles.p, p.ntransects, p.nsub, p.grid->ncell,
+                p.grid->nx, ld, nt, nz, nlayers, levels, sverdrup, fill, p.class_partial.p, partial_steps, series,
+                section, s);
+}
+
+int nfx_flux_tracer(nfx_pli** self, const void* u, const void* v, const void* e3u, const void* e3v, int dtype,
+                    int e3_nt, const double* thickness, const double* arc1, const double* arc2, int nt, int nz,
+                    int64_t ld, const void* tracer, int tr_nt, double tfill, double ref, int nlayers,
+                    const int* layer_levels, int sverdrup, double fill, double* series, double* section,
+                    void* stream) {
+    return guarded([&] {
+        NFX_REQUIRE(self && *self, "NULL handle");
+        PliDev& p = (*self)->d;
+        NFX_REQUIRE(p.grid, "setGrid was not called");
+        DeviceGuard g(p.grid->device);
+        NFX_REQUIRE(u && v && arc1 && arc2 && tracer && (series || section), "NULL pointer");
+        NFX_REQUIRE((e3u == nullptr) == (e3v == nullptr), "e3u and e3v go together");
+        NFX_REQUIRE((thickness != nullptr) != (e3u != nullptr), "needs exactly one of thickness and (e3u, e3v)");
+        NFX_REQUIRE(nt >= 0 && nz > 0 && nz <= 3000, "bad sizes");
+        NFX_REQUIRE(dtype == NFX_F64 || dtype == NFX_F32, "dtype must be NFX_F64 or NFX_F32");
+        NFX_REQUIRE(ld >= p.grid->ncell, "ld must be >= the number of cells");
+        NFX_REQUIRE(!e3u || e3_nt == 1 || e3_nt == nt, "e3u/e3v must hold 1 (time-invariant) or nt time steps");
+        NFX_REQUIRE(tr_nt == 1 || tr_nt == nt, "the tracer must hold 1 (time-invariant) or nt time steps");
+        check_layer_levels(nz, nlayers, layer_levels);
+        section_csr(p);
+        if (nt == 0 || p.nsub == 0) return;
+        const cudaStream_t s = (cudaStream_t)stream;
+        int steps = 1;                      // the partial sums are scratch of the series only
+        if (series)
+            steps = tile_partials(p, nlayers, nt, s);   // builds the tiles too
+        else
+            class_tiles(p, s);
+        const int* levels = device_levels(p, nz, nlayers, layer_levels, s);
+        run_tracer(p, u, v, dtype, thickness, e3u, e3v, e3u && e3_nt != 1 ? (int64_t)nz * ld : 0, arc1, arc2, tracer,
+                   tr_nt != 1 ? (int64_t)nz * ld : 0, tfill, ref, ld, nt, nz, nlayers, levels, sverdrup, fill, steps,
+                   series, section, s);
     });
 }
 
@@ -1181,7 +1234,7 @@ struct HostChunk {
     int t0;                    // first time step of the chunk
     int n;
     int slot;                  // staging slot of the chunk (0 or 1)
-    const void* cf;            // class field at the chunk's first step (nullptr without one)
+    const void* cf;            // auxiliary T-grid field (class field, tracer) at the chunk's first step, or nullptr
     int64_t c_tstride;         // its step stride (0: time-invariant)
 };
 
@@ -1510,6 +1563,49 @@ struct ClassPass : PerStepPass {
     }
 };
 
+// tracer transport: one tracer pass per chunk, series (nt, nlayers, M) and / or section (nt, nlayers, nsub), both
+// staged whole on the device (the series first) and copied back at the end
+struct TracerPass : HostPass {
+    int sverdrup = 0, nlayers = 1, partial_steps = 1, nt = 0;
+    double fill = 0.0, tfill = 0.0, ref = 0.0;
+    const int* layer_levels = nullptr;
+    const int* levels = nullptr;
+    double* series = nullptr;       // host outputs (either may be NULL)
+    double* section = nullptr;
+    int64_t n_series = 0, n_section = 0;   // values per step
+    bool begin(PliDev& p, int, int, int nz) override {
+        check_layer_levels(nz, nlayers, layer_levels);
+        section_csr(p);
+        n_series = series ? (int64_t)nlayers * p.ntransects : 0;
+        n_section = section ? (int64_t)nlayers * p.nsub : 0;
+        return p.nsub != 0;
+    }
+    void prepare(PliDev& p, int, int nt_, int nz, int chunk_steps, double*, cudaStream_t ks) override {
+        nt = nt_;
+        p.stage_series.ensure((size_t)nt * (n_series + n_section));
+        if (series)
+            partial_steps = tile_partials(p, nlayers, chunk_steps, ks);   // builds the tiles too
+        else
+            class_tiles(p, ks);
+        levels = device_levels(p, nz, nlayers, layer_levels, ks);
+    }
+    void chunk(PliDev& p, int dtype, int nz, const HostChunk& k, cudaStream_t ks) override {
+        const int64_t ncell = p.grid->ncell;
+        double* d_series = series ? p.stage_series.p + (size_t)k.t0 * n_series : nullptr;
+        double* d_section = section ? p.stage_series.p + (size_t)nt * n_series + (size_t)k.t0 * n_section : nullptr;
+        run_tracer(p, k.u, k.v, dtype, k.thickness, k.e3u, k.e3v, k.e3_tstride, k.arc1, k.arc2, k.cf, k.c_tstride,
+                   tfill, ref, ncell, k.n, nz, nlayers, levels, sverdrup, fill, partial_steps, d_series, d_section, ks);
+    }
+    void finish(PliDev& p, double*, cudaStream_t ks) override {
+        if (series)
+            NFX_CUDA(cudaMemcpyAsync(series, p.stage_series.p, sizeof(double) * (size_t)nt * n_series,
+                                     cudaMemcpyDeviceToHost, ks));
+        if (section)
+            NFX_CUDA(cudaMemcpyAsync(section, p.stage_series.p + (size_t)nt * n_series,
+                                     sizeof(double) * (size_t)nt * n_section, cudaMemcpyDeviceToHost, ks));
+    }
+};
+
 int nfx_flux_series_host(nfx_pli** self, const void* u, const void* v, int dtype_flags, const double* thickness,
                          const double* arc1, const double* arc2, int nt, int nz, int sverdrup, double fill, int order,
                          int chunk_steps, double* series) {
@@ -1617,6 +1713,31 @@ int nfx_flux_classes_host(nfx_pli** self, const void* u, const void* v, const vo
         pass.bounds = class_bounds;
         host_pipeline(self, u, v, dtype_flags, thickness, e3u, e3v, e3_nt, e3_on_device, arc1, arc2, nt, nz,
                       chunk_steps, classes, pass, cfield, c_nt);
+    });
+}
+
+int nfx_flux_tracer_host(nfx_pli** self, const void* u, const void* v, const void* e3u, const void* e3v,
+                         int dtype_flags, int e3_nt, int e3_on_device, const double* thickness, const double* arc1,
+                         const double* arc2, int nt, int nz, const void* tracer, int tr_nt, double tfill, double ref,
+                         int nlayers, const int* layer_levels, int sverdrup, double fill, int chunk_steps,
+                         double* series, double* section) {
+    return guarded([&] {
+        NFX_REQUIRE((thickness != nullptr) != (e3u != nullptr || e3v != nullptr),
+                    "needs exactly one of thickness and (e3u, e3v)");
+        NFX_REQUIRE(tracer && (series || section), "NULL pointer");
+        NFX_REQUIRE(nz <= 3000, "bad sizes");
+        NFX_REQUIRE(tr_nt == 1 || tr_nt == nt, "the tracer must hold 1 (time-invariant) or nt time steps");
+        TracerPass pass;
+        pass.sverdrup = sverdrup;
+        pass.fill = fill;
+        pass.tfill = tfill;
+        pass.ref = ref;
+        pass.nlayers = nlayers;
+        pass.layer_levels = layer_levels;
+        pass.series = series;
+        pass.section = section;
+        host_pipeline(self, u, v, dtype_flags, thickness, e3u, e3v, e3_nt, e3_on_device, arc1, arc2, nt, nz,
+                      chunk_steps, series ? series : section, pass, tracer, tr_nt);
     });
 }
 

@@ -312,5 +312,16 @@ void flux_classes(const void* u, const void* v, int dtype, const double* thickne
                   const int64_t* tile_start, int64_t ntiles, const int64_t* tr_tiles, int ntransects, int64_t ncell,
                   int64_t ld, int nt, int nz, int sverdrup, double fill, double* partial, int partial_steps,
                   double* classes, cudaStream_t s);
+// tracer transport (nfx_section.cu): per layer (levels: device, nlayers + 1) the section flux of every crossing with
+// each edge's level terms weighted by the tracer at its C-grid face (tracer (1 or nt, nz, ld) of the dtype of u, v;
+// tr_tstride 0 or nz * ld; the grid nx cells wide).  section (nt, nlayers, nsub) and / or series (nt, nlayers, M), the
+// crossings folded over the warp tiles of flux_classes; partial: scratch of partial_steps * ntiles * nlayers doubles
+// (with series), the steps are run in batches of at most partial_steps.
+void flux_tracer(const void* u, const void* v, int dtype, const double* thickness, const void* e3u, const void* e3v,
+                 int64_t e3_tstride, const double* arc1, const double* arc2, const int32_t* idx, const double* w,
+                 const int32_t* cell, const void* tracer, int64_t tr_tstride, double tfill, double ref,
+                 const int64_t* tile_start, int64_t ntiles, const int64_t* tr_tiles, int ntransects, int64_t nsub,
+                 int64_t ncell, int nx, int64_t ld, int nt, int nz, int nlayers, const int* levels, int sverdrup,
+                 double fill, double* partial, int partial_steps, double* series, double* section, cudaStream_t s);
 
 }  // namespace nfx

@@ -322,6 +322,165 @@ __global__ void k_reduce_class_tiles(const double* __restrict__ partial, int nt,
     classes[((t0 + t) * K + j) * ntransects + m] = a;
 }
 
+// Tracer transport: the flux of every crossing weighted by a tracer tau (temperature, salinity...) taken at the C-grid
+// face of each of its edges.  Face of edge e of crossing s in cell c (flux_index order S, E, N, W):
+//   S: eV[south(c)], the T cells south(c) and c      E: eU[c], c and east(c)
+//   N: eV[c], c and north(c) (none in the top row)   W: eU[west(c)], west(c) and c        (east / west x-periodic)
+// At level k the face value q is 0.5 * (tau_a + tau_b) - ref with both sides present, tau_a - ref with one side, 0 with
+// none (missing: NaN or the marker tfill, compared in the storage type).  Per layer and edge the thread sums
+// A_e += (d_k * u_e,k) * q_e,k over the layer's levels in ascending order from +0 (d_k: dz, or e3u / e3v; u cleaned as
+// in section_level) and turns the 4 sums into the crossing's value with section_value.  With tau == 1 and ref == 0,
+// q == 1 and every term is the section's: the value is fluxSection's bit for bit.
+// One thread per (time step, crossing) in the warp tiles of k_flux_classes; the lanes past the end of a tile run the
+// tile's first crossing and count +0, so every lane reaches the shuffles.  Per level the thread gathers its 4 columns
+// (section_load) and the tracer at 5 cells: c is shared by all 4 faces.  At a layer boundary it forms the value once,
+// stores it to `section` (streaming) and / or folds the tile with the shuffle tree of k_flux_classes into
+// partial[(step - t0, tile, layer)], which k_reduce_class_tiles adds up per transect (K = nlayers).
+// levels in flight (9 loads per level, 13 with E3) and CTAs per SM: 122-128 registers, no spills; every shape with 3
+// CTAs per SM (80 registers) spills, even with one level in flight (profiles/r8_tracer_ptxas.md)
+template <typename T, bool E3>
+struct TracerShape {
+    static constexpr int unroll = E3 ? 1 : 3;
+    static constexpr int ctas = 2;
+};
+
+// the face value q of a face between the T cells a and b (has_b false: no cell b)
+template <typename T>
+__device__ __forceinline__ double face_tracer(T a, T b, bool has_b, T tfill, int has_tfill, double ref) {
+    const bool pa = !(a != a) && !(has_tfill && a == tfill);
+    const bool pb = has_b && !(b != b) && !(has_tfill && b == tfill);
+    if (pa && pb) return __dsub_rn(__dmul_rn(0.5, __dadd_rn((double)a, (double)b)), ref);
+    if (pa) return __dsub_rn((double)a, ref);
+    if (pb) return __dsub_rn((double)b, ref);
+    return 0.0;
+}
+
+template <typename T, bool E3>
+__global__ void __launch_bounds__(kSectionBlock, TracerShape<T, E3>::ctas)
+k_flux_tracer(const T* __restrict__ u, const T* __restrict__ v, const T* __restrict__ e3u, const T* __restrict__ e3v,
+              int64_t e3_tstride, const double* __restrict__ dz, const double* __restrict__ arc1,
+              const double* __restrict__ arc2, const int32_t* __restrict__ idx, const double* __restrict__ w,
+              const int32_t* __restrict__ cell, const T* __restrict__ tr, int64_t tr_tstride, T tfill, int has_tfill,
+              double ref, const int64_t* __restrict__ tile_start, int64_t ntiles, int64_t nsub, int64_t ncell, int nx,
+              int64_t ld, int nz, int nlayers, const int* __restrict__ levels, double scale, int use_scale, T fill,
+              int has_fill, int64_t t0, double* __restrict__ section, double* __restrict__ partial) {
+    constexpr int UNROLL = TracerShape<T, E3>::unroll;
+    extern __shared__ double s_dz[];                        // [nz] dz (without E3), then [nlayers + 1] boundaries
+    int* s_lev = reinterpret_cast<int*>(s_dz + (E3 ? 0 : nz));
+    if constexpr (!E3)
+        for (int k = threadIdx.x; k < nz; k += kSectionBlock) s_dz[k] = dz[k];
+    for (int i = threadIdx.x; i <= nlayers; i += kSectionBlock)
+        s_lev[i] = levels ? levels[i] : (i == 0 ? 0 : nz);  // levels == nullptr: one layer, the whole column
+    __syncthreads();
+    const int64_t tile = (int64_t)blockIdx.x * (kSectionBlock / 32) + threadIdx.x / 32;
+    if (tile >= ntiles) return;                             // the whole warp
+    const int lane = threadIdx.x & 31;
+    const int64_t t = t0 + blockIdx.y;
+    const int64_t s0 = tile_start[tile] + lane;
+    const bool present = s0 < tile_start[tile + 1];
+    const int64_t s = present ? s0 : tile_start[tile];
+    const T* pc[4];
+    const T* pe[4];
+    double arc[4], wt[4], acc[4] = {0.0, 0.0, 0.0, 0.0};
+    bool live[4];
+    section_edges<T, E3>(u, v, e3u, e3v, arc1, arc2, idx, w, s, ncell, t * nz * ld, t * e3_tstride, pc, pe, arc, wt,
+                         live);
+    // the tracer at c and at its east, west, north and south neighbours (no north cell in the top row, no south cell in
+    // row 0: c itself, a harmless address; the S edge of row 0 is not live)
+    const int64_t c = cell[s];
+    const int i = (int)(c % nx);
+    const bool has_n = c + nx < ncell;
+    const T* pt = tr + t * tr_tstride + c;
+    const int64_t o_e = i + 1 < nx ? 1 : 1 - nx, o_w = i >= 1 ? -1 : nx - 1, o_n = has_n ? nx : 0,
+                  o_s = c >= nx ? -(int64_t)nx : 0;
+    double* sec = section ? section + (t * nlayers) * nsub + s : nullptr;
+    double* part = partial ? partial + ((int64_t)blockIdx.y * ntiles + tile) * nlayers : nullptr;
+    int layer = 0, next = s_lev[1];
+    const int kend = s_lev[nlayers];
+    int k = s_lev[0];
+    // level kk into the 4 tracer-weighted column sums; after the last level of a layer: the value, stored and / or
+    // folded over the tile (the layering is the same for every thread: the branch does not diverge)
+    auto step = [&](int kk, const T (&x)[4], const T (&ex)[4], const T (&ta)[5]) {
+        const double q[4] = {face_tracer<T>(ta[4], ta[0], true, tfill, has_tfill, ref),
+                             face_tracer<T>(ta[0], ta[1], true, tfill, has_tfill, ref),
+                             face_tracer<T>(ta[0], ta[3], has_n, tfill, has_tfill, ref),
+                             face_tracer<T>(ta[2], ta[0], true, tfill, has_tfill, ref)};
+        const double d = E3 ? 0.0 : s_dz[kk];
+#pragma unroll
+        for (int e = 0; e < 4; ++e) {
+            const double de = E3 ? clean<T>(ex[e], fill, has_fill) : d;
+            acc[e] = __dadd_rn(acc[e], __dmul_rn(__dmul_rn(de, clean<T>(x[e], fill, has_fill)), q[e]));
+        }
+        if (kk + 1 == next) {
+            const double r = section_value(acc, arc, wt, live, scale, use_scale);
+#pragma unroll
+            for (int e = 0; e < 4; ++e) acc[e] = 0.0;
+            if (sec && present) __stcs(sec + (int64_t)layer * nsub, r);
+            if (part) {
+                double a = present ? r : 0.0;
+#pragma unroll
+                for (int o = 16; o > 0; o >>= 1) a = __dadd_rn(a, __shfl_down_sync(0xffffffffu, a, o));
+                if (lane == 0) part[layer] = a;
+            }
+            ++layer;
+            next = layer < nlayers ? s_lev[layer + 1] : -1;
+        }
+    };
+    // the 5 tracer values of level kk: c, east, west, north, south
+    auto load_tracer = [&](int kk, T (&ta)[5]) {
+        const T* p = pt + (int64_t)kk * ld;
+        ta[0] = __ldg(p);
+        ta[1] = __ldg(p + o_e);
+        ta[2] = __ldg(p + o_w);
+        ta[3] = __ldg(p + o_n);
+        ta[4] = __ldg(p + o_s);
+    };
+    for (; k + UNROLL <= kend; k += UNROLL) {
+        T x[UNROLL][4], ex[UNROLL][4], ta[UNROLL][5];
+#pragma unroll
+        for (int q = 0; q < UNROLL; ++q) {
+            section_load<T, E3>(pc, pe, (int64_t)(k + q) * ld, (int64_t)(k + q) * ld, x[q], ex[q]);
+            load_tracer(k + q, ta[q]);
+        }
+#pragma unroll
+        for (int q = 0; q < UNROLL; ++q) step(k + q, x[q], ex[q], ta[q]);
+    }
+    for (; k < kend; ++k) {
+        T x[4], ex[4], ta[5];
+        section_load<T, E3>(pc, pe, (int64_t)k * ld, (int64_t)k * ld, x, ex);
+        load_tracer(k, ta);
+        step(k, x, ex, ta);
+    }
+}
+
+template <typename T, bool E3>
+void launch_tracer(const void* u, const void* v, const void* e3u, const void* e3v, int64_t e3_tstride,
+                   const double* dz, const double* arc1, const double* arc2, const int32_t* idx, const double* w,
+                   const int32_t* cell, const void* tracer, int64_t tr_tstride, double tfill, double ref,
+                   const int64_t* tile_start, int64_t ntiles, const int64_t* tr_tiles, int ntransects, int64_t nsub,
+                   int64_t ncell, int nx, int64_t ld, int nt, int nz, int nlayers, const int* levels, int sverdrup,
+                   double fill, double* partial, int partial_steps, double* series, double* section, cudaStream_t s) {
+    const double scale = 6371000.0 / 1.e6;
+    const size_t smem = (E3 ? 0 : sizeof(double) * nz) + sizeof(int) * (nlayers + 1);
+    const unsigned gx = (unsigned)((ntiles + kSectionBlock / 32 - 1) / (kSectionBlock / 32));
+    const int batch = series ? std::min(partial_steps, 65535) : 65535;
+    for (int t0 = 0; t0 < nt; t0 += batch) {
+        const int n = std::min(batch, nt - t0);
+        k_flux_tracer<T, E3><<<dim3(gx, (unsigned)n), kSectionBlock, smem, s>>>(
+            (const T*)u, (const T*)v, (const T*)e3u, (const T*)e3v, e3_tstride, dz, arc1, arc2, idx, w, cell,
+            (const T*)tracer, tr_tstride, (T)tfill, !(tfill != tfill), ref, tile_start, ntiles, nsub, ncell, nx, ld, nz,
+            nlayers, levels, scale, sverdrup, (T)fill, !(fill != fill), t0, section, series ? partial : nullptr);
+        count_launch();
+        NFX_CUDA(cudaGetLastError());
+        if (!series) continue;
+        const int64_t nr = (int64_t)n * ntransects * nlayers;
+        k_reduce_class_tiles<<<(unsigned)((nr + 255) / 256), 256, 0, s>>>(partial, n, ntiles, nlayers, tr_tiles,
+                                                                         ntransects, t0, series);
+        count_launch();
+        NFX_CUDA(cudaGetLastError());
+    }
+}
+
 template <typename T, bool E3>
 void launch_classes(const void* u, const void* v, const void* e3u, const void* e3v, int64_t e3_tstride,
                     const double* dz, const double* arc1, const double* arc2, const int32_t* idx, const double* w,
@@ -485,6 +644,40 @@ void flux_classes(const void* u, const void* v, int dtype, const double* thickne
             NFX_CLASSES(float, false);
     }
 #undef NFX_CLASSES
+}
+
+void flux_tracer(const void* u, const void* v, int dtype, const double* thickness, const void* e3u, const void* e3v,
+                 int64_t e3_tstride, const double* arc1, const double* arc2, const int32_t* idx, const double* w,
+                 const int32_t* cell, const void* tracer, int64_t tr_tstride, double tfill, double ref,
+                 const int64_t* tile_start, int64_t ntiles, const int64_t* tr_tiles, int ntransects, int64_t nsub,
+                 int64_t ncell, int nx, int64_t ld, int nt, int nz, int nlayers, const int* levels, int sverdrup,
+                 double fill, double* partial, int partial_steps, double* series, double* section, cudaStream_t s) {
+    NFX_REQUIRE(u && v && arc1 && arc2 && idx && w && cell && tracer && tile_start && tr_tiles &&
+                    (series || section) && (!series || partial), "tracer: NULL pointer");
+    NFX_REQUIRE((e3u == nullptr) == (e3v == nullptr) && (thickness != nullptr) != (e3u != nullptr),
+                "tracer: needs exactly one of thickness and (e3u, e3v)");
+    NFX_REQUIRE(nz > 0 && nz <= 3000 && nt >= 0 && ld >= ncell && nx > 0 && ncell % nx == 0 && partial_steps >= 1,
+                "tracer: bad sizes");
+    NFX_REQUIRE(ntiles / (kSectionBlock / 32) < 2147483647ll, "tracer: too many sub-segments");
+    if (nt == 0 || ntiles == 0) return;
+    const bool e3 = e3u != nullptr;
+#define NFX_TRACER(T, E3)                                                                                             \
+    launch_tracer<T, E3>(u, v, e3u, e3v, e3_tstride, thickness, arc1, arc2, idx, w, cell, tracer, tr_tstride, tfill,  \
+                         ref, tile_start, ntiles, tr_tiles, ntransects, nsub, ncell, nx, ld, nt, nz, nlayers, levels, \
+                         sverdrup, fill, partial, partial_steps, series, section, s)
+    if (dtype == NFX_F64) {
+        if (e3)
+            NFX_TRACER(double, true);
+        else
+            NFX_TRACER(double, false);
+    } else {
+        NFX_REQUIRE(dtype == NFX_F32, "tracer: dtype must be NFX_F64 or NFX_F32");
+        if (e3)
+            NFX_TRACER(float, true);
+        else
+            NFX_TRACER(float, false);
+    }
+#undef NFX_TRACER
 }
 
 }  // namespace nfx

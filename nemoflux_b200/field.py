@@ -444,8 +444,39 @@ class Field(object):
         into the classes [b_j, b_{j+1}) of bounds, see PolylineIntegral.fluxClasses.  var is read from `file` (default:
         the T file), (nt, nz, ny, nx) or time-invariant (nz, ny, nx), with its _FillValue, block by block next to uo/vo
         on the pipeline of fluxSeries, and converted to the storage type of uo/vo."""
-        import torch
         b = numpy.asarray(bounds, numpy.float64).reshape(-1)
+        out = numpy.zeros((self.nt, b.size - 1, len(self.plis)))
+
+        def run(t0, m, c, cfill, *args, **kw):
+            out[t0:t0 + m] = _host(self.pli.fluxClasses(*args, cfield=c, bounds=b, cfill=cfill, **kw))
+        self._over_chunks_with(var, file, run, chunk_steps, prefetch, device_decode)
+        return out
+
+    def fluxTracer(self, var, file=None, ref=0.0, layers=None, section=False, chunk_steps=0, prefetch=True,
+                   device_decode=None):
+        """tracer transport: every transect's flux weighted by the T-grid variable `var` (thetao, so...) at the C-grid
+        faces, minus ref, see PolylineIntegral.fluxTracer: (nt, M), or (nt, nlayers, M) with layers (level
+        boundaries, see levelsForDepths); section=True: (nt, nlayers, nsub) per crossing, one layer per level by
+        default.  var is read as fluxClasses reads its class field: from `file` (default: the T file), with its
+        _FillValue, block by block next to uo/vo, converted to the storage type of uo/vo."""
+        if section:
+            nlev = self.nz if layers is None else len(layers) - 1
+            out = numpy.zeros((self.nt, nlev, self.pli.getNumberOfSubsegments()))
+        else:
+            out = numpy.zeros(self._series_shape(layers))
+
+        def run(t0, m, c, tfill, *args, **kw):
+            out[t0:t0 + m] = _host(self.pli.fluxTracer(*args, tracer=c, ref=ref, tfill=tfill, layers=layers,
+                                                       section=section, **kw))
+        self._over_chunks_with(var, file, run, chunk_steps, prefetch, device_decode)
+        return out
+
+    def _over_chunks_with(self, var, file, run, chunk_steps, prefetch, device_decode):
+        """run(t0, m, c, cfill, u, v, thickness, arc1, arc2, sverdrup=, fill=, e3u=, e3v=) over the blocks of
+        _over_chunks, with c the T-grid variable `var` of `file` (default: the T file) next to uo/vo in their storage
+        type and cfill its _FillValue: (nt, nz, ny, nx) read block by block on the reader thread, or (nz, ny, nx) (or
+        one step) converted, and uploaded, once"""
+        import torch
         nc = ncio.open_dataset(file or self.tFile)
         try:
             cv = nc[var]
@@ -458,7 +489,6 @@ class Field(object):
             cfill = self._fill(nc, var)
             fixed = self._slab(nc, var, 0, 1) if steady else None
             once = {}                       # the time-invariant field, converted (and uploaded) once per form
-            out = numpy.zeros((self.nt, b.size - 1, len(self.plis)))
 
             def read(t0, m, dtype):
                 """on the reader thread, next to uo/vo: the block in the storage type and byte order of uo/vo"""
@@ -474,11 +504,10 @@ class Field(object):
                     c = once[key]
                 else:
                     c = aux if on_host else torch.from_numpy(aux).to(u.device).reshape(m, self.nz, -1)
-                out[t0:t0 + m] = _host(self.pli.fluxClasses(u, v, *args, cfield=c, bounds=b, cfill=cfill, **kw))
+                run(t0, m, c, cfill, u, v, *args, **kw)
             self._over_chunks(fn, chunk_steps, prefetch, device_decode, aux=None if steady else read)
         finally:
             nc.close()
-        return out
 
     def _over_chunks(self, fn, chunk_steps, prefetch, device_decode, steps=None, aux=None):
         """fn(t0, m, u, v, thickness, arc1, arc2, sverdrup=, fill=, e3u=, e3v=) over blocks [t0, t0 + m) of the time

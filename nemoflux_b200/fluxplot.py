@@ -2,7 +2,7 @@
 
     python -m nemoflux_b200.fluxplot -t T.nc -u U.nc -v V.nc -i "../data/nz/S*.txt" [-s] [--output series.csv]
         [--layers "0,10,35,75" | --depthLayers "0,200,1000,6000" | --classField NAME[:FILE] --classBounds=b0,b1,...]
-        [--section section.nc] [--timeMean N|month|year]
+        [--section section.nc] [--timeMean N|month|year] [--tracer NAME[:FILE] [--tracerRef R]]
 
 The reference loops ``for itime: fld.update(); for pli: pli.getIntegral(...)`` (fluxplot.py:51-59); here the
 whole (nt, M) series comes from Field.fluxSeries() (K2+K3 over chunks of time steps).  The series is printed
@@ -17,6 +17,10 @@ file, see writeSection.
 (thetao, so, sigma0...; from the T file unless FILE is given): one column per (transect, class), headed
 label[b_j–b_{j+1}), the water with b_j <= value < b_{j+1} (Field.fluxClasses).  Not combined with --layers /
 --depthLayers.
+--tracer NAME[:FILE] [--tracerRef R] weights every transect's flux by a T-grid tracer (thetao, so...; from the T file
+unless FILE is given) taken at the C-grid faces, minus R (default 0): the heat, salt or freshwater it carries
+(Field.fluxTracer), in tracer units x flux units.  One column per transect, or per (transect, layer) with --layers /
+--depthLayers, headed label[NAME] or label[NAME top-bottom m].  Not combined with --classField or --section.
 --timeMean N|month|year averages over windows of N steps, or of the steps of each calendar month / year
 (timeobj.timeWindows): the printed and CSV series become window means (windowMeans), one row per window labelled
 first/last (the dates of its first and last step), and the --section file holds window means computed on the device
@@ -70,6 +74,13 @@ def windowMeans(x, bounds):
 def classLabels(labels, bounds):
     """column headings of a class series, transect-major: label[b_j–b_{j+1})"""
     return [f'{lab}[{b0:g}–{b1:g})' for lab in labels for b0, b1 in zip(bounds[:-1], bounds[1:])]
+
+
+def tracerLabels(labels, name, iface=None, layers=None):
+    """column headings of a tracer series, transect-major: label[NAME], or label[NAME top-bottom m] per layer"""
+    if layers is None:
+        return [f'{lab}[{name}]' for lab in labels]
+    return [f'{lab}[{name} {iface[k0]:g}-{iface[k1]:g} m]' for lab in labels for k0, k1 in zip(layers[:-1], layers[1:])]
 
 
 def writeSection(path, fld, layers, units, windows=None):
@@ -145,7 +156,15 @@ def main(argv=None):
                     help='write the transport section (flux per cell crossing and layer) to this NetCDF file')
     ap.add_argument('--timeMean', type=parseTimeMean, default=None,
                     help='average over windows of N steps, or per calendar month / year: N|month|year')
+    ap.add_argument('--tracer', default=None,
+                    help='transport of a T-grid tracer at the cell faces: NAME or NAME:FILE (default file: the T file)')
+    ap.add_argument('--tracerRef', type=float, default=None,
+                    help='reference value subtracted from the tracer (default 0): --tracerRef=34.8')
     a = ap.parse_args(argv)
+    if a.tracerRef is not None and a.tracer is None:
+        ap.error('--tracerRef needs --tracer')
+    if a.tracer is not None and (a.classField is not None or a.section):
+        ap.error('--tracer cannot be combined with --classField or --section')
     if (a.classField is None) != (a.classBounds is None):
         ap.error('--classField and --classBounds go together')
     pts, names = parseTransects(a.lonLatPoints, a.iFiles)
@@ -155,6 +174,9 @@ def main(argv=None):
     if a.classField is not None:
         var, _, cfile = a.classField.partition(':')
         series = fld.fluxClasses(var, a.classBounds, file=cfile or None)
+    elif a.tracer is not None:
+        tvar, _, tfile = a.tracer.partition(':')
+        series = fld.fluxTracer(tvar, file=tfile or None, ref=a.tracerRef or 0.0, layers=layers)
     else:
         series = fld.fluxSeries(layers=layers)
     timeVals = [fld.timeObj.getTimeAsDate(i) for i in range(fld.nt)]
@@ -166,7 +188,12 @@ def main(argv=None):
     units = 'Sv' if a.sverdrup else 'A m^2/s'
     labels = [os.path.basename(n) for n in names]
     rows = series
-    if layers is not None:
+    if a.tracer is not None:
+        units = f'{tvar} x {units}'
+        labels = tracerLabels(labels, tvar, fld.layerInterfaces() if layers is not None else None, layers)
+        if layers is not None:
+            rows = numpy.asarray(series).transpose(0, 2, 1).reshape(len(series), -1)   # (time, transect-major layers)
+    elif layers is not None:
         iface = fld.layerInterfaces()
         labels = [f'{lab}[{iface[k0]:g}-{iface[k1]:g} m]' for lab in labels for k0, k1 in zip(layers[:-1], layers[1:])]
         rows = numpy.asarray(series).transpose(0, 2, 1).reshape(len(series), -1)   # (time, transect-major layers)

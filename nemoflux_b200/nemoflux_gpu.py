@@ -427,17 +427,7 @@ class PolylineIntegral(object):
             return out
         keep = (u, v, e3u, e3v)  # keep pinned tensors alive while numpy views are in use
         h = _host_inputs(u, v, thickness, arc1, arc2, e3u, e3v)
-        c = numpy.asarray(cfield.numpy() if isinstance(cfield, torch.Tensor) else cfield)
-        if c.dtype != h.u.dtype:
-            raise ValueError(f'cfield must have the dtype and byte order of uo ({h.u.dtype}), got {c.dtype}')
-        nz, ny, nx = h.u.shape[1:]
-        if c.ndim == 3 and c.shape == (nz, ny, nx):
-            c = c[None]
-        if c.ndim == 3:
-            c = c.reshape(c.shape[0], c.shape[1], ny, nx) if c.shape[2] == ny * nx else c
-        if c.ndim != 4 or c.shape[1:] != (nz, ny, nx) or c.shape[0] not in (1, h.nt):
-            raise ValueError(f'cfield must be (1 or nt, nz, ny, nx) or (nz, ny, nx), got shape {c.shape}')
-        c = numpy.ascontiguousarray(c)
+        c = _class_field_host(cfield, h)
         res = numpy.zeros((h.nt, b.size - 1, m), numpy.float64)
         pu, pv, e3_nt, on_device = h.e3 if h.e3 is not None else (None, None, 0, False)
         _lib.call('nfx_flux_classes_host', ctypes.byref(self._h), _np_ptr(h.u), _np_ptr(h.v), pu, pv, h.code, e3_nt,
@@ -446,6 +436,66 @@ class PolylineIntegral(object):
                   int(chunk_steps), _np_ptr(res))
         del keep
         return res
+
+    def fluxTracer(self, u, v, thickness, arc1, arc2, tracer, ref=0.0, tfill=float('nan'), layers=None, section=False,
+                   sverdrup=False, fill=float('nan'), e3u=None, e3v=None, chunk_steps=0):
+        """tracer transport: the flux across every transect weighted by a tracer (temperature, salinity...) taken at
+        the C-grid face of every edge -> float64, (nt, M) for layers=None and (nt, N, M) otherwise, as fluxSeries; with
+        section=True the value of every crossing, (nt, N, nsub), one layer per level by default, as fluxSection.
+
+        Arguments as fluxSection (CUDA tensors on the current stream, or host arrays through the chunk pipeline), plus:
+        tracer, at the T points, with the dtype, byte order and plane layout of uo/vo, (1 or nt, nz, ...) (a (nz, ny,
+        nx) tracer is time-invariant); tfill its missing-value marker (compared in the storage type; NaN is always
+        missing); ref a reference value subtracted from the face value.
+
+        The face of an edge lies between two T cells (E: c and east(c), W: west(c) and c, N: c and north(c), none in
+        the top row, S: south(c) and c; x-periodic); its value at level k is 0.5 * (tau_a + tau_b) - ref with both
+        sides present, tau - ref with one, 0 with none.  Every level term of fluxSection's edge sums is multiplied by
+        it: with tracer == 1 and ref == 0 the section is fluxSection's bit for bit.  The series folds the crossings of
+        a transect as fluxClasses does (32-crossing tiles by a fixed tree, tiles in order): the bits depend only on the
+        inputs, whatever chunk_steps, the byte order or the side of the inputs.  Units: tracer units x flux units."""
+        torch = _torch()
+        lev = _layer_levels(layers)
+        m = self.getNumberOfTransects()
+        nsub = self.getNumberOfSubsegments()
+        width = nsub if section else m
+
+        def levels(nz):
+            if lev is not None:
+                return lev
+            return numpy.arange(nz + 1, dtype=numpy.int32) if section else numpy.array([0, nz], numpy.int32)
+
+        def shaped(x):          # (nt, M) for a series without layers
+            return x if section or lev is not None else x.reshape(x.shape[0], m)
+        if isinstance(u, torch.Tensor) and u.is_cuda:
+            u, v, nt, nz, ncell, ld = self._device_inputs(u, v, thickness, arc1, arc2, e3u, e3v)
+            use_e3 = e3u is not None or e3v is not None
+            tracer, tr_nt = _class_field_device(tracer, u, nt, nz, ncell, ld, 'tracer')
+            lv = levels(nz)
+            out = torch.zeros((nt, lv.size - 1, width), dtype=torch.float64, device=u.device)
+            if nt == 0 or nsub == 0:        # nothing to compute: no launch (empty tensors have no device address)
+                return shaped(out)
+            e3_nt = _check_e3(e3u, e3v, u, nt, nz, ncell, ld) if use_e3 else 0
+            ptr = lambda t: _t_ptr(t) if t is not None else None   # noqa: E731
+            with torch.cuda.device(u.device):
+                _lib.call('nfx_flux_tracer', ctypes.byref(self._h), _t_ptr(u), _t_ptr(v), ptr(e3u), ptr(e3v),
+                          _dtype_code(str(u.dtype)), e3_nt, None if use_e3 else _t_ptr(thickness), _t_ptr(arc1),
+                          _t_ptr(arc2), nt, nz, ld, _t_ptr(tracer), tr_nt, float(tfill), float(ref), lv.size - 1,
+                          _np_ptr(lv), int(bool(sverdrup)), float(fill), None if section else _t_ptr(out),
+                          _t_ptr(out) if section else None, _stream_ptr())
+            return shaped(out)
+        keep = (u, v, e3u, e3v)  # keep pinned tensors alive while numpy views are in use
+        h = _host_inputs(u, v, thickness, arc1, arc2, e3u, e3v)
+        c = _class_field_host(tracer, h, 'tracer')
+        lv = levels(h.nz)
+        res = numpy.zeros((h.nt, lv.size - 1, width), numpy.float64)
+        pu, pv, e3_nt, on_device = h.e3 if h.e3 is not None else (None, None, 0, False)
+        _lib.call('nfx_flux_tracer_host', ctypes.byref(self._h), _np_ptr(h.u), _np_ptr(h.v), pu, pv, h.code, e3_nt,
+                  int(on_device), None if h.th is None else _np_ptr(h.th), _np_ptr(h.a1), _np_ptr(h.a2), h.nt, h.nz,
+                  _np_ptr(c), c.shape[0], float(tfill), float(ref), lv.size - 1, _np_ptr(lv), int(bool(sverdrup)),
+                  float(fill), int(chunk_steps), None if section else _np_ptr(res), _np_ptr(res) if section else None)
+        del keep
+        return shaped(res)
 
     def _section_device_inputs(self, u, v, thickness, arc1, arc2, e3u, e3v, lev):
         """checks of the CUDA inputs of fluxSection / sectionWindowSums -> (u, v, nt, nz, ncell, ld, levels), the
@@ -867,20 +917,38 @@ def _check_e3(e3u, e3v, u, nt, nz, ncell, ld):
     return int(e3u.shape[0])
 
 
-def _class_field_device(c, u, nt, nz, ncell, ld):
-    """the class field of fluxClasses on the device: a CUDA tensor with the dtype and plane layout of uo, (1 or nt, nz,
-    ny, nx), (1 or nt, nz, cells) or (nz, ny, nx) -> (c with a time axis, its number of time steps)"""
+def _class_field_device(c, u, nt, nz, ncell, ld, name='cfield'):
+    """a T-grid field next to uo/vo on the device (the class field of fluxClasses, the tracer of fluxTracer): a CUDA
+    tensor with the dtype and plane layout of uo, (1 or nt, nz, ny, nx), (1 or nt, nz, cells) or (nz, ny, nx) -> (c with
+    a time axis, its number of time steps)"""
     torch = _torch()
     if not isinstance(c, torch.Tensor) or not c.is_cuda or c.dtype != u.dtype:
-        raise TypeError('cfield must be a CUDA tensor with the dtype of uo/vo')
+        raise TypeError(f'{name} must be a CUDA tensor with the dtype of uo/vo')
     if c.dim() == 3 and c.shape[0] == nz and c.shape[1] * c.shape[2] == ncell and c.shape[2] != ncell:
         c = c.unsqueeze(0)                                  # (z, y, x): time-invariant
-    cnt, cnz, cncell, cld = _plane_layout(c, 'cfield')
+    cnt, cnz, cncell, cld = _plane_layout(c, name)
     # the kernel steps levels by ld and time steps by nz * ld, the layout of uo/vo
     if (cnz, cncell) != (nz, ncell) or cnt not in (1, nt) or (cld != ld and cnz > 1) or \
             (cnt > 1 and c.stride(0) != nz * ld):
-        raise ValueError('cfield must be (1 or nt, nz, cells) with the plane layout of uo/vo')
+        raise ValueError(f'{name} must be (1 or nt, nz, cells) with the plane layout of uo/vo')
     return c, int(cnt)
+
+
+def _class_field_host(c, h, name='cfield'):
+    """the same next to host uo/vo (h: _host_inputs): the dtype and byte order of uo, (1 or nt, nz, ny, nx),
+    (1 or nt, nz, ny*nx) or (nz, ny, nx) -> C-contiguous (1 or nt, nz, ny, nx)"""
+    torch = _torch()
+    c = numpy.asarray(c.numpy() if isinstance(c, torch.Tensor) else c)
+    if c.dtype != h.u.dtype:
+        raise ValueError(f'{name} must have the dtype and byte order of uo ({h.u.dtype}), got {c.dtype}')
+    nz, ny, nx = h.u.shape[1:]
+    if c.ndim == 3 and c.shape == (nz, ny, nx):
+        c = c[None]
+    if c.ndim == 3:
+        c = c.reshape(c.shape[0], c.shape[1], ny, nx) if c.shape[2] == ny * nx else c
+    if c.ndim != 4 or c.shape[1:] != (nz, ny, nx) or c.shape[0] not in (1, h.nt):
+        raise ValueError(f'{name} must be (1 or nt, nz, ny, nx) or (nz, ny, nx), got shape {c.shape}')
+    return numpy.ascontiguousarray(c)
 
 
 def _require_cuda(t, dtype, name):
