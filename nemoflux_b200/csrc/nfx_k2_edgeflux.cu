@@ -573,7 +573,8 @@ void bswap_inplace(void* p, size_t n, int esize, cudaStream_t s) {
 // One launch over `ncols` adjacent columns (a panel of the grid, pointers already offset to its first column)
 // and `nt` time steps; ld = cells per level plane.  eflux: (nt, 2*ncols).  Layered (levels: device, nlayers + 1
 // ascending level boundaries): eflux (nt, nlayers, 2*ncols), layer i summed over the levels [levels[i], levels[i+1]);
-// always the direct-load kernel (the TMA variant sums whole columns only).
+// always the direct-load kernel (the TMA variant sums whole columns only).  Any nt: more than 65535 steps run in
+// slices of 65535.
 void edgeflux_assemble_panel(const void* u, const void* v, int dtype, const double* thickness, const double* arc1,
                              const double* arc2, int nt, int nz, int64_t ncols, int64_t ld, int sverdrup, double fill,
                              double* eflux, int keep_l2, const K2Options& opt, cudaStream_t s, const void* e3u,
@@ -591,9 +592,22 @@ void edgeflux_assemble_panel(const void* u, const void* v, int dtype, const doub
     NFX_REQUIRE(nlayers >= 1 && (levels != nullptr || nlayers == 1), "edgeflux: bad layering");
     NFX_REQUIRE(nt >= 0 && nz > 0 && ncols > 0 && ld >= ncols, "edgeflux: bad sizes");
     NFX_REQUIRE(dtype == NFX_F64 || dtype == NFX_F32, "edgeflux: dtype must be NFX_F64 or NFX_F32");
-    NFX_REQUIRE(nt <= 65535, "edgeflux: at most 65535 time steps per call");
     NFX_REQUIRE(nz <= 3000, "edgeflux: at most 3000 levels (dz and dz * 2^896 live in 48 KB of shared memory)");
     if (nt == 0) return;
+    if (nt > 65535) {
+        // gridDim.y carries the time steps: slices of at most 65535 steps, each a call of its own on the arrays offset
+        // to its first step (every slice picks its load width from its own addresses; the bits do not depend on it)
+        const int64_t esize = dtype == NFX_F64 ? 8 : 4;
+        for (int t0 = 0; t0 < nt; t0 += 65535) {
+            const int64_t off = (int64_t)t0 * nz * ld * esize, e3_off = (int64_t)t0 * e3_tstride * esize;
+            edgeflux_assemble_panel((const char*)u + off, (const char*)v + off, dtype, thickness, arc1, arc2,
+                                    std::min(65535, nt - t0), nz, ncols, ld, sverdrup, fill,
+                                    eflux + (int64_t)t0 * nlayers * 2 * ncols, keep_l2, opt, s,
+                                    e3u ? (const char*)e3u + e3_off : nullptr, e3v ? (const char*)e3v + e3_off : nullptr,
+                                    e3_tstride, nlayers, levels);
+        }
+        return;
+    }
     const double scale = 6371000.0 / 1.e6;  // field.py:12,226
     const int has_fill = !(fill != fill);
     const uintptr_t addr_bits = ((uintptr_t)u) | ((uintptr_t)v) | ((uintptr_t)eflux) | ((uintptr_t)e3u) | ((uintptr_t)e3v) |
